@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- PairHMM forward throughput (GCUPS) on B200, BASELINE.json's metric on BASELINE.json's configs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: row parameters, float forward kernels, the fallback-task builder,
 the double re-run (pmm_launch of include/pairhmm_cuda.h).  At N = 1 the workload is configs[1] of BASELINE.json
@@ -66,7 +66,12 @@ def parse():
     ap.add_argument("--no-sw", action="store_true", help="skip the Smith-Waterman block (SURVEY.md section 8f row 4)")
     ap.add_argument("--queue-jobs-per-gpu", type=int, default=192)
     ap.add_argument("--timeline", default="", help="write the pool's per-job timeline of the queue run to this .jsonl")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 # ---- clocks during the timed region ----------------------------------------------------------------------------------
@@ -204,6 +209,30 @@ def parity_of(raw, out, mask, ref) -> dict:
             "log10_bit_equal": bool(np.array_equal(out.view(np.uint64), out_r.view(np.uint64)))}
 
 
+DUMP_LIMIT_BYTES = 64_000_000          # 64 MB, files with their headers
+NPY_HEADER_RESERVE = 1024              # per file; np.save writes 128 bytes of header for a 1-D array
+
+
+def dump_outputs(path: str, raw, log10, mask, limit: int = DUMP_LIMIT_BYTES):
+    """Write what a caller of the timed path receives, one entry per pair in job order (regions in order, read-major):
+    raw.npy (float32 likelihoods of the float pass), log10.npy (float64 final log10 likelihoods) and fallback.npy (float32,
+    1 where the pair was re-run in double).  The inputs depend only on the arguments, so two builds run with the same
+    arguments can be compared file by file.  When the files would exceed `limit` bytes in all, a fixed seeded sample of the
+    pairs is written instead, in pair order, and pair_index.npy (float64) names the pairs it holds."""
+    arrays = {"raw": np.asarray(raw, dtype=np.float32).ravel(), "log10": np.asarray(log10, dtype=np.float64).ravel(),
+              "fallback": np.asarray(mask, dtype=np.float32).ravel()}
+    n = arrays["raw"].size
+    per_pair = sum(a.itemsize for a in arrays.values())
+    if n * per_pair + 3 * NPY_HEADER_RESERVE > limit:
+        keep = (limit - 4 * NPY_HEADER_RESERVE) // (per_pair + 8)
+        idx = np.sort(np.random.Generator(np.random.PCG64(0)).choice(n, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["pair_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def fallback_cells(batches, mask) -> int:
     """Cells (read_len x hap_len) of the pairs that take the double re-run."""
     pos, tot = 0, 0
@@ -248,7 +277,12 @@ def run_reference(args, rank: int, out=sys.stdout):
     cells = cells_of(batches)
     for _ in range(args.warmup):
         cpu_reference_pass(lib, batches, threads)
-    total = sum(cpu_reference_pass(lib, batches, threads)[0] for _ in range(args.steps))
+    total = 0.0
+    for _ in range(args.steps):
+        dt, res = cpu_reference_pass(lib, batches, threads)
+        total += dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *(np.concatenate([r[k].ravel() for r in res]) for k in range(3)))
     val = cells * args.steps / total * 1e-9
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -598,12 +632,14 @@ def _main(args, real_stdout):
     dev_s = gpu.timed_launches(args.steps)
     barrier()
     sampler.t1 = time.time()
+    raw, out, mask, nfb = gpu.results()                    # the last timed step's results
+    mask = mask.astype(bool)
     dev_noflush_s = gpu.timed_overlapped(args.steps)
     clocks = sampler.stop()
     log("timed region done")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, raw, out, mask)
     f32_ms, fb_ms = gpu.kernel_ms(min(args.steps, 10))
-    raw, out, mask, nfb = gpu.results()
-    mask = mask.astype(bool)
     st = eng.stats()
     pairs = int(st["pairs"])
     assert np.isfinite(raw).all() and not np.isnan(out).any()
