@@ -4,21 +4,19 @@
 // /root/reference/pairhmm/host/PairHMMFpga.cpp:125-162).  There is no CPU compute path in this file: without a
 // GPU every entry point fails with PMM_ERR_NO_DEVICE.
 #include "../../include/pairhmm_cuda.h"
+#include "cuda_util.h"
+#include "host_workers.h"
 #include "pmm_kernels.cuh"
 #include "pmm_plan.h"
 #include "pmm_tables.h"
 
 #include <algorithm>
 #include <atomic>
-#include <condition_variable>
-#include <mutex>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <functional>
-#include <numeric>
 #include <string>
 #include <thread>
 #include <vector>
@@ -33,36 +31,94 @@ constexpr size_t kAlign = 256;
 constexpr uint32_t kCtrlWords = kCtrlCursors + 32 * 104;
 inline size_t align_up(size_t x) { return (x + kAlign - 1) / kAlign * kAlign; }
 
-struct DevBuf {
-    void* p = nullptr; size_t cap = 0;
-    cudaError_t reserve(size_t n)
-    {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
-        size_t want = std::max(n, (size_t)4096);
-        want += want / 4;                         // grow-only with slack: buffers are recycled across jobs like the
-        cudaError_t e = cudaMalloc(&p, want);     // reference's scratch blocks (PairHMMTask.cpp:19-25,48,70)
-        if (e == cudaSuccess) cap = want;
-        return e;
-    }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+// Typed pointer to the section at byte offset `off` of a buffer (host or device side of the input arena).
+template <class T> T* section(void* base, size_t off) { return reinterpret_cast<T*>(static_cast<char*>(base) + off); }
+
+// The input arena, one H2D copy per job: read blob | descs | hap blob | descs | spos | tasks | regions | groups.
+struct ArenaLayout { size_t rblob = 0, rdesc = 0, hblob = 0, hdesc = 0, spos = 0, tasks = 0, regions = 0, groups = 0, bytes = 0; };
+ArenaLayout arena_layout(size_t rblob_bytes, uint32_t num_read, size_t hblob_bytes, uint32_t num_hap, uint64_t num_tasks,
+                         uint32_t num_region, size_t num_groups)
+{
+    ArenaLayout a;
+    size_t off = 0;
+    auto put = [&](size_t& at, size_t bytes) { at = off; off = align_up(off + bytes); };
+    put(a.rblob, rblob_bytes);
+    put(a.rdesc, sizeof(ReadDesc) * num_read);
+    put(a.hblob, hblob_bytes);
+    put(a.hdesc, sizeof(HapDesc) * num_hap);
+    put(a.spos, sizeof(uint32_t) * (num_hap + 1));
+    put(a.tasks, sizeof(Task) * num_tasks);
+    put(a.regions, sizeof(RegionDesc) * num_region);
+    put(a.groups, sizeof(GroupDesc) * num_groups);
+    a.bytes = off;
+    return a;
+}
+
+// The pinned block a launch's results are copied to: 256-byte header (control words) | raw floats | fallback indices |
+// doubles of the fallback pairs.
+struct OutLayout { size_t raw, idx, dres, bytes; };
+OutLayout out_layout(uint64_t pairs)
+{
+    OutLayout o;
+    o.raw = 256;
+    o.idx = o.raw + align_up(sizeof(float) * pairs);
+    o.dres = o.idx + align_up(sizeof(uint32_t) * pairs);
+    o.bytes = o.dres + sizeof(double) * pairs + 256;
+    return o;
+}
+
+// What pmm_stage_* leaves for pmm_launch and the fetches; every stage replaces it as a whole.
+struct StagedJob {
+    ArenaLayout at;                     // sections of the input arena
+    uint32_t num_region = 0, num_groups = 0, num_tasks = 0, num_rows = 0;
+    uint64_t pairs = 0;
+    uint32_t max_hap_len = 0;
+    std::vector<LaunchSeg> segs;        // one float-kernel launch each
+    int f64_rows = kF64K;               // rows per lane of the double kernel (pick_f64_rows) ...
+    bool f64_striped = true;            // ... and whether its longest read needs more than one stripe of 32 x rows
 };
 
-struct PinBuf {
-    void* p = nullptr; size_t cap = 0;
-    cudaError_t reserve(size_t n)
+// A job as stage() takes it.  read_off / hap_off (num + 1 entries) and the regions are what the planner reads; the
+// device-side blobs are the concatenation of read_parts / hap_parts, and the descriptors give every read's five tracks
+// (off, stride, len) and every haplotype (off, len) inside those blobs.  The context keeps one, reused by every job: the
+// flat builder points read_off, hap_off and regions at the caller's arrays, the other builders at roff, hoff and
+// own_regions.
+struct BlobPart { const uint8_t* p; size_t n; };
+struct JobSource {
+    uint32_t num_read = 0, num_hap = 0, num_region = 0;
+    const uint32_t* read_off = nullptr;
+    const uint32_t* hap_off = nullptr;
+    const pmm_region_t* regions = nullptr;
+    std::vector<BlobPart> read_parts, hap_parts;
+    std::vector<ReadDesc> rdesc;
+    std::vector<HapDesc> hdesc;
+    std::vector<uint32_t> roff, hoff;
+    std::vector<pmm_region_t> own_regions;
+
+    void reset()
     {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFreeHost(p);
-        p = nullptr; cap = 0;
-        size_t want = std::max(n, (size_t)4096);
-        want += want / 4;
-        cudaError_t e = cudaMallocHost(&p, want);
-        if (e == cudaSuccess) cap = want;
-        return e;
+        roff.assign(1, 0); hoff.assign(1, 0);
+        rdesc.clear(); hdesc.clear(); read_parts.clear(); hap_parts.clear(); own_regions.clear();
     }
-    void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
+    // Reads and haplotypes gathered from the caller's pointers: the five tracks of a read back to back, like the wire
+    // format.
+    void add_read(const char* const tracks[5], uint32_t len)
+    {
+        rdesc.push_back(ReadDesc{(uint32_t)(5ull * roff.back()), len, len});
+        roff.push_back(roff.back() + len);
+        for (int t = 0; t < 5; ++t) read_parts.push_back(BlobPart{reinterpret_cast<const uint8_t*>(tracks[t]), len});
+    }
+    void add_hap(const char* bases, uint32_t len)
+    {
+        hdesc.push_back(HapDesc{hoff.back(), len});
+        hoff.push_back(hoff.back() + len);
+        hap_parts.push_back(BlobPart{reinterpret_cast<const uint8_t*>(bases), len});
+    }
+    void use_own_arrays()
+    {
+        num_read = (uint32_t)rdesc.size(); num_hap = (uint32_t)hdesc.size(); num_region = (uint32_t)own_regions.size();
+        read_off = roff.data(); hap_off = hoff.data(); regions = own_regions.data();
+    }
 };
 
 }  // namespace
@@ -72,10 +128,20 @@ struct PinBuf {
 // results are copied to.  A fetch always refers to the set of the last launch.
 struct ResultSet {
     DevBuf d_raw, d_fb_tasks, d_fb_idx, d_fb_hap, d_fb_rows, d_dres, d_ctrl;
-    PinBuf h_out;                       // control words | raw floats | fallback indices | doubles
+    PinBuf h_out;                       // see out_layout
     cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};    // launch starts, float pass over, double re-run over
     cudaEvent_t ev_raw = nullptr, ev_lists = nullptr;   // the copies out of this set are over (its next user waits for them)
 };
+
+namespace {
+struct HostOut { uint32_t* ctrl; float* raw; uint32_t* idx; double* dres; };
+HostOut host_out(const ResultSet& r, uint64_t pairs)
+{
+    const OutLayout l = out_layout(pairs);
+    return HostOut{section<uint32_t>(r.h_out.p, 0), section<float>(r.h_out.p, l.raw), section<uint32_t>(r.h_out.p, l.idx),
+                   section<double>(r.h_out.p, l.dres)};
+}
+}  // namespace
 
 struct pmm_ctx {
     int device = 0;
@@ -99,12 +165,9 @@ struct pmm_ctx {
     int spin_us = 0;                    // "sync" = "hybrid": poll this long, then sleep on the blocking event
     bool auto_sync = false;             // "sync" = "auto": spin while few threads of the process do, else sleep
     std::string err;
-    int tasks_per_warp = 16;
+    PlanOptions plan_opt = plan_defaults();   // how stage() cuts jobs into warp-tasks (pmm_set_option)
     bool fast = false;                  // "mode" option: fast = contracted float kernels + exact re-check near the threshold
     float guard = 0.0078125f;           // "guard" option: relative half-width of the re-check band around 1e-28f (2^-7)
-    int f64_rows = kF64K;               // rows per lane of the double kernel for the staged job (pick_f64_rows)
-    bool f64_striped = true;            // ... and whether its longest read needs more than one stripe of 32 x rows
-    Variant force{0, 0, false};         // "force_variant" option (tuning sweeps): K,W of the float kernel
     int f64_tasks_per_warp = 6;         // "f64_tasks_per_warp": tasks the double re-run aims at per resident warp ...
     int f64_max_run = 6;                // "f64_max_run": ... and the most haplotypes it puts into one task (tools/f64_sweep.py)
     bool overlap = true;                // "overlap": consecutive launches overlap by one pass (off: a launch ends with its own re-run)
@@ -114,25 +177,14 @@ struct pmm_ctx {
     DeviceTables dtab{};
 
     // job state
-    PinBuf h_in;  DevBuf d_in;          // one arena: read blob | descs | hap blob | descs | spos | tasks | regions
+    PinBuf h_in;  DevBuf d_in;          // the input arena, see arena_layout
     DevBuf d_params, d_stream, d_iyf, d_iyd, d_tiny_tasks, d_scratch, d_scratch64, d_probe;
-    size_t off_rblob = 0, off_rdesc = 0, off_hblob = 0, off_hdesc = 0, off_spos = 0, off_tasks = 0, off_regions = 0, off_groups = 0;
-    uint32_t num_groups = 0;
-    uint32_t num_read = 0, num_hap = 0, num_region = 0, num_tasks = 0, num_rows = 0;
-    uint64_t pairs = 0, cells = 0;
-    uint32_t max_hap_len = 0;
-    std::vector<LaunchSeg> segs;
-    std::vector<pmm_region_t> regions;
+    StagedJob job;
     bool staged = false, launched = false;
     bool have_raw = false, have_lists = false;   // what of the last launch's results is already in h_out
     uint32_t spec = 0;                           // fallback entries copied back speculatively by pmm_launch
     pmm_stats_t stats{};
-
-    // scratch reused by the one-shot calls
-    std::vector<uint32_t> tmp_roff, tmp_hoff;
-    std::vector<ReadDesc> tmp_rdesc;
-    std::vector<HapDesc> tmp_hdesc;
-    std::vector<float> tmp_raw;
+    JobSource src;                               // scratch of the job builders, reused from job to job
 
     int fail_cuda(cudaError_t e, const char* what)
     {
@@ -164,22 +216,12 @@ int ensure_tables(pmm_ctx* c)
     return PMM_OK;
 }
 
-// Where the bytes of a job come from.  The device-side blobs are the concatenation of `parts`; the descriptors give
-// every read's five tracks (off, stride, len) and every haplotype (off, len) inside those blobs.  Two producers:
-// five flat track arrays (stride = total bases) and the reference's wire format taken as it is (stride = len,
-// interface/PairHMMHostInterface.cpp:175-207) -- the latter makes staging a serialized block one memcpy.
-struct BlobPart { const uint8_t* p; size_t n; };
-struct JobSource {
-    std::vector<BlobPart> read_parts, hap_parts;
-    const ReadDesc* rdesc = nullptr;
-    const HapDesc* hdesc = nullptr;
-};
-
-// Common staging: reads are given as (offset, length) into five tracks, haplotypes likewise into one.
-int stage_common(pmm_ctx* c, uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, const uint32_t* hap_off,
-                 const JobSource& src, uint32_t num_region, const pmm_region_t* regions)
+// The one staging path: plan the job, lay out and fill the pinned input arena, reserve the device buffers, enqueue the
+// H2D copy and the haplotype stream build.
+int stage(pmm_ctx* c, const JobSource& src)
 {
     auto t0 = std::chrono::steady_clock::now();
+    cudaSetDevice(c->device);
     c->staged = false; c->launched = false;
     // the pinned input arena is about to be repacked: the previous job's H2D copy out of it must be over
     // (stage, launch, stage with no fetch in between)
@@ -193,9 +235,7 @@ int stage_common(pmm_ctx* c, uint32_t num_read, const uint32_t* read_off, uint32
     size_t sz_rblob = 0, sz_hblob = 0;
     for (const BlobPart& bp : src.read_parts) sz_rblob += bp.n;
     for (const BlobPart& bp : src.hap_parts) sz_hblob += bp.n;
-    const size_t sz_rdesc = sizeof(ReadDesc) * num_read, sz_hdesc = sizeof(HapDesc) * num_hap;
-    const size_t sz_spos = sizeof(uint32_t) * (num_hap + 1), sz_regions = sizeof(RegionDesc) * num_region;
-    size_t sz_tasks = 0, sz_groups = 0, arena = 0;
+    StagedJob job;
     cudaError_t arena_err = cudaSuccess;
 
     // The planner calls back once it knows how many tasks and groups there are; the input arena is laid out and
@@ -203,61 +243,51 @@ int stage_common(pmm_ctx* c, uint32_t num_read, const uint32_t* read_off, uint32
     Plan plan;
     {
         std::string perr;
-        rc = plan_job(num_read, read_off, num_hap, hap_off, num_region, regions, c->sm_count, c->tasks_per_warp, plan, perr,
-                      c->force.K ? &c->force : nullptr, [&](const Plan& p) -> Task* {
-            sz_tasks = sizeof(Task) * p.num_tasks; sz_groups = sizeof(GroupDesc) * p.groups.size();
-            size_t off = 0;
-            c->off_rblob = off; off = align_up(off + sz_rblob);
-            c->off_rdesc = off; off = align_up(off + sz_rdesc);
-            c->off_hblob = off; off = align_up(off + sz_hblob);
-            c->off_hdesc = off; off = align_up(off + sz_hdesc);
-            c->off_spos = off; off = align_up(off + sz_spos);
-            c->off_tasks = off; off = align_up(off + sz_tasks);
-            c->off_regions = off; off = align_up(off + sz_regions);
-            c->off_groups = off; off = align_up(off + sz_groups);
-            arena = off;
-            if ((arena_err = c->h_in.reserve(arena)) != cudaSuccess) return nullptr;
-            if ((arena_err = c->d_in.reserve(arena)) != cudaSuccess) return nullptr;
-            return reinterpret_cast<Task*>(static_cast<char*>(c->h_in.p) + c->off_tasks);
+        rc = plan_job(src.num_read, src.read_off, src.num_hap, src.hap_off, src.num_region, src.regions, c->sm_count, c->plan_opt,
+                      plan, perr, [&](const Plan& p) -> Task* {
+            job.at = arena_layout(sz_rblob, src.num_read, sz_hblob, src.num_hap, p.num_tasks, src.num_region, p.groups.size());
+            if ((arena_err = c->h_in.reserve(job.at.bytes)) != cudaSuccess) return nullptr;
+            if ((arena_err = c->d_in.reserve(job.at.bytes)) != cudaSuccess) return nullptr;
+            return section<Task>(c->h_in.p, job.at.tasks);
         });
         if (arena_err != cudaSuccess) return c->fail_cuda(arena_err, "input arena");
         if (rc) return c->fail(rc, perr);
     }
     static const bool trace = getenv("PMM_TRACE_STAGE") != nullptr;       // phase times of staging on stderr
     const auto t_plan = std::chrono::steady_clock::now();
-    const uint32_t max_hap = plan.max_hap_len;
-    const uint64_t pairs = plan.pairs, cells = plan.cells;
-    const std::vector<RegionDesc>& rdesc = plan.regions;
-    c->max_hap_len = max_hap;
-    c->f64_rows = pick_f64_rows(plan.max_read_len);
-    c->f64_striped = plan.max_read_len + 1 > 32u * (uint32_t)c->f64_rows;
-    c->segs = plan.segs;
+    const ArenaLayout& at = job.at;
+    const uint64_t pairs = plan.pairs;
+    job.num_region = src.num_region; job.num_groups = (uint32_t)plan.groups.size();
+    job.num_tasks = (uint32_t)plan.num_tasks; job.num_rows = (uint32_t)plan.rows;
+    job.pairs = pairs;
+    job.max_hap_len = plan.max_hap_len;
+    job.segs = std::move(plan.segs);
+    job.f64_rows = pick_f64_rows(plan.max_read_len);
+    job.f64_striped = plan.max_read_len + 1 > 32u * (uint32_t)job.f64_rows;
 
     // ---- pack the rest of the input arena ---------------------------------------------------------------------
-    char* hb = static_cast<char*>(c->h_in.p);
     {
-        char* w = hb + c->off_rblob;
+        uint8_t* w = section<uint8_t>(c->h_in.p, at.rblob);
         for (const BlobPart& bp : src.read_parts) { memcpy(w, bp.p, bp.n); w += bp.n; }
-        w = hb + c->off_hblob;
+        w = section<uint8_t>(c->h_in.p, at.hblob);
         for (const BlobPart& bp : src.hap_parts) { memcpy(w, bp.p, bp.n); w += bp.n; }
     }
-    memcpy(hb + c->off_rdesc, src.rdesc, sz_rdesc);
-    memcpy(hb + c->off_hdesc, src.hdesc, sz_hdesc);
-    uint32_t* spos = reinterpret_cast<uint32_t*>(hb + c->off_spos);
+    memcpy(section<ReadDesc>(c->h_in.p, at.rdesc), src.rdesc.data(), sizeof(ReadDesc) * src.num_read);
+    memcpy(section<HapDesc>(c->h_in.p, at.hdesc), src.hdesc.data(), sizeof(HapDesc) * src.num_hap);
+    uint32_t* spos = section<uint32_t>(c->h_in.p, at.spos);
     uint32_t pos = 0;
-    for (uint32_t h = 0; h < num_hap; ++h) { spos[h] = pos; pos += src.hdesc[h].len + 1; }
-    spos[num_hap] = pos;                           // final separator
-    memcpy(hb + c->off_regions, rdesc.data(), sz_regions);
-    memcpy(hb + c->off_groups, plan.groups.data(), sz_groups);
-    c->num_groups = (uint32_t)plan.groups.size();
+    for (uint32_t h = 0; h < src.num_hap; ++h) { spos[h] = pos; pos += src.hdesc[h].len + 1; }
+    spos[src.num_hap] = pos;                       // final separator
+    memcpy(section<RegionDesc>(c->h_in.p, at.regions), plan.regions.data(), sizeof(RegionDesc) * src.num_region);
+    memcpy(section<GroupDesc>(c->h_in.p, at.groups), plan.groups.data(), sizeof(GroupDesc) * plan.groups.size());
 
     const auto t_pack = std::chrono::steady_clock::now();
     // ---- device buffers -------------------------------------------------------------------------------------
     const size_t stream_bytes = kStreamFrontPad + (size_t)pos + 1 + kStreamTailPad;
     PMM_CUDA(c, c->d_stream.reserve(stream_bytes));
     PMM_CUDA(c, c->d_params.reserve(sizeof(float) * plan.param_floats));
-    PMM_CUDA(c, c->d_iyf.reserve(sizeof(float) * num_hap));
-    PMM_CUDA(c, c->d_iyd.reserve(sizeof(double) * num_hap));
+    PMM_CUDA(c, c->d_iyf.reserve(sizeof(float) * src.num_hap));
+    PMM_CUDA(c, c->d_iyd.reserve(sizeof(double) * src.num_hap));
     if (c->fast) PMM_CUDA(c, c->d_tiny_tasks.reserve(sizeof(Task) * pairs));     // re-check list of the guard band
     for (ResultSet& r : c->rs) {
         PMM_CUDA(c, r.d_raw.reserve(sizeof(float) * pairs));
@@ -267,7 +297,7 @@ int stage_common(pmm_ctx* c, uint32_t num_read, const uint32_t* read_off, uint32
         PMM_CUDA(c, r.d_fb_rows.reserve(sizeof(uint32_t) * 2 * plan.rows));
         PMM_CUDA(c, r.d_dres.reserve(sizeof(double) * pairs));
         PMM_CUDA(c, r.d_ctrl.reserve(sizeof(uint32_t) * kCtrlWords));
-        PMM_CUDA(c, r.h_out.reserve(256 + align_up(sizeof(float) * pairs) + align_up(sizeof(uint32_t) * pairs) + sizeof(double) * pairs + 256));
+        PMM_CUDA(c, r.h_out.reserve(out_layout(pairs).bytes));
     }
     // carry rows of the striped kernels: one haplotype (+2 separators) per warp, three rows of doubles
     {
@@ -276,204 +306,165 @@ int stage_common(pmm_ctx* c, uint32_t num_read, const uint32_t* read_off, uint32
         const int ctas32 = std::max(std::max(forward_f32_ctas_per_sm(kStripedK, 32, true, false), forward_f32_ctas_per_sm(kStripedK, 32, true, true)),
                                     recheck_f32_ctas_per_sm());
         // the float and the double kernel of neighbouring launches can be on the GPU together: a scratch of their own each
-        PMM_CUDA(c, c->d_scratch.reserve((size_t)c->sm_count * ctas32 * kWarpsPerCta * 3 * (size_t)(max_hap + 8) * sizeof(float)));
-        PMM_CUDA(c, c->d_scratch64.reserve((size_t)c->sm_count * ctas64 * kWarpsPerCta * 3 * (size_t)(max_hap + 8) * sizeof(double)));
+        PMM_CUDA(c, c->d_scratch.reserve((size_t)c->sm_count * ctas32 * kWarpsPerCta * 3 * (size_t)(job.max_hap_len + 8) * sizeof(float)));
+        PMM_CUDA(c, c->d_scratch64.reserve((size_t)c->sm_count * ctas64 * kWarpsPerCta * 3 * (size_t)(job.max_hap_len + 8) * sizeof(double)));
     }
 
     cudaStream_t s = c->stream;
-    PMM_CUDA(c, cudaMemcpyAsync(c->d_in.p, c->h_in.p, arena, cudaMemcpyHostToDevice, s));
+    PMM_CUDA(c, cudaMemcpyAsync(c->d_in.p, c->h_in.p, at.bytes, cudaMemcpyHostToDevice, s));
     PMM_CUDA(c, cudaEventRecord(c->ev_h2d, s));
     c->h2d_pending = true;
     PMM_CUDA(c, cudaMemsetAsync(c->d_stream.p, 0, kStreamFrontPad, s));
     PMM_CUDA(c, cudaMemsetAsync(static_cast<char*>(c->d_stream.p) + kStreamFrontPad + pos + 1, 0, kStreamTailPad, s));
-    char* db = static_cast<char*>(c->d_in.p);
     const HostTables& ht = host_tables();
-    PMM_CUDA(c, launch_build_stream(reinterpret_cast<uint8_t*>(db + c->off_hblob), reinterpret_cast<HapDesc*>(db + c->off_hdesc),
-                                    reinterpret_cast<uint32_t*>(db + c->off_spos), num_hap,
+    PMM_CUDA(c, launch_build_stream(section<uint8_t>(c->d_in.p, at.hblob), section<HapDesc>(c->d_in.p, at.hdesc),
+                                    section<uint32_t>(c->d_in.p, at.spos), src.num_hap,
                                     static_cast<uint8_t*>(c->d_stream.p) + kStreamFrontPad,
                                     static_cast<float*>(c->d_iyf.p), static_cast<double*>(c->d_iyd.p), ht.ic_f, ht.ic_d, s));
 
-    c->num_read = num_read; c->num_hap = num_hap; c->num_region = num_region; c->num_tasks = (uint32_t)plan.num_tasks;
-    c->num_rows = (uint32_t)plan.rows;
-    c->pairs = pairs; c->cells = cells;
-    c->regions.assign(regions, regions + num_region);
     c->stats = pmm_stats_t{};
-    c->stats.pairs = pairs; c->stats.cells = cells; c->stats.h2d_bytes = arena; c->stats.f32_tasks = c->num_tasks;
+    c->stats.pairs = pairs; c->stats.cells = plan.cells; c->stats.h2d_bytes = at.bytes; c->stats.f32_tasks = job.num_tasks;
     c->stats.ms_stage = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (trace) {
         auto us = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double, std::micro>(b - a).count(); };
-        fprintf(stderr, "[stage] %u reads x %u haps, %zu tasks: plan %.0f us, pack %.0f us, reserve + enqueue %.0f us\n", num_read, num_hap,
+        fprintf(stderr, "[stage] %u reads x %u haps, %zu tasks: plan %.0f us, pack %.0f us, reserve + enqueue %.0f us\n", src.num_read, src.num_hap,
                 (size_t)plan.num_tasks, us(t0, t_plan), us(t_plan, t_pack), us(t_pack, std::chrono::steady_clock::now()));
     }
+    c->job = std::move(job);
     c->staged = true;
     return PMM_OK;
 }
 
-// Walk the reference's wire format (PairHMMHostInterface.cpp:175-207) and return offsets into the blob.
-bool scan_reads(const uint8_t* p, uint64_t n, std::vector<uint32_t>& off, std::vector<uint32_t>& len)
+// Walk one block of the reference's wire format (PairHMMHostInterface.cpp:175-207): a count, then per element a length
+// word and `tracks` arrays of that many bytes (reads 5, haplotypes 1).  Calls each(offset of the first array, length).
+template <class F> bool scan_wire(const uint8_t* p, uint64_t n, uint32_t tracks, F&& each)
 {
-    if (n < 4) return false;
+    if (!p || n < 4) return false;
     int32_t num; memcpy(&num, p, 4);
     if (num < 0) return false;
     uint64_t pos = 4;
-    if ((uint64_t)num > (n - 4) / 4) return false;          // every read takes at least its length word
-    off.resize(num); len.resize(num);
+    if ((uint64_t)num > (n - 4) / 4) return false;          // every element takes at least its length word
     for (int32_t i = 0; i < num; ++i) {
         if (pos + 4 > n) return false;
         int32_t l; memcpy(&l, p + pos, 4); pos += 4;
-        if (l < 0 || pos + 5ull * l > n) return false;
-        off[i] = (uint32_t)pos; len[i] = (uint32_t)l; pos += 5ull * l;
+        if (l < 0 || pos + (uint64_t)tracks * l > n) return false;
+        each((uint32_t)pos, (uint32_t)l); pos += (uint64_t)tracks * l;
     }
     return true;
 }
 
-bool scan_haps(const uint8_t* p, uint64_t n, std::vector<uint32_t>& off, std::vector<uint32_t>& len)
-{
-    if (n < 4) return false;
-    int32_t num; memcpy(&num, p, 4);
-    if (num < 0) return false;
-    uint64_t pos = 4;
-    if ((uint64_t)num > (n - 4) / 4) return false;
-    off.resize(num); len.resize(num);
-    for (int32_t i = 0; i < num; ++i) {
-        if (pos + 4 > n) return false;
-        int32_t l; memcpy(&l, p + pos, 4); pos += 4;
-        if (l < 0 || pos + (uint64_t)l > n) return false;
-        off[i] = (uint32_t)pos; len[i] = (uint32_t)l; pos += l;
-    }
-    return true;
-}
+// ---- job builders: each fills c->src ------------------------------------------------------------------------
 
-// The wire format as the job source: lengths go to tmp_roff / tmp_hoff for the planner, the blobs are the serialized
-// buffers themselves.
-int source_from_serialized(pmm_ctx* c, const void* reads_ser, uint64_t reads_bytes, const void* haps_ser, uint64_t haps_bytes,
-                           JobSource& src)
-{
-    std::vector<uint32_t> roff, rlen, hoff, hlen;
-    const uint8_t* rp = static_cast<const uint8_t*>(reads_ser);
-    const uint8_t* hp = static_cast<const uint8_t*>(haps_ser);
-    if (!rp || !hp || !scan_reads(rp, reads_bytes, roff, rlen) || !scan_haps(hp, haps_bytes, hoff, hlen))
-        return c->fail(PMM_ERR_INVALID, "malformed serialized block");
-    if (reads_bytes >= (1ull << 31) || haps_bytes >= (1ull << 31)) return c->fail(PMM_ERR_INVALID, "serialized block larger than 2 GiB");
-    const size_t nr = roff.size(), nh = hoff.size();
-    c->tmp_roff.assign(nr + 1, 0); c->tmp_hoff.assign(nh + 1, 0);
-    c->tmp_rdesc.resize(nr); c->tmp_hdesc.resize(nh);
-    for (size_t i = 0; i < nr; ++i) {
-        c->tmp_roff[i + 1] = c->tmp_roff[i] + rlen[i];
-        c->tmp_rdesc[i] = ReadDesc{roff[i], rlen[i], rlen[i]};
-    }
-    for (size_t i = 0; i < nh; ++i) {
-        c->tmp_hoff[i + 1] = c->tmp_hoff[i] + hlen[i];
-        c->tmp_hdesc[i] = HapDesc{hoff[i], hlen[i]};
-    }
-    src.read_parts = {BlobPart{rp, (size_t)reads_bytes}};
-    src.hap_parts = {BlobPart{hp, (size_t)haps_bytes}};
-    src.rdesc = c->tmp_rdesc.data(); src.hdesc = c->tmp_hdesc.data();
-    return PMM_OK;
-}
-
-// Five flat tracks + one haplotype array, (offset, length) per element.
-void source_from_flat(pmm_ctx* c, uint32_t num_read, const uint32_t* read_off, const uint8_t* const tracks[5],
-                      uint32_t num_hap, const uint32_t* hap_off, const uint8_t* hap_bases, JobSource& src)
+// Five flat tracks + one haplotype array, (offset, length) per element; the offsets and regions are the caller's.
+void source_from_flat(JobSource& s, uint32_t num_read, const uint32_t* read_off, const uint8_t* const tracks[5],
+                      uint32_t num_hap, const uint32_t* hap_off, const uint8_t* hap_bases, uint32_t num_region, const pmm_region_t* regions)
 {
     const uint32_t r_base = read_off[0], h_base = hap_off[0];
     const size_t total_bases = read_off[num_read] - r_base, total_hap = hap_off[num_hap] - h_base;
-    c->tmp_rdesc.resize(num_read); c->tmp_hdesc.resize(num_hap);
+    s.rdesc.resize(num_read); s.hdesc.resize(num_hap);
     for (uint32_t i = 0; i < num_read; ++i)
-        c->tmp_rdesc[i] = ReadDesc{read_off[i] - r_base, (uint32_t)total_bases, read_off[i + 1] - read_off[i]};
-    for (uint32_t h = 0; h < num_hap; ++h) c->tmp_hdesc[h] = HapDesc{hap_off[h] - h_base, hap_off[h + 1] - hap_off[h]};
-    src.read_parts.clear();
-    for (int t = 0; t < 5; ++t) src.read_parts.push_back(BlobPart{tracks[t] + r_base, total_bases});
-    src.hap_parts = {BlobPart{hap_bases + h_base, total_hap}};
-    src.rdesc = c->tmp_rdesc.data(); src.hdesc = c->tmp_hdesc.data();
+        s.rdesc[i] = ReadDesc{read_off[i] - r_base, (uint32_t)total_bases, read_off[i + 1] - read_off[i]};
+    for (uint32_t h = 0; h < num_hap; ++h) s.hdesc[h] = HapDesc{hap_off[h] - h_base, hap_off[h + 1] - hap_off[h]};
+    s.read_parts.clear();
+    for (int t = 0; t < 5; ++t) s.read_parts.push_back(BlobPart{tracks[t] + r_base, total_bases});
+    s.hap_parts.assign(1, BlobPart{hap_bases + h_base, total_hap});
+    s.num_read = num_read; s.read_off = read_off;
+    s.num_hap = num_hap; s.hap_off = hap_off;
+    s.num_region = num_region; s.regions = regions;
 }
 
-int stage_single_region(pmm_ctx* c, const JobSource& src)
+// The wire format, one region: the blobs are the serialized buffers themselves (stride = len), which makes staging a
+// serialized block one memcpy.
+int source_from_serialized(pmm_ctx* c, const void* reads_ser, uint64_t reads_bytes, const void* haps_ser, uint64_t haps_bytes,
+                           int* num_read, int* num_hap)
 {
-    const uint32_t nr = (uint32_t)c->tmp_roff.size() - 1, nh = (uint32_t)c->tmp_hoff.size() - 1;
+    JobSource& s = c->src;
+    s.reset();
+    const uint8_t* rp = static_cast<const uint8_t*>(reads_ser);
+    const uint8_t* hp = static_cast<const uint8_t*>(haps_ser);
+    const bool ok = scan_wire(rp, reads_bytes, 5, [&](uint32_t off, uint32_t len) {
+                        s.rdesc.push_back(ReadDesc{off, len, len}); s.roff.push_back(s.roff.back() + len); }) &&
+                    scan_wire(hp, haps_bytes, 1, [&](uint32_t off, uint32_t len) {
+                        s.hdesc.push_back(HapDesc{off, len}); s.hoff.push_back(s.hoff.back() + len); });
+    if (!ok) return c->fail(PMM_ERR_INVALID, "malformed serialized block");
+    if (reads_bytes >= (1ull << 31) || haps_bytes >= (1ull << 31)) return c->fail(PMM_ERR_INVALID, "serialized block larger than 2 GiB");
+    s.read_parts.assign(1, BlobPart{rp, (size_t)reads_bytes});
+    s.hap_parts.assign(1, BlobPart{hp, (size_t)haps_bytes});
+    const uint32_t nr = (uint32_t)s.rdesc.size(), nh = (uint32_t)s.hdesc.size();
+    if (num_read) *num_read = (int)nr;
+    if (num_hap) *num_hap = (int)nh;
     if (nr == 0 || nh == 0) return c->fail(PMM_ERR_INVALID, "empty batch");
-    pmm_region_t reg{0, nr, 0, nh};
-    return stage_common(c, nr, c->tmp_roff.data(), nh, c->tmp_hoff.data(), src, 1, &reg);
+    s.own_regions.assign(1, pmm_region_t{0, nr, 0, nh});
+    s.use_own_arrays();
+    return PMM_OK;
 }
 
-// Host worker threads for the per-result log10 (the one piece of the path that stays on the host so that it uses the
-// host libm like the reference).  Created once per process on first use; a fetch hands out chunks and takes part
-// itself, so small jobs never wait for a wake-up.  A call that finds the workers taken runs on its own thread.
-class HostWorkers {
- public:
-    static HostWorkers& get() { static HostWorkers w; return w; }
-    void run(uint64_t n, uint64_t grain, const std::function<void(uint64_t, uint64_t)>& f)
-    {
-        if (n <= grain || th_.empty()) { f(0, n); return; }
-        // Workers busy with another context's results: the process is streaming jobs through several contexts, and
-        // the caller's own thread is the parallelism (24 feeder threads on an 8-GPU box) -- do not queue up behind them.
-        std::unique_lock<std::mutex> call(call_mu_, std::try_to_lock);
-        if (!call.owns_lock()) { f(0, n); return; }
-        {
-            std::lock_guard<std::mutex> lk(mu_);
-            fn_ = &f; n_ = n; grain_ = grain; next_.store(0); busy_ = (int)th_.size(); ++gen_;
-        }
-        cv_work_.notify_all();
-        work();
-        std::unique_lock<std::mutex> lk(mu_);
-        cv_done_.wait(lk, [&] { return busy_ == 0; });
-        fn_ = nullptr;
-    }
-
- private:
-    HostWorkers()
-    {
-        const unsigned hw = std::thread::hardware_concurrency();
-        const unsigned n = hw > 1 ? std::min(hw - 1, 7u) : 0;
-        for (unsigned k = 0; k < n; ++k) th_.emplace_back([this] { loop(); });
-    }
-    ~HostWorkers()
-    {
-        { std::lock_guard<std::mutex> lk(mu_); stop_ = true; }
-        cv_work_.notify_all();
-        for (auto& t : th_) t.join();
-    }
-    void work()
-    {
-        for (;;) {
-            const uint64_t a = next_.fetch_add(grain_);
-            if (a >= n_) return;
-            (*fn_)(a, std::min(n_, a + grain_));
-        }
-    }
-    void loop()
-    {
-        uint64_t seen = 0;
-        for (;;) {
-            {
-                std::unique_lock<std::mutex> lk(mu_);
-                cv_work_.wait(lk, [&] { return stop_ || gen_ != seen; });
-                if (stop_) return;
-                seen = gen_;
-            }
-            work();
-            { std::lock_guard<std::mutex> lk(mu_); --busy_; }
-            cv_done_.notify_one();
-        }
-    }
-    std::vector<std::thread> th_;
-    std::mutex mu_, call_mu_;
-    std::condition_variable cv_work_, cv_done_;
-    const std::function<void(uint64_t, uint64_t)>* fn_ = nullptr;
-    uint64_t n_ = 0, grain_ = 1, gen_ = 0;
-    std::atomic<uint64_t> next_{0};
-    int busy_ = 0;
-    bool stop_ = false;
-};
-
-void parallel_for(uint64_t n, uint64_t grain, const std::function<void(uint64_t, uint64_t)>& f)
+// pmm_read_t / pmm_hap_t arrays, one region: every track of every read is one part of the blob.
+int source_from_structs(pmm_ctx* c, const pmm_read_t* reads, int num_read, const pmm_hap_t* haps, int num_hap)
 {
-    HostWorkers::get().run(n, std::max<uint64_t>(grain, 1), f);
+    JobSource& s = c->src;
+    s.reset();
+    s.read_parts.reserve(5 * (size_t)num_read); s.hap_parts.reserve(num_hap);
+    for (int i = 0; i < num_read; ++i) {
+        const pmm_read_t& r = reads[i];
+        if (r.len <= 0 || !r._b || !r._q || !r._i || !r._d || !r._c) return c->fail(PMM_ERR_INVALID, "read of length 0 or null track");
+        const char* tr[5] = {r._b, r._q, r._i, r._d, r._c};
+        s.add_read(tr, (uint32_t)r.len);
+        if (5ull * s.roff.back() >= (1ull << 31)) return c->fail(PMM_ERR_INVALID, "batch larger than 2 GiB: split it");
+    }
+    for (int i = 0; i < num_hap; ++i) {
+        if (haps[i].len <= 0 || !haps[i]._b) return c->fail(PMM_ERR_INVALID, "haplotype of length 0 or null");
+        s.add_hap(haps[i]._b, (uint32_t)haps[i].len);
+    }
+    s.own_regions.assign(1, pmm_region_t{0, (uint32_t)num_read, 0, (uint32_t)num_hap});
+    s.use_own_arrays();
+    return PMM_OK;
 }
-}  // namespace
 
-// the same workers for the other engine of this library (sw_engine.cu: staging and CIGAR scatter)
-namespace pmm { void host_parallel_for(uint64_t n, uint64_t grain, const std::function<void(uint64_t, uint64_t)>& f) { parallel_for(n, grain, f); } }
+// A GKL-shaped batch: one testcase per pair, pointers shared between the pairs of a read and of a haplotype.  Consecutive
+// testcases with the same read are a row; consecutive rows with the same haplotype sequence are a region.  The results
+// of the regions, read-major, are then exactly the testcases' order.
+int source_from_testcases(pmm_ctx* c, const pmm_testcase_t* tc, uint64_t n)
+{
+    auto same_read = [](const pmm_testcase_t& a, const pmm_testcase_t& b) {
+        return a.rs == b.rs && a.rslen == b.rslen && a.q == b.q && a.i == b.i && a.d == b.d && a.c == b.c; };
+    JobSource& s = c->src;
+    s.reset();
+    uint64_t k = 0, prev_row = 0, prev_len = 0;        // previous row: testcases [prev_row, prev_row + prev_len)
+    uint64_t hbytes = 0;
+    bool have_prev = false;
+    while (k < n) {
+        uint64_t e = k + 1;
+        while (e < n && same_read(tc[k], tc[e])) ++e;
+        const pmm_testcase_t& t = tc[k];
+        if (t.rslen <= 0 || !t.rs || !t.q || !t.i || !t.d || !t.c) return c->fail(PMM_ERR_INVALID, "read of length 0 or null track");
+        bool same_haps = have_prev && e - k == prev_len;
+        for (uint64_t z = 0; same_haps && z < e - k; ++z)
+            same_haps = tc[k + z].hap == tc[prev_row + z].hap && tc[k + z].haplen == tc[prev_row + z].haplen;
+        if (!same_haps) {
+            // a new region: its haplotypes are this row's
+            s.own_regions.push_back(pmm_region_t{(uint32_t)s.rdesc.size(), 0, (uint32_t)s.hdesc.size(), (uint32_t)(e - k)});
+            for (uint64_t z = k; z < e; ++z) {
+                if (tc[z].haplen <= 0 || !tc[z].hap) return c->fail(PMM_ERR_INVALID, "haplotype of length 0 or null");
+                s.add_hap(tc[z].hap, (uint32_t)tc[z].haplen);
+                hbytes += (uint32_t)tc[z].haplen;
+            }
+        }
+        const char* tr[5] = {t.rs, t.q, t.i, t.d, t.c};
+        s.add_read(tr, (uint32_t)t.rslen);
+        if (5ull * s.roff.back() + hbytes >= (1ull << 31)) return c->fail(PMM_ERR_INVALID, "batch larger than 2 GiB: split it");
+        s.own_regions.back().num_read++;
+        prev_row = k; prev_len = e - k; have_prev = true;
+        k = e;
+    }
+    uint64_t pairs = 0;
+    for (const pmm_region_t& r : s.own_regions) pairs += (uint64_t)r.num_read * r.num_hap;
+    if (pairs != n) return c->fail(PMM_ERR_INVALID, "internal: testcase grouping lost pairs");
+    s.use_own_arrays();
+    return PMM_OK;
+}
+
+}  // namespace
 
 // The double re-run's stream, at the priority of the float pass's.  (Tried: one level above it, so that a re-run's blocks
 // take freed slots before the next float pass's -- no difference in throughput on configs 2, 3 and 4 or through the pool,
@@ -498,6 +489,37 @@ template <class F> static int guarded(pmm_ctx* c, F&& f)
     }
 }
 
+// The one-shot entries: the job a builder left in c->src (`built` is the builder's status), staged, launched, fetched.
+template <class Fetch> static int stage_launch_fetch(pmm_ctx* c, int built, Fetch&& fetch)
+{
+    int rc = built;
+    if (rc || (rc = stage(c, c->src)) || (rc = pmm_launch(c))) return rc;
+    return fetch();
+}
+
+// The peak probes: one warm-up launch(warm_iters), then the best of three timed launch(iters) of `ops` lane instructions
+// each, in lane instructions per second.
+template <class Launch> static int probe_rate(pmm_ctx* c, Launch&& launch, int warm_iters, int iters, double ops, double* rate)
+{
+    PMM_CUDA(c, launch(warm_iters));
+    cudaEvent_t end;
+    PMM_CUDA(c, cudaEventCreate(&end));
+    double best = 0;
+    cudaError_t e = cudaSuccess;
+    for (int rep = 0; rep < 3 && e == cudaSuccess; ++rep) {
+        e = cudaEventRecord(c->ev_probe, c->stream);
+        if (e == cudaSuccess) e = launch(iters);
+        if (e == cudaSuccess) e = cudaEventRecord(end, c->stream);
+        if (e == cudaSuccess) e = cudaEventSynchronize(end);
+        float ms = 0;
+        if (e == cudaSuccess) { cudaEventElapsedTime(&ms, c->ev_probe, end); best = std::max(best, ops / (ms * 1e-3)); }
+    }
+    cudaEventDestroy(end);
+    if (e != cudaSuccess) return c->fail_cuda(e, "peak probe");
+    *rate = best;
+    return PMM_OK;
+}
+
 // =========================================================================================================
 extern "C" {
 
@@ -512,25 +534,12 @@ int pmm_create(int device, pmm_ctx** out)
 {
     if (!out) return PMM_ERR_INVALID;
     *out = nullptr;
-    int n = 0;
-    cudaError_t e = cudaGetDeviceCount(&n);
-    if (e != cudaSuccess || n == 0) {
-        cudaGetLastError();
-        g_create_error = "no CUDA device visible; this engine has no CPU fallback";
-        return PMM_ERR_NO_DEVICE;
-    }
-    if (device < 0) { if (cudaGetDevice(&device) != cudaSuccess) device = 0; }
-    if (device >= n) { g_create_error = "device index out of range"; return PMM_ERR_INVALID; }
-    cudaDeviceProp prop;
-    if ((e = cudaSetDevice(device)) != cudaSuccess || (e = cudaGetDeviceProperties(&prop, device)) != cudaSuccess) {
-        g_create_error = cudaGetErrorString(e); return PMM_ERR_CUDA;
-    }
-    if (prop.major != 10) {
-        g_create_error = std::string("kernels are built for sm_100a only; device is ") + prop.name;
-        return PMM_ERR_NO_DEVICE;
-    }
+    int sm_count = 0;
+    const int rc = open_device<PMM_ERR_INVALID, PMM_ERR_CUDA, PMM_ERR_NO_DEVICE>(device, sm_count, g_create_error, "this engine");
+    if (rc) return rc;
     pmm_ctx* c = new pmm_ctx();
-    c->device = device; c->sm_count = prop.multiProcessorCount;
+    c->device = device; c->sm_count = sm_count;
+    cudaError_t e;
     if ((e = cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking)) != cudaSuccess) {
         g_create_error = cudaGetErrorString(e); delete c; return PMM_ERR_CUDA;
     }
@@ -568,16 +577,11 @@ void pmm_destroy(pmm_ctx* c)
     if (c->f64_stream) cudaStreamSynchronize(c->f64_stream);
     if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
     if (c->list_stream) cudaStreamSynchronize(c->list_stream);
-    for (DevBuf* b : {&c->tables, &c->d_in, &c->d_params, &c->d_stream, &c->d_iyf, &c->d_iyd, &c->d_tiny_tasks, &c->d_scratch,
-                      &c->d_scratch64, &c->d_probe}) b->release();
     for (ResultSet& r : c->rs) {
-        for (DevBuf* b : {&r.d_raw, &r.d_fb_tasks, &r.d_fb_idx, &r.d_fb_hap, &r.d_fb_rows, &r.d_dres, &r.d_ctrl}) b->release();
-        r.h_out.release();
         for (auto& ev : r.ev) if (ev) cudaEventDestroy(ev);
         if (r.ev_raw) cudaEventDestroy(r.ev_raw);
         if (r.ev_lists) cudaEventDestroy(r.ev_lists);
     }
-    c->h_in.release();
     if (c->ev_probe) cudaEventDestroy(c->ev_probe);
     if (c->f64_stream) cudaStreamDestroy(c->f64_stream);
     if (c->ev_block) cudaEventDestroy(c->ev_block);
@@ -614,11 +618,12 @@ int pmm_set_option(pmm_ctx* c, const char* key, const char* value)
         int least = 0, greatest = 0;
         PMM_CUDA(c, cudaDeviceGetStreamPriorityRange(&least, &greatest));        // numerically: greatest <= least
         const int prio = std::min(least, greatest + rank);
-        cudaStream_t ns = nullptr, nd = nullptr;
-        PMM_CUDA(c, cudaStreamCreateWithPriority(&ns, cudaStreamNonBlocking, prio));
-        PMM_CUDA(c, create_f64_stream(&nd, prio));
         PMM_CUDA(c, cudaStreamSynchronize(c->own_stream));
         PMM_CUDA(c, cudaStreamSynchronize(c->f64_stream));
+        cudaStream_t ns = nullptr, nd = nullptr;
+        cudaError_t e = cudaStreamCreateWithPriority(&ns, cudaStreamNonBlocking, prio);
+        if (e == cudaSuccess && (e = create_f64_stream(&nd, prio)) != cudaSuccess) cudaStreamDestroy(ns);
+        if (e != cudaSuccess) return c->fail_cuda(e, "priority streams");
         const bool was_own = c->stream == c->own_stream;
         cudaStreamDestroy(c->own_stream); cudaStreamDestroy(c->f64_stream);
         c->own_stream = ns; c->f64_stream = nd;
@@ -628,20 +633,20 @@ int pmm_set_option(pmm_ctx* c, const char* key, const char* value)
     if (k == "tasks_per_warp") {
         const int v = atoi(value);
         if (v < 1 || v > 64) return c->fail(PMM_ERR_INVALID, "tasks_per_warp out of range");
-        c->tasks_per_warp = v;
+        c->plan_opt.tasks_per_warp = v;
         return PMM_OK;
     }
     if (k == "small_job_widening") {
         const std::string v(value);
         if (v != "0" && v != "1" && v != "on" && v != "off") return c->fail(PMM_ERR_INVALID, "small_job_widening is \"on\" or \"off\"");
-        set_small_job_widening(v == "1" || v == "on");   // process-wide (the planner has no context)
+        c->plan_opt.widening = v == "1" || v == "on";
         return PMM_OK;
     }
     if (k == "run_tiers") {
         int d = -1, share = kRunTierShare, top = kRunTierTop;
         if (std::sscanf(value, "%d,%d,%d", &d, &share, &top) < 1 || d < 0 || d > 64 || share < 1 || share > 100 || top < 1 || top > 64)
             return c->fail(PMM_ERR_INVALID, "run_tiers is \"depth[,share[,top]]\", depth 0..64, share 1..100, top 1..64");
-        set_run_tiers(d, share, top);                // process-wide (the planner has no context)
+        c->plan_opt.tiers = RunTiers{d, share, top};
         return PMM_OK;
     }
     if (k == "f64_tasks_per_warp" || k == "f64_max_run") {
@@ -680,38 +685,40 @@ int pmm_set_option(pmm_ctx* c, const char* key, const char* value)
         int K = 0, W = 0;
         if (sscanf(value, "%d,%d", &K, &W) != 2 || (K > 0 && !forward_f32_has_variant(K, W)))
             return c->fail(PMM_ERR_INVALID, "force_variant wants \"K,W\" of an instantiated float kernel, \"0,0\" (planner's choice) or \"-1,0\" (no consolidation of rare variants)");
-        c->force = Variant{K, W, false};
+        c->plan_opt.force = K > 0 ? Variant{K, W, false} : Variant{0, 0, false};
+        c->plan_opt.keep_all_variants = K < 0;
         return PMM_OK;
     }
     return c->fail(PMM_ERR_INVALID, "unknown option " + k);
 }
 
-static int pmm_stage_flat_impl(pmm_ctx* c, uint32_t num_read, const uint32_t* read_off,
+int pmm_stage_flat(pmm_ctx* c, uint32_t num_read, const uint32_t* read_off,
                    const uint8_t* bases, const uint8_t* q, const uint8_t* i, const uint8_t* d, const uint8_t* cc,
                    uint32_t num_hap, const uint32_t* hap_off, const uint8_t* hap_bases,
                    uint32_t num_region, const pmm_region_t* regions)
 {
-    if (!c) return PMM_ERR_INVALID;
-    if (!bases || !q || !i || !d || !cc || !hap_bases) return c->fail(PMM_ERR_INVALID, "null track");
-    cudaSetDevice(c->device);
-    if (!read_off || !hap_off || !num_read || !num_hap) return c->fail(PMM_ERR_INVALID, "empty job");
-    if (read_off[num_read] < read_off[0] || hap_off[num_hap] < hap_off[0]) return c->fail(PMM_ERR_INVALID, "offsets not ascending");
-    for (uint32_t k = 0; k < num_read; ++k) if (read_off[k + 1] < read_off[k]) return c->fail(PMM_ERR_INVALID, "offsets not ascending");
-    for (uint32_t k = 0; k < num_hap; ++k) if (hap_off[k + 1] < hap_off[k]) return c->fail(PMM_ERR_INVALID, "offsets not ascending");
-    const uint8_t* const tracks[5] = {bases, q, i, d, cc};
-    JobSource src;
-    source_from_flat(c, num_read, read_off, tracks, num_hap, hap_off, hap_bases, src);
-    return stage_common(c, num_read, read_off, num_hap, hap_off, src, num_region, regions);
+    return guarded(c, [&]() -> int {
+        if (!c) return PMM_ERR_INVALID;
+        if (!bases || !q || !i || !d || !cc || !hap_bases) return c->fail(PMM_ERR_INVALID, "null track");
+        if (!read_off || !hap_off || !num_read || !num_hap) return c->fail(PMM_ERR_INVALID, "empty job");
+        // before source_from_flat takes offsets relative to the first ones
+        if (read_off[num_read] < read_off[0] || hap_off[num_hap] < hap_off[0]) return c->fail(PMM_ERR_INVALID, "offsets not ascending");
+        for (uint32_t k = 0; k < num_read; ++k) if (read_off[k + 1] < read_off[k]) return c->fail(PMM_ERR_INVALID, "offsets not ascending");
+        for (uint32_t k = 0; k < num_hap; ++k) if (hap_off[k + 1] < hap_off[k]) return c->fail(PMM_ERR_INVALID, "offsets not ascending");
+        const uint8_t* const tracks[5] = {bases, q, i, d, cc};
+        source_from_flat(c->src, num_read, read_off, tracks, num_hap, hap_off, hap_bases, num_region, regions);
+        return stage(c, c->src);
+    });
 }
 
 int pmm_launch(pmm_ctx* c)
 {
     if (!c) return PMM_ERR_INVALID;
     if (!c->staged) return c->fail(PMM_ERR_STATE, "pmm_launch before pmm_stage_*");
-    if (c->fast && c->d_tiny_tasks.cap < sizeof(Task) * c->pairs) return c->fail(PMM_ERR_STATE, "mode changed to fast after pmm_stage_*: stage the job again");
+    const StagedJob& j = c->job;
+    if (c->fast && c->d_tiny_tasks.cap < sizeof(Task) * j.pairs) return c->fail(PMM_ERR_STATE, "mode changed to fast after pmm_stage_*: stage the job again");
     cudaSetDevice(c->device);
     cudaStream_t s = c->stream, sd = c->f64_stream;
-    char* db = static_cast<char*>(c->d_in.p);
     // This launch takes the other result set: the previous launch's double re-run may still be using its own.
     ResultSet& prev = c->rs[c->cur];
     c->cur ^= 1;
@@ -730,33 +737,33 @@ int pmm_launch(pmm_ctx* c)
     PMM_CUDA(c, cudaMemsetAsync(ctrl, 0, sizeof(uint32_t) * kCtrlWords, s));
 
     ForwardArgs a{};
-    a.read_blob = reinterpret_cast<uint8_t*>(db + c->off_rblob);
-    a.reads = reinterpret_cast<ReadDesc*>(db + c->off_rdesc);
+    a.read_blob = section<uint8_t>(c->d_in.p, j.at.rblob);
+    a.reads = section<ReadDesc>(c->d_in.p, j.at.rdesc);
     a.stream = static_cast<uint8_t*>(c->d_stream.p) + kStreamFrontPad;
-    a.spos = reinterpret_cast<uint32_t*>(db + c->off_spos);
+    a.spos = section<uint32_t>(c->d_in.p, j.at.spos);
     a.tab = c->dtab;
     a.scratch = c->d_scratch.p;
-    a.scratch_stride = c->max_hap_len + 8;
+    a.scratch_stride = j.max_hap_len + 8;
 
     // ---- row parameters, once per read (the reference recomputes them per pair) --------------------------------
     a.params = static_cast<float*>(c->d_params.p);
-    PMM_CUDA(c, launch_read_params(a.read_blob, a.reads, reinterpret_cast<GroupDesc*>(db + c->off_groups), c->num_groups,
+    PMM_CUDA(c, launch_read_params(a.read_blob, a.reads, section<GroupDesc>(c->d_in.p, j.at.groups), j.num_groups,
                                    c->dtab, static_cast<float*>(c->d_params.p), s));
     ++launches;
 
     // ---- float pass, one launch per (K, W) variant present in the job; results below 1e-28f are appended to the
     //      fallback list by the kernel itself (PairHMMWorker.cpp:176) ----------------------------------------------
-    if (c->segs.size() > 100) return c->fail(PMM_ERR_INVALID, "too many kernel variants in one job");
+    if (j.segs.size() > 100) return c->fail(PMM_ERR_INVALID, "too many kernel variants in one job");
     // fast mode: results within the guard band around the threshold are re-run by an exact kernel before the decision
     // is taken, so the decision (and the float value of those pairs) is the reference's, bit for bit
     const float thr = 1e-28f;
-    FallbackQueue fq{ctrl + 0, (uint32_t)c->pairs,
+    FallbackQueue fq{ctrl + 0, (uint32_t)j.pairs,
                      c->fast ? thr * (1.0f - c->guard) : thr, c->fast ? thr * (1.0f + c->guard) : thr,
                      static_cast<Task*>(c->d_tiny_tasks.p), ctrl + 2};
     uint32_t cursor = kCtrlCursors;
-    for (const LaunchSeg& seg : c->segs) {
+    for (const LaunchSeg& seg : j.segs) {
         a.inity = c->d_iyf.p;
-        a.tasks = reinterpret_cast<Task*>(db + c->off_tasks) + seg.task_first;
+        a.tasks = section<Task>(c->d_in.p, j.at.tasks) + seg.task_first;
         a.ntasks = seg.task_count; a.ntasks_dev = nullptr;
         a.counter = ctrl + cursor; cursor += 32;
         a.out = R.d_raw.p;
@@ -777,24 +784,22 @@ int pmm_launch(pmm_ctx* c)
     PMM_CUDA(c, cudaEventRecord(R.ev[1], s));
     // The raw floats are final now: copy them back on the copy stream while the double pass runs, so that a fetch can
     // take log10f of them (host libm) under it.
-    {
-        char* ho = static_cast<char*>(R.h_out.p);
-        PMM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, R.ev[1], 0));
-        PMM_CUDA(c, cudaMemcpyAsync(ho + 256, R.d_raw.p, sizeof(float) * c->pairs, cudaMemcpyDeviceToHost, c->copy_stream));
-        PMM_CUDA(c, cudaEventRecord(R.ev_raw, c->copy_stream));
-    }
+    const HostOut ho = host_out(R, j.pairs);
+    PMM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, R.ev[1], 0));
+    PMM_CUDA(c, cudaMemcpyAsync(ho.raw, R.d_raw.p, sizeof(float) * j.pairs, cudaMemcpyDeviceToHost, c->copy_stream));
+    PMM_CUDA(c, cudaEventRecord(R.ev_raw, c->copy_stream));
 
     // ---- double re-run (PairHMMWorker.cpp:176-184): the results below the threshold become tasks, the failing haplotypes
     //      of a read together; their number is only known on the device.  On its own stream: the next launch's float pass
     //      (this stream) starts as soon as this one's is over and runs next to it ------------------------------------------
     PMM_CUDA(c, cudaStreamWaitEvent(sd, R.ev[1], 0));
-    const int KD = c->f64_rows;
-    const int f64_ctas = c->sm_count * std::max(1, forward_f64_ctas_per_sm(KD, c->f64_striped));
+    const int KD = j.f64_rows;
+    const int f64_ctas = c->sm_count * std::max(1, forward_f64_ctas_per_sm(KD, j.f64_striped));
     FallbackBuild fb{};
     fb.raw = static_cast<float*>(R.d_raw.p);
-    fb.regions = reinterpret_cast<RegionDesc*>(db + c->off_regions);
+    fb.regions = section<RegionDesc>(c->d_in.p, j.at.regions);
     fb.reads = a.reads;
-    fb.num_region = c->num_region; fb.num_rows = c->num_rows;
+    fb.num_region = j.num_region; fb.num_rows = j.num_rows;
     fb.threshold = thr;
     fb.ctrl = ctrl;
     fb.tasks = static_cast<Task*>(R.d_fb_tasks.p);
@@ -802,8 +807,8 @@ int pmm_launch(pmm_ctx* c)
     fb.hap_list = static_cast<uint32_t*>(R.d_fb_hap.p);
     fb.row_slot = static_cast<uint32_t*>(R.d_fb_rows.p);
     fb.spos = a.spos;
-    fb.max_hap_len = c->max_hap_len;
-    fb.capacity = (uint32_t)c->pairs;
+    fb.max_hap_len = j.max_hap_len;
+    fb.capacity = (uint32_t)j.pairs;
     fb.single_stripe_rows = 32u * (uint32_t)KD;
     fb.target_tasks = (uint32_t)(f64_ctas * kWarpsPerCta * c->f64_tasks_per_warp);
     fb.max_run = (uint32_t)c->f64_max_run;
@@ -813,7 +818,7 @@ int pmm_launch(pmm_ctx* c)
     a.ntasks = 0; a.ntasks_dev = ctrl + 3; a.counter = ctrl + cursor; cursor += 32;
     a.tiny_threshold = ldexp(1.0, -800); a.tiny_count = ctrl + 1;
     a.scratch = c->d_scratch64.p;
-    PMM_CUDA(c, launch_forward_f64(KD, c->f64_striped, a, f64_ctas, sd));
+    PMM_CUDA(c, launch_forward_f64(KD, j.f64_striped, a, f64_ctas, sd));
     ++launches;
     PMM_CUDA(c, cudaEventRecord(R.ev[2], sd));
     // What is queued on the launch stream from here on (the next launch, an event of the caller's) comes after the
@@ -823,18 +828,13 @@ int pmm_launch(pmm_ctx* c)
     // The length of the fallback list is only known on the device.  Copy the control words and a first slice of the list
     // (an eighth of the pairs) back right behind the double pass, so that the common case needs no further round trip;
     // the rest, if any, follows in the fetch.
-    {
-        char* ho = static_cast<char*>(R.h_out.p);
-        uint32_t* hidx = reinterpret_cast<uint32_t*>(ho + 256 + align_up(sizeof(float) * c->pairs));
-        double* hd = reinterpret_cast<double*>(reinterpret_cast<char*>(hidx) + align_up(sizeof(uint32_t) * c->pairs));
-        c->spec = (uint32_t)std::min<uint64_t>(c->pairs, std::max<uint64_t>(1024, c->pairs / 8));
-        cudaStream_t ls = c->list_stream;                       // not a kernels' stream: the next job need not wait for these
-        PMM_CUDA(c, cudaStreamWaitEvent(ls, R.ev[2], 0));
-        PMM_CUDA(c, cudaMemcpyAsync(ho, R.d_ctrl.p, 12, cudaMemcpyDeviceToHost, ls));
-        PMM_CUDA(c, cudaMemcpyAsync(hidx, R.d_fb_idx.p, sizeof(uint32_t) * c->spec, cudaMemcpyDeviceToHost, ls));
-        PMM_CUDA(c, cudaMemcpyAsync(hd, R.d_dres.p, sizeof(double) * c->spec, cudaMemcpyDeviceToHost, ls));
-        PMM_CUDA(c, cudaEventRecord(R.ev_lists, ls));
-    }
+    c->spec = (uint32_t)std::min<uint64_t>(j.pairs, std::max<uint64_t>(1024, j.pairs / 8));
+    cudaStream_t ls = c->list_stream;                           // not a kernels' stream: the next job need not wait for these
+    PMM_CUDA(c, cudaStreamWaitEvent(ls, R.ev[2], 0));
+    PMM_CUDA(c, cudaMemcpyAsync(ho.ctrl, R.d_ctrl.p, 12, cudaMemcpyDeviceToHost, ls));
+    PMM_CUDA(c, cudaMemcpyAsync(ho.idx, R.d_fb_idx.p, sizeof(uint32_t) * c->spec, cudaMemcpyDeviceToHost, ls));
+    PMM_CUDA(c, cudaMemcpyAsync(ho.dres, R.d_dres.p, sizeof(double) * c->spec, cudaMemcpyDeviceToHost, ls));
+    PMM_CUDA(c, cudaEventRecord(R.ev_lists, ls));
     c->stats.kernel_launches = launches;
     c->launched = true;
     return PMM_OK;
@@ -911,18 +911,6 @@ static cudaError_t wait_stream(pmm_ctx* c, cudaStream_t st)
     return cudaEventSynchronize(c->ev_block);
 }
 
-struct HostOut { uint32_t* ctrl; float* raw; uint32_t* idx; double* dres; };
-static HostOut host_out(const pmm_ctx* c)
-{
-    char* ho = static_cast<char*>(c->R().h_out.p);
-    HostOut o;
-    o.ctrl = reinterpret_cast<uint32_t*>(ho);                                       // 256 B header
-    o.raw = reinterpret_cast<float*>(ho + 256);
-    o.idx = reinterpret_cast<uint32_t*>(ho + 256 + align_up(sizeof(float) * c->pairs));
-    o.dres = reinterpret_cast<double*>(reinterpret_cast<char*>(o.idx) + align_up(sizeof(uint32_t) * c->pairs));
-    return o;
-}
-
 // The raw floats of the last launch are in h_out (copied by pmm_launch on the copy stream; the double pass may still run).
 static int ensure_raw(pmm_ctx* c)
 {
@@ -942,10 +930,10 @@ static int ensure_lists(pmm_ctx* c)
     if (c->have_lists) return PMM_OK;
     cudaSetDevice(c->device);
     cudaStream_t s = c->list_stream;
-    const HostOut o = host_out(c);
+    const HostOut o = host_out(c->R(), c->job.pairs);
     PMM_CUDA(c, wait_stream(c, s));
     const uint32_t nfb = o.ctrl[0], spec = c->spec;
-    uint64_t d2h = 12 + sizeof(float) * c->pairs + (sizeof(uint32_t) + sizeof(double)) * spec;
+    uint64_t d2h = 12 + sizeof(float) * c->job.pairs + (sizeof(uint32_t) + sizeof(double)) * spec;
     if (nfb > spec) {
         PMM_CUDA(c, cudaMemcpyAsync(o.idx + spec, static_cast<uint32_t*>(c->R().d_fb_idx.p) + spec, sizeof(uint32_t) * (nfb - spec), cudaMemcpyDeviceToHost, s));
         PMM_CUDA(c, cudaMemcpyAsync(o.dres + spec, static_cast<double*>(c->R().d_dres.p) + spec, sizeof(double) * (nfb - spec), cudaMemcpyDeviceToHost, s));
@@ -964,7 +952,7 @@ static int ensure_lists(pmm_ctx* c)
 static void log10_of_raw(const float* raw, uint64_t n, double* out)
 {
     const float licf = host_tables().log10_ic_f;
-    parallel_for(n, 1 << 13, [&](uint64_t a, uint64_t b) { for (uint64_t k = a; k < b; ++k) out[k] = (double)(log10f(raw[k]) - licf); });
+    host_parallel_for(n, 1 << 13, [&](uint64_t a, uint64_t b) { for (uint64_t k = a; k < b; ++k) out[k] = (double)(log10f(raw[k]) - licf); });
 }
 // log10(d) - log10(2^1020) for the pairs that fell back (PairHMMWorker.cpp:184)
 static int log10_of_fallback(const uint32_t* fb_index, const double* fb_value, uint64_t n_fb, uint64_t n, double* out)
@@ -982,10 +970,10 @@ static int fetch_log10_common(pmm_ctx* c, double* out, uint32_t* nfb_out)
 {
     int rc = ensure_raw(c);
     if (rc) return rc;
-    const HostOut o = host_out(c);
-    log10_of_raw(o.raw, c->pairs, out);
+    const HostOut o = host_out(c->R(), c->job.pairs);
+    log10_of_raw(o.raw, c->job.pairs, out);
     if ((rc = ensure_lists(c))) return rc;
-    if (log10_of_fallback(o.idx, o.dres, o.ctrl[0], c->pairs, out) != PMM_OK) return c->fail(PMM_ERR_CUDA, "fallback index out of range");
+    if (log10_of_fallback(o.idx, o.dres, o.ctrl[0], c->job.pairs, out) != PMM_OK) return c->fail(PMM_ERR_CUDA, "fallback index out of range");
     if (nfb_out) *nfb_out = o.ctrl[0];
     return PMM_OK;
 }
@@ -993,11 +981,11 @@ static int fetch_log10_common(pmm_ctx* c, double* out, uint32_t* nfb_out)
 int pmm_fetch_raw(pmm_ctx* c, float* out_raw, uint64_t cap)
 {
     if (!c || !out_raw) return PMM_ERR_INVALID;
-    if (cap < c->pairs) return c->fail(PMM_ERR_INVALID, "output buffer too small");
+    if (cap < c->job.pairs) return c->fail(PMM_ERR_INVALID, "output buffer too small");
     auto t0 = std::chrono::steady_clock::now();
     int rc = ensure_raw(c);
     if (rc) return rc;
-    memcpy(out_raw, host_out(c).raw, sizeof(float) * c->pairs);
+    memcpy(out_raw, host_out(c->R(), c->job.pairs).raw, sizeof(float) * c->job.pairs);
     c->stats.ms_fetch = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return PMM_OK;
 }
@@ -1005,11 +993,11 @@ int pmm_fetch_raw(pmm_ctx* c, float* out_raw, uint64_t cap)
 int pmm_fetch_fallback_mask(pmm_ctx* c, uint8_t* mask, uint64_t cap)
 {
     if (!c || !mask) return PMM_ERR_INVALID;
-    if (cap < c->pairs) return c->fail(PMM_ERR_INVALID, "mask buffer too small");
+    if (cap < c->job.pairs) return c->fail(PMM_ERR_INVALID, "mask buffer too small");
     int rc = ensure_lists(c);
     if (rc) return rc;
-    memset(mask, 0, c->pairs);
-    const HostOut o = host_out(c);
+    memset(mask, 0, c->job.pairs);
+    const HostOut o = host_out(c->R(), c->job.pairs);
     for (uint32_t k = 0; k < o.ctrl[0]; ++k) mask[o.idx[k]] = 1;
     return PMM_OK;
 }
@@ -1024,7 +1012,7 @@ int pmm_host_finish_log10(const float* raw, uint64_t n, const uint32_t* fb_index
 int pmm_fetch_log10(pmm_ctx* c, double* out, uint64_t cap, uint64_t* n_fallback)
 {
     if (!c || !out) return PMM_ERR_INVALID;
-    if (cap < c->pairs) return c->fail(PMM_ERR_INVALID, "output buffer too small");
+    if (cap < c->job.pairs) return c->fail(PMM_ERR_INVALID, "output buffer too small");
     auto t0 = std::chrono::steady_clock::now();
     uint32_t nfb = 0;
     int rc = fetch_log10_common(c, out, &nfb);
@@ -1037,7 +1025,7 @@ int pmm_fetch_log10(pmm_ctx* c, double* out, uint64_t cap, uint64_t* n_fallback)
 int pmm_fetch_log10_indexed(pmm_ctx* c, double* out, uint64_t cap, uint32_t* fb_index, uint64_t fb_cap, uint64_t* n_fallback)
 {
     if (!c || !out || !n_fallback) return PMM_ERR_INVALID;
-    if (cap < c->pairs) return c->fail(PMM_ERR_INVALID, "output buffer too small");
+    if (cap < c->job.pairs) return c->fail(PMM_ERR_INVALID, "output buffer too small");
     auto t0 = std::chrono::steady_clock::now();
     uint32_t nfb = 0;
     int rc = fetch_log10_common(c, out, &nfb);
@@ -1045,7 +1033,7 @@ int pmm_fetch_log10_indexed(pmm_ctx* c, double* out, uint64_t cap, uint32_t* fb_
     *n_fallback = nfb;
     if (fb_index) {
         if (fb_cap < nfb) return c->fail(PMM_ERR_INVALID, "fallback index buffer too small");
-        memcpy(fb_index, host_out(c).idx, sizeof(uint32_t) * nfb);
+        memcpy(fb_index, host_out(c->R(), c->job.pairs).idx, sizeof(uint32_t) * nfb);
     }
     c->stats.ms_fetch = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return PMM_OK;
@@ -1056,7 +1044,7 @@ int pmm_fetch_fallback(pmm_ctx* c, uint32_t* index, double* value, uint64_t cap,
     if (!c || !count) return PMM_ERR_INVALID;
     int rc = ensure_lists(c);
     if (rc) return rc;
-    const HostOut o = host_out(c);
+    const HostOut o = host_out(c->R(), c->job.pairs);
     const uint32_t nfb = o.ctrl[0];
     *count = nfb;
     if (!index && !value) return PMM_OK;
@@ -1066,17 +1054,14 @@ int pmm_fetch_fallback(pmm_ctx* c, uint32_t* index, double* value, uint64_t cap,
     return PMM_OK;
 }
 
-static int pmm_stage_serialized_impl(pmm_ctx* c, const void* reads_ser, uint64_t reads_bytes, const void* haps_ser,
+int pmm_stage_serialized(pmm_ctx* c, const void* reads_ser, uint64_t reads_bytes, const void* haps_ser,
                          uint64_t haps_bytes, int* num_read, int* num_hap)
 {
-    if (!c) return PMM_ERR_INVALID;
-    cudaSetDevice(c->device);
-    JobSource src;
-    int rc = source_from_serialized(c, reads_ser, reads_bytes, haps_ser, haps_bytes, src);
-    if (rc) return rc;
-    if (num_read) *num_read = (int)c->tmp_roff.size() - 1;
-    if (num_hap) *num_hap = (int)c->tmp_hoff.size() - 1;
-    return stage_single_region(c, src);
+    return guarded(c, [&]() -> int {
+        if (!c) return PMM_ERR_INVALID;
+        const int rc = source_from_serialized(c, reads_ser, reads_bytes, haps_ser, haps_bytes, num_read, num_hap);
+        return rc ? rc : stage(c, c->src);
+    });
 }
 
 int pmm_get_stats(const pmm_ctx* c, pmm_stats_t* out)
@@ -1086,198 +1071,70 @@ int pmm_get_stats(const pmm_ctx* c, pmm_stats_t* out)
     return PMM_OK;
 }
 
-static int pmm_forward_raw_serialized_impl(pmm_ctx* c, const void* reads_ser, uint64_t reads_bytes, const void* haps_ser,
-                               uint64_t haps_bytes, float* out_raw, uint64_t cap, int* num_read, int* num_hap)
-{
-    if (!c || !out_raw) return PMM_ERR_INVALID;
-    cudaSetDevice(c->device);
-    JobSource src;
-    int rc = source_from_serialized(c, reads_ser, reads_bytes, haps_ser, haps_bytes, src);
-    if (rc) return rc;
-    if (num_read) *num_read = (int)c->tmp_roff.size() - 1;
-    if (num_hap) *num_hap = (int)c->tmp_hoff.size() - 1;
-    if ((rc = stage_single_region(c, src))) return rc;
-    if ((rc = pmm_launch(c))) return rc;
-    return pmm_fetch_raw(c, out_raw, cap);
-}
-
-static int pmm_forward_log10_serialized_impl(pmm_ctx* c, const void* reads_ser, uint64_t reads_bytes, const void* haps_ser,
-                                 uint64_t haps_bytes, double* out, uint64_t cap, int* num_read, int* num_hap,
-                                 uint64_t* n_fallback)
-{
-    if (!c || !out) return PMM_ERR_INVALID;
-    cudaSetDevice(c->device);
-    JobSource src;
-    int rc = source_from_serialized(c, reads_ser, reads_bytes, haps_ser, haps_bytes, src);
-    if (rc) return rc;
-    if (num_read) *num_read = (int)c->tmp_roff.size() - 1;
-    if (num_hap) *num_hap = (int)c->tmp_hoff.size() - 1;
-    if ((rc = stage_single_region(c, src))) return rc;
-    if ((rc = pmm_launch(c))) return rc;
-    return pmm_fetch_log10(c, out, cap, n_fallback);
-}
-
-static int pmm_forward_log10_impl(pmm_ctx* c, const pmm_read_t* reads, int num_read, const pmm_hap_t* haps, int num_hap,
-                      double* out, uint64_t* n_fallback)
-{
-    if (!c || !reads || !haps || !out || num_read <= 0 || num_hap <= 0) return c ? c->fail(PMM_ERR_INVALID, "bad arguments") : PMM_ERR_INVALID;
-    cudaSetDevice(c->device);
-    // every track of every read is one part of the blob, laid out like the wire format (five tracks of a read back to back)
-    JobSource src;
-    c->tmp_roff.assign(num_read + 1, 0); c->tmp_hoff.assign(num_hap + 1, 0);
-    c->tmp_rdesc.resize(num_read); c->tmp_hdesc.resize(num_hap);
-    src.read_parts.reserve(5 * (size_t)num_read); src.hap_parts.reserve(num_hap);
-    uint64_t off = 0;
-    for (int i = 0; i < num_read; ++i) {
-        const pmm_read_t& r = reads[i];
-        if (r.len <= 0 || !r._b || !r._q || !r._i || !r._d || !r._c) return c->fail(PMM_ERR_INVALID, "read of length 0 or null track");
-        const uint32_t len = (uint32_t)r.len;
-        c->tmp_roff[i + 1] = c->tmp_roff[i] + len;
-        c->tmp_rdesc[i] = ReadDesc{(uint32_t)off, len, len};
-        const char* tr[5] = {r._b, r._q, r._i, r._d, r._c};
-        for (int t = 0; t < 5; ++t) src.read_parts.push_back(BlobPart{reinterpret_cast<const uint8_t*>(tr[t]), len});
-        off += 5ull * len;
-        if (off >= (1ull << 31)) return c->fail(PMM_ERR_INVALID, "batch larger than 2 GiB: split it");
-    }
-    off = 0;
-    for (int i = 0; i < num_hap; ++i) {
-        if (haps[i].len <= 0 || !haps[i]._b) return c->fail(PMM_ERR_INVALID, "haplotype of length 0 or null");
-        const uint32_t len = (uint32_t)haps[i].len;
-        c->tmp_hoff[i + 1] = c->tmp_hoff[i] + len;
-        c->tmp_hdesc[i] = HapDesc{(uint32_t)off, len};
-        src.hap_parts.push_back(BlobPart{reinterpret_cast<const uint8_t*>(haps[i]._b), len});
-        off += len;
-    }
-    src.rdesc = c->tmp_rdesc.data(); src.hdesc = c->tmp_hdesc.data();
-    int rc = stage_single_region(c, src);
-    if (rc) return rc;
-    if ((rc = pmm_launch(c))) return rc;
-    return pmm_fetch_log10(c, out, (uint64_t)num_read * num_hap, n_fallback);
-}
-
-// A GKL-shaped batch: one testcase per pair, pointers shared between the pairs of a read and of a haplotype.  Consecutive
-// testcases with the same read are a row; consecutive rows with the same haplotype sequence are a region.  The results
-// of the regions, read-major, are then exactly the testcases' order.
-static int pmm_forward_log10_testcases_impl(pmm_ctx* c, const pmm_testcase_t* tc, uint64_t n, double* out, uint64_t* n_fallback)
-{
-    if (!c) return PMM_ERR_INVALID;
-    if (!tc || !out || !n) return c->fail(PMM_ERR_INVALID, "bad arguments");
-    if (n >= (1ull << 31)) return c->fail(PMM_ERR_INVALID, "more than 2^31 pairs in one batch: split it");
-    cudaSetDevice(c->device);
-    auto same_read = [](const pmm_testcase_t& a, const pmm_testcase_t& b) {
-        return a.rs == b.rs && a.rslen == b.rslen && a.q == b.q && a.i == b.i && a.d == b.d && a.c == b.c; };
-    JobSource src;
-    std::vector<pmm_region_t> regions;
-    std::vector<uint32_t>& roff = c->tmp_roff; std::vector<uint32_t>& hoff = c->tmp_hoff;
-    roff.assign(1, 0); hoff.assign(1, 0);
-    c->tmp_rdesc.clear(); c->tmp_hdesc.clear();
-    uint64_t rbytes = 0, hbytes = 0;
-    uint64_t k = 0, prev_row = 0, prev_len = 0;        // previous row: testcases [prev_row, prev_row + prev_len)
-    bool have_prev = false;
-    while (k < n) {
-        uint64_t e = k + 1;
-        while (e < n && same_read(tc[k], tc[e])) ++e;
-        const pmm_testcase_t& t = tc[k];
-        if (t.rslen <= 0 || !t.rs || !t.q || !t.i || !t.d || !t.c) return c->fail(PMM_ERR_INVALID, "read of length 0 or null track");
-        bool same_haps = have_prev && e - k == prev_len;
-        for (uint64_t z = 0; same_haps && z < e - k; ++z)
-            same_haps = tc[k + z].hap == tc[prev_row + z].hap && tc[k + z].haplen == tc[prev_row + z].haplen;
-        if (!same_haps) {
-            // a new region: its haplotypes are this row's
-            pmm_region_t rg{(uint32_t)c->tmp_rdesc.size(), 0, (uint32_t)c->tmp_hdesc.size(), (uint32_t)(e - k)};
-            for (uint64_t z = k; z < e; ++z) {
-                if (tc[z].haplen <= 0 || !tc[z].hap) return c->fail(PMM_ERR_INVALID, "haplotype of length 0 or null");
-                const uint32_t len = (uint32_t)tc[z].haplen;
-                c->tmp_hdesc.push_back(HapDesc{(uint32_t)hbytes, len});
-                hoff.push_back(hoff.back() + len);
-                src.hap_parts.push_back(BlobPart{reinterpret_cast<const uint8_t*>(tc[z].hap), len});
-                hbytes += len;
-            }
-            regions.push_back(rg);
-        }
-        const uint32_t len = (uint32_t)t.rslen;
-        c->tmp_rdesc.push_back(ReadDesc{(uint32_t)rbytes, len, len});
-        roff.push_back(roff.back() + len);
-        const char* tr[5] = {t.rs, t.q, t.i, t.d, t.c};
-        for (int z = 0; z < 5; ++z) src.read_parts.push_back(BlobPart{reinterpret_cast<const uint8_t*>(tr[z]), len});
-        rbytes += 5ull * len;
-        if (rbytes + hbytes >= (1ull << 31)) return c->fail(PMM_ERR_INVALID, "batch larger than 2 GiB: split it");
-        regions.back().num_read++;
-        prev_row = k; prev_len = e - k; have_prev = true;
-        k = e;
-    }
-    src.rdesc = c->tmp_rdesc.data(); src.hdesc = c->tmp_hdesc.data();
-    int rc = stage_common(c, (uint32_t)c->tmp_rdesc.size(), roff.data(), (uint32_t)c->tmp_hdesc.size(), hoff.data(), src,
-                          (uint32_t)regions.size(), regions.data());
-    if (rc) return rc;
-    if (c->pairs != n) return c->fail(PMM_ERR_INVALID, "internal: testcase grouping lost pairs");
-    if ((rc = pmm_launch(c))) return rc;
-    return pmm_fetch_log10(c, out, n, n_fallback);
-}
-
-static int pmm_plan_flat_impl(uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, const uint32_t* hap_off,
-                  uint32_t num_region, const pmm_region_t* regions, int sm_count, int tasks_per_warp,
-                  pmm_task_info_t* out, uint64_t capacity, uint64_t* num_tasks)
-{
-    Plan plan; std::string perr;
-    int rc = plan_job(num_read, read_off, num_hap, hap_off, num_region, regions, sm_count, tasks_per_warp, plan, perr);
-    if (rc) { g_create_error = perr; return rc; }
-    if (num_tasks) *num_tasks = plan.tasks.size();
-    if (!out) return PMM_OK;
-    if (capacity < plan.tasks.size()) { g_create_error = "task buffer too small"; return PMM_ERR_INVALID; }
-    for (const LaunchSeg& seg : plan.segs)
-        for (uint32_t k = seg.task_first; k < seg.task_first + seg.task_count; ++k) {
-            const Task& t = plan.tasks[k];
-            pmm_task_info_t& o = out[k];
-            for (int z = 0; z < 4; ++z) { o.read[z] = t.read[z]; o.out_base[z] = t.out_base[z]; }
-            o.hap_first = t.hap_first; o.num_hap = t.nhaps; o.num_read = t.nreads;
-            o.rows_per_lane = (uint32_t)seg.v.K; o.lanes_per_read = (uint32_t)seg.v.W; o.striped = seg.v.striped ? 1u : 0u;
-        }
-    return PMM_OK;
-}
-
-int pmm_stage_flat(pmm_ctx* c, uint32_t num_read, const uint32_t* read_off,
-                   const uint8_t* bases, const uint8_t* q, const uint8_t* i, const uint8_t* d, const uint8_t* cc,
-                   uint32_t num_hap, const uint32_t* hap_off, const uint8_t* hap_bases,
-                   uint32_t num_region, const pmm_region_t* regions)
-{
-    return guarded(c, [&] { return pmm_stage_flat_impl(c, num_read, read_off, bases, q, i, d, cc, num_hap, hap_off, hap_bases, num_region, regions); });
-}
-
-int pmm_stage_serialized(pmm_ctx* c, const void* reads_ser, uint64_t reads_bytes, const void* haps_ser,
-                         uint64_t haps_bytes, int* num_read, int* num_hap)
-{
-    return guarded(c, [&] { return pmm_stage_serialized_impl(c, reads_ser, reads_bytes, haps_ser, haps_bytes, num_read, num_hap); });
-}
-
 int pmm_forward_raw_serialized(pmm_ctx* c, const void* reads_ser, uint64_t reads_bytes, const void* haps_ser,
                                uint64_t haps_bytes, float* out_raw, uint64_t cap, int* num_read, int* num_hap)
 {
-    return guarded(c, [&] { return pmm_forward_raw_serialized_impl(c, reads_ser, reads_bytes, haps_ser, haps_bytes, out_raw, cap, num_read, num_hap); });
+    return guarded(c, [&]() -> int {
+        if (!c || !out_raw) return PMM_ERR_INVALID;
+        return stage_launch_fetch(c, source_from_serialized(c, reads_ser, reads_bytes, haps_ser, haps_bytes, num_read, num_hap),
+                                  [&] { return pmm_fetch_raw(c, out_raw, cap); });
+    });
 }
 
 int pmm_forward_log10_serialized(pmm_ctx* c, const void* reads_ser, uint64_t reads_bytes, const void* haps_ser,
                                  uint64_t haps_bytes, double* out, uint64_t cap, int* num_read, int* num_hap,
                                  uint64_t* n_fallback)
 {
-    return guarded(c, [&] { return pmm_forward_log10_serialized_impl(c, reads_ser, reads_bytes, haps_ser, haps_bytes, out, cap, num_read, num_hap, n_fallback); });
+    return guarded(c, [&]() -> int {
+        if (!c || !out) return PMM_ERR_INVALID;
+        return stage_launch_fetch(c, source_from_serialized(c, reads_ser, reads_bytes, haps_ser, haps_bytes, num_read, num_hap),
+                                  [&] { return pmm_fetch_log10(c, out, cap, n_fallback); });
+    });
 }
 
 int pmm_forward_log10(pmm_ctx* c, const pmm_read_t* reads, int num_read, const pmm_hap_t* haps, int num_hap,
                       double* out, uint64_t* n_fallback)
 {
-    return guarded(c, [&] { return pmm_forward_log10_impl(c, reads, num_read, haps, num_hap, out, n_fallback); });
+    return guarded(c, [&]() -> int {
+        if (!c || !reads || !haps || !out || num_read <= 0 || num_hap <= 0) return c ? c->fail(PMM_ERR_INVALID, "bad arguments") : PMM_ERR_INVALID;
+        return stage_launch_fetch(c, source_from_structs(c, reads, num_read, haps, num_hap),
+                                  [&] { return pmm_fetch_log10(c, out, (uint64_t)num_read * num_hap, n_fallback); });
+    });
+}
+
+int pmm_forward_log10_testcases(pmm_ctx* c, const pmm_testcase_t* tc, uint64_t n, double* out, uint64_t* n_fallback)
+{
+    return guarded(c, [&]() -> int {
+        if (!c) return PMM_ERR_INVALID;
+        if (!tc || !out || !n) return c->fail(PMM_ERR_INVALID, "bad arguments");
+        if (n >= (1ull << 31)) return c->fail(PMM_ERR_INVALID, "more than 2^31 pairs in one batch: split it");
+        return stage_launch_fetch(c, source_from_testcases(c, tc, n), [&] { return pmm_fetch_log10(c, out, n, n_fallback); });
+    });
 }
 
 int pmm_plan_flat(uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, const uint32_t* hap_off,
                   uint32_t num_region, const pmm_region_t* regions, int sm_count, int tasks_per_warp,
                   pmm_task_info_t* out, uint64_t capacity, uint64_t* num_tasks)
 {
-    return guarded(nullptr, [&] { return pmm_plan_flat_impl(num_read, read_off, num_hap, hap_off, num_region, regions, sm_count, tasks_per_warp, out, capacity, num_tasks); });
-}
-int pmm_forward_log10_testcases(pmm_ctx* c, const pmm_testcase_t* tc, uint64_t n, double* out, uint64_t* n_fallback)
-{
-    return guarded(c, [&] { return pmm_forward_log10_testcases_impl(c, tc, n, out, n_fallback); });
+    return guarded(nullptr, [&]() -> int {
+        PlanOptions opt = plan_defaults();
+        opt.tasks_per_warp = tasks_per_warp;
+        Plan plan; std::string perr;
+        int rc = plan_job(num_read, read_off, num_hap, hap_off, num_region, regions, sm_count, opt, plan, perr);
+        if (rc) { g_create_error = perr; return rc; }
+        if (num_tasks) *num_tasks = plan.tasks.size();
+        if (!out) return PMM_OK;
+        if (capacity < plan.tasks.size()) { g_create_error = "task buffer too small"; return PMM_ERR_INVALID; }
+        for (const LaunchSeg& seg : plan.segs)
+            for (uint32_t k = seg.task_first; k < seg.task_first + seg.task_count; ++k) {
+                const Task& t = plan.tasks[k];
+                pmm_task_info_t& o = out[k];
+                for (int z = 0; z < 4; ++z) { o.read[z] = t.read[z]; o.out_base[z] = t.out_base[z]; }
+                o.hap_first = t.hap_first; o.num_hap = t.nhaps; o.num_read = t.nreads;
+                o.rows_per_lane = (uint32_t)seg.v.K; o.lanes_per_read = (uint32_t)seg.v.W; o.striped = seg.v.striped ? 1u : 0u;
+            }
+        return PMM_OK;
+    });
 }
 
 int pmm_host_table(int which, void* out, uint64_t capacity_bytes)
@@ -1304,21 +1161,11 @@ int pmm_measure_fp32_peak(pmm_ctx* c, double* lane_instr_per_s, double* sm_mhz)
     cudaSetDevice(c->device);
     const int ctas = c->sm_count * 8, iters = 500;
     PMM_CUDA(c, c->d_probe.reserve(sizeof(float) * ctas * 256));
-    cudaStream_t s = c->stream;
-    PMM_CUDA(c, launch_fp32_probe(static_cast<float*>(c->d_probe.p), 25, ctas, s));
-    double best = 0;
-    for (int rep = 0; rep < 3; ++rep) {
-        PMM_CUDA(c, cudaEventRecord(c->ev_probe, s));
-        PMM_CUDA(c, launch_fp32_probe(static_cast<float*>(c->d_probe.p), iters, ctas, s));
-        cudaEvent_t e1; cudaEventCreate(&e1);
-        PMM_CUDA(c, cudaEventRecord(e1, s));
-        PMM_CUDA(c, cudaEventSynchronize(e1));
-        float ms = 0; cudaEventElapsedTime(&ms, c->ev_probe, e1); cudaEventDestroy(e1);
-        const double ops = (double)ctas * 256 * iters * 512.0;
-        best = std::max(best, ops / (ms * 1e-3));
-    }
-    *lane_instr_per_s = best;
-    if (sm_mhz) *sm_mhz = best / ((double)c->sm_count * 128.0) * 1e-6;   // lower bound: assumes 128 lanes/clk/SM fully used
+    float* sink = static_cast<float*>(c->d_probe.p);
+    const int rc = probe_rate(c, [&](int n) { return launch_fp32_probe(sink, n, ctas, c->stream); }, 25, iters,
+                              (double)ctas * 256 * iters * 512.0, lane_instr_per_s);
+    if (rc) return rc;
+    if (sm_mhz) *sm_mhz = *lane_instr_per_s / ((double)c->sm_count * 128.0) * 1e-6;   // lower bound: assumes 128 lanes/clk/SM fully used
     return PMM_OK;
 }
 
@@ -1343,23 +1190,9 @@ int pmm_measure_fp64_peak(pmm_ctx* c, double* lane_instr_per_s)
     cudaSetDevice(c->device);
     const int ctas = c->sm_count * 8, iters = 60;
     PMM_CUDA(c, c->d_probe.reserve(sizeof(double) * ctas * 256));
-    cudaStream_t s = c->stream;
-    PMM_CUDA(c, launch_fp64_probe(static_cast<double*>(c->d_probe.p), 5, ctas, s));
-    double best = 0;
-    cudaEvent_t e1;
-    PMM_CUDA(c, cudaEventCreate(&e1));
-    for (int rep = 0; rep < 3; ++rep) {
-        cudaEventRecord(c->ev_probe, s);
-        cudaError_t e = launch_fp64_probe(static_cast<double*>(c->d_probe.p), iters, ctas, s);
-        if (e == cudaSuccess) e = cudaEventRecord(e1, s);
-        if (e == cudaSuccess) e = cudaEventSynchronize(e1);
-        if (e != cudaSuccess) { cudaEventDestroy(e1); return c->fail_cuda(e, "fp64 probe"); }
-        float ms = 0; cudaEventElapsedTime(&ms, c->ev_probe, e1);
-        best = std::max(best, (double)ctas * 256 * iters * 512.0 / (ms * 1e-3));
-    }
-    cudaEventDestroy(e1);
-    *lane_instr_per_s = best;
-    return PMM_OK;
+    double* sink = static_cast<double*>(c->d_probe.p);
+    return probe_rate(c, [&](int n) { return launch_fp64_probe(sink, n, ctas, c->stream); }, 5, iters,
+                      (double)ctas * 256 * iters * 512.0, lane_instr_per_s);
 }
 
 }  // extern "C"

@@ -9,7 +9,6 @@
 #include "pmm_plan.h"
 
 #include <algorithm>
-#include <atomic>
 #include <cstdio>
 #include <cstdlib>
 #include <numeric>
@@ -61,36 +60,20 @@ static Variant pick_variant_uncached(int R, int wmin)
 
 struct Group { Variant v; uint32_t region; uint32_t reads[kMaxGroups]; uint32_t n; };
 
-// Graded runs (plan_job): tasks per resident warp in each tier of run sizes (0 = runs of equal size, the round-1
-// behaviour), the share of a warp's launch one task may take (per cent), and the largest run.  Process-wide;
-// PMM_RUN_TIERS="depth,share,top" or set_run_tiers() for tuning sweeps.
-static std::atomic<int> g_widen{-1};
-bool small_job_widening()
+const PlanOptions& plan_defaults()
 {
-    int v = g_widen.load(std::memory_order_relaxed);
-    if (v < 0) { const char* e = std::getenv("PMM_SMALL_JOB_WIDENING"); v = e && *e ? (std::atoi(e) != 0) : 1; g_widen.store(v, std::memory_order_relaxed); }
-    return v != 0;
+    static const PlanOptions d = [] {
+        PlanOptions o;
+        if (const char* e = std::getenv("PMM_SMALL_JOB_WIDENING"); e && *e) o.widening = std::atoi(e) != 0;
+        if (const char* e = std::getenv("PMM_RUN_TIERS")) {
+            int depth = kRunTierDepth, share = kRunTierShare, top = kRunTierTop;
+            std::sscanf(e, "%d,%d,%d", &depth, &share, &top);
+            o.tiers = RunTiers{std::max(0, std::min(64, depth)), std::max(1, std::min(100, share)), std::max(1, std::min(64, top))};
+        }
+        return o;
+    }();
+    return d;
 }
-void set_small_job_widening(bool on) { g_widen.store(on ? 1 : 0, std::memory_order_relaxed); }
-
-static std::atomic<int> g_tiers{-1};                                    // depth | share << 8 | top << 16
-static int pack_tiers(int d, int share, int top)
-{
-    d = std::max(0, std::min(64, d)); share = std::max(1, std::min(100, share)); top = std::max(1, std::min(64, top));
-    return d | share << 8 | top << 16;
-}
-RunTiers run_tiers()
-{
-    int v = g_tiers.load(std::memory_order_relaxed);
-    if (v < 0) {
-        int d = kRunTierDepth, share = kRunTierShare, top = kRunTierTop;
-        if (const char* e = std::getenv("PMM_RUN_TIERS")) std::sscanf(e, "%d,%d,%d", &d, &share, &top);
-        v = pack_tiers(d, share, top);
-        g_tiers.store(v, std::memory_order_relaxed);
-    }
-    return RunTiers{v & 255, (v >> 8) & 255, (v >> 16) & 255};
-}
-void set_run_tiers(int depth, int share, int top) { g_tiers.store(pack_tiers(depth, share, top), std::memory_order_relaxed); }
 
 // Every variant present costs one kernel launch, and a launch is inefficient when it has few tasks: it lasts at
 // least as long as its longest task, and its tail leaves most of the GPU idle.  A mixed-length job (config 5: 10 % of
@@ -144,12 +127,11 @@ static void merge_rare_variants(std::vector<Group>& groups, const std::vector<Re
 }
 
 int plan_job(uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, const uint32_t* hap_off,
-             uint32_t num_region, const pmm_region_t* regions, int sm_count, int tasks_per_warp,
-             Plan& plan, std::string& err, const Variant* force, const std::function<Task*(const Plan&)>& task_dst)
+             uint32_t num_region, const pmm_region_t* regions, int sm_count, const PlanOptions& opt,
+             Plan& plan, std::string& err, const std::function<Task*(const Plan&)>& task_dst)
 {
     plan = Plan();
-    const bool keep_all_variants = force && force->K < 0;             // tuning sweeps: "-1,0" = no consolidation
-    if (keep_all_variants) force = nullptr;
+    const Variant* force = opt.force.K > 0 ? &opt.force : nullptr;
     if (!num_read || !num_hap || !num_region || !read_off || !hap_off || !regions) { err = "empty job"; return PMM_ERR_INVALID; }
     const uint64_t total_bases = (uint64_t)read_off[num_read] - read_off[0];
     const uint64_t total_hap = (uint64_t)hap_off[num_hap] - hap_off[0];
@@ -188,7 +170,7 @@ int plan_job(uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, cons
     // or a quarter as long and there are two or four times as many (a 10 x 5 toy region: float pass 85 -> ~30 us).  Wider
     // while the tasks still find at most two warps per SMSP.
     int wmin = 8;
-    if (!force && small_job_widening()) {
+    if (!force && opt.widening) {
         uint64_t t0 = 0;                                                // one-haplotype tasks with the default variants
         for (uint32_t g = 0; g < num_region; ++g) {
             const pmm_region_t& r = regions[g];
@@ -232,7 +214,7 @@ int plan_job(uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, cons
     // ---- runs of haplotypes: at least about tasks_per_warp queued tasks per resident warp (a bound that only jobs of more
     //      than ~38 000 group x haplotype units reach; below it the graded runs decide) --------------------------------
     const uint64_t resident_warps = (uint64_t)std::max(1, sm_count) * 16;
-    const uint64_t target_tasks = std::max<uint64_t>(1, resident_warps * (uint64_t)std::max(1, tasks_per_warp));
+    const uint64_t target_tasks = std::max<uint64_t>(1, resident_warps * (uint64_t)std::max(1, opt.tasks_per_warp));
     plan.haps_per_task = (uint32_t)std::max<uint64_t>(1, (group_haps + target_tasks - 1) / target_tasks);
     // Graded runs.  What a task pays once -- its row-parameter loads and weight table, the wavefront's fill and drain, the
     // checked steps at both ends -- is about 3 % of a one-haplotype task, so long runs are cheaper; but the launch's tail is
@@ -242,7 +224,7 @@ int plan_job(uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, cons
     // steady loop with one haplotype per task).  A job with fewer than depth tasks per warp keeps one haplotype per task.
     double f1 = 0.0, f2 = 0.0;
     uint32_t top = plan.haps_per_task;
-    const RunTiers tiers = run_tiers();
+    const RunTiers& tiers = opt.tiers;
     if (tiers.depth > 0 && group_haps > 0) {
         // resident warps of the launch most groups belong to (min_ctas<float, K> of pmm_kernels.cu x 4 warps)
         std::vector<uint32_t> by_k(kMaxK + 2, 0);
@@ -260,7 +242,7 @@ int plan_job(uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, cons
             top = std::max(top, cap);
         }
     }
-    if (!force && !keep_all_variants)
+    if (!force && !opt.keep_all_variants)
         merge_rare_variants(groups, plan.regions, hap_off, sm_count, top * (plan.max_hap_len + 1));
 
     // launches ordered by variant (largest footprint first); stable within a variant

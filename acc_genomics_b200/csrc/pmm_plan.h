@@ -32,13 +32,21 @@ inline double step_cost(int K) { return 12.25 * K + 9.0; }
 // longer than `share` per cent of a warp's steps in the launch; at most `top` haplotypes per run.
 struct RunTiers { int depth, share, top; };
 constexpr int kRunTierDepth = 2, kRunTierShare = 40, kRunTierTop = 4;
-RunTiers run_tiers();
-void set_run_tiers(int depth, int share, int top);
 
-// Small jobs (fewer one-haplotype tasks than two warps per SMSP could take after widening) get more lanes per read, i.e.
-// shorter and more tasks; process-wide switch for tuning (PMM_SMALL_JOB_WIDENING=0).
-bool small_job_widening();
-void set_small_job_widening(bool on);
+// How plan_job cuts a job.  Each engine context owns one (pmm_set_option); a new context and pmm_plan_flat start from
+// plan_defaults().
+struct PlanOptions {
+    // Small jobs (fewer one-haplotype tasks than two warps per SMSP could take after widening) get more lanes per read,
+    // i.e. shorter and more tasks.
+    bool widening = true;
+    RunTiers tiers{kRunTierDepth, kRunTierShare, kRunTierTop};
+    int tasks_per_warp = 16;            // queue depth per resident warp
+    Variant force{0, 0, false};         // tuning sweeps: K > 0 = this variant for every read that fits it
+    bool keep_all_variants = false;     // tuning sweeps: every variant a launch of its own (no consolidation of rare ones)
+};
+
+// The defaults, with PMM_SMALL_JOB_WIDENING=0|1 and PMM_RUN_TIERS="depth[,share[,top]]" applied (read once per process).
+const PlanOptions& plan_defaults();
 
 // Best (K, W) for a read of R bases; pick_variant_wide: among the variants with at least wmin lanes per read.
 Variant pick_variant(int R);
@@ -46,8 +54,8 @@ Variant pick_variant_wide(int R, int wmin);
 
 // Returns PMM_OK or PMM_ERR_INVALID with a message.
 int plan_job(uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, const uint32_t* hap_off,
-             uint32_t num_region, const pmm_region_t* regions, int sm_count, int tasks_per_warp,
-             Plan& plan, std::string& err, const Variant* force = nullptr,   // force: tuning sweeps only
+             uint32_t num_region, const pmm_region_t* regions, int sm_count, const PlanOptions& opt,
+             Plan& plan, std::string& err,
              // called once the task count (plan.num_tasks), groups and launches are known; returns where to write the tasks
              const std::function<Task*(const Plan&)>& task_dst = nullptr);
 

@@ -2,6 +2,8 @@
 // pairs first, one kernel launch per chunk, results back.  Stands where the reference has its per-pair CPU loop
 // (/root/reference/htc-sw/host/FalconSW_AVX.cpp:304-313) and the FPGA dispatch (host/sw_host.cpp:13-15).  No CPU path.
 #include "../../include/smithwaterman_cuda.h"
+#include "cuda_util.h"
+#include "host_workers.h"
 #include "sw_kernels.cuh"
 
 #include <algorithm>
@@ -9,32 +11,14 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <functional>
 #include <numeric>
 #include <string>
 #include <vector>
 
 using namespace sw;
 
-// host worker threads shared with the PairHMM engine (pmm_engine.cu)
-namespace pmm { void host_parallel_for(uint64_t n, uint64_t grain, const std::function<void(uint64_t, uint64_t)>& f); }
-
 namespace {
 std::string g_sw_create_error;
-
-struct Buf {
-    void* p = nullptr; size_t cap = 0; bool pinned = false;
-    cudaError_t reserve(size_t n)
-    {
-        if (n <= cap) return cudaSuccess;
-        release();
-        size_t want = std::max(n, (size_t)4096); want += want / 4;
-        cudaError_t e = pinned ? cudaMallocHost(&p, want) : cudaMalloc(&p, want);
-        if (e == cudaSuccess) cap = want; else p = nullptr;
-        return e;
-    }
-    void release() { if (p) { if (pinned) cudaFreeHost(p); else cudaFree(p); } p = nullptr; cap = 0; }
-};
 }  // namespace
 
 constexpr uint64_t kCigarScratchBytes = 256ull << 20;   // per-chunk scratch rows of the traceback (cigar_cap elements per pair)
@@ -44,12 +28,11 @@ struct sw_ctx {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev[2] = {nullptr, nullptr};
     std::string err;
-    Buf d_seq1, d_seq2, d_pairs, d_bt, d_cigars, d_compact, d_first, d_nelem, d_off, d_score, d_counter;
-    Buf h_stage, h_out, h_cig;
+    DevBuf d_seq1, d_seq2, d_pairs, d_bt, d_cigars, d_compact, d_first, d_nelem, d_off, d_score, d_counter;
+    PinBuf h_stage, h_out, h_cig;
     uint64_t compact_hint = 16;                   // CIGAR elements per pair the compact array is sized for (grows on overflow)
     uint64_t bt_budget_words = (1ull << 30);      // 4 GiB of backtrack codes per chunk
     sw_stats_t stats{};
-    sw_ctx() { h_stage.pinned = true; h_out.pinned = true; h_cig.pinned = true; }
     int fail(int code, const std::string& m) { err = m; return code; }
     int fail_cuda(cudaError_t e, const char* what) { err = std::string(what) + ": " + cudaGetErrorString(e); return SW_ERR_CUDA; }
 };
@@ -62,23 +45,13 @@ int sw_create(int device, sw_ctx** out)
 {
     if (!out) return SW_ERR_INVALID;
     *out = nullptr;
-    int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) {
-        cudaGetLastError();
-        g_sw_create_error = "no CUDA device visible; the aligner has no CPU fallback";
-        return SW_ERR_NO_DEVICE;
-    }
-    if (device < 0 && cudaGetDevice(&device) != cudaSuccess) device = 0;
-    if (device >= n) { g_sw_create_error = "device index out of range"; return SW_ERR_INVALID; }
-    cudaDeviceProp prop;
-    cudaError_t e;
-    if ((e = cudaSetDevice(device)) != cudaSuccess || (e = cudaGetDeviceProperties(&prop, device)) != cudaSuccess) {
-        g_sw_create_error = cudaGetErrorString(e); return SW_ERR_CUDA;
-    }
-    if (prop.major != 10) { g_sw_create_error = std::string("kernels are built for sm_100a only; device is ") + prop.name; return SW_ERR_NO_DEVICE; }
+    int sm_count = 0;
+    const int rc = open_device<SW_ERR_INVALID, SW_ERR_CUDA, SW_ERR_NO_DEVICE>(device, sm_count, g_sw_create_error, "the aligner");
+    if (rc) return rc;
     sw_ctx* c = new sw_ctx();
-    c->device = device; c->sm_count = prop.multiProcessorCount;
-    if ((e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking)) != cudaSuccess) { g_sw_create_error = cudaGetErrorString(e); delete c; return SW_ERR_CUDA; }
+    c->device = device; c->sm_count = sm_count;
+    const cudaError_t e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
+    if (e != cudaSuccess) { g_sw_create_error = cudaGetErrorString(e); delete c; return SW_ERR_CUDA; }
     cudaEventCreate(&c->ev[0]); cudaEventCreate(&c->ev[1]);
     *out = c;
     return SW_OK;
@@ -89,7 +62,6 @@ void sw_destroy(sw_ctx* c)
     if (!c) return;
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->stream);
-    for (Buf* b : {&c->d_seq1, &c->d_seq2, &c->d_pairs, &c->d_bt, &c->d_cigars, &c->d_compact, &c->d_first, &c->d_nelem, &c->d_off, &c->d_score, &c->d_counter, &c->h_stage, &c->h_out, &c->h_cig}) b->release();
     cudaEventDestroy(c->ev[0]); cudaEventDestroy(c->ev[1]);
     cudaStreamDestroy(c->stream);
     delete c;

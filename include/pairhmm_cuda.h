@@ -76,12 +76,12 @@ int  pmm_device_count(void);
  *   "tasks_per_warp"  = target queue depth per resident warp used when cutting regions into warp-tasks
  *   "small_job_widening" = "on" (default): a job with fewer warp-tasks than the GPU can spread over its SMSPs gets 16 or 32
  *                       lanes per read instead of the variant that wastes the fewest issue slots -- shorter, more numerous
- *                       tasks, i.e. a shorter critical path for a per-region caller.  Process-wide
+ *                       tasks, i.e. a shorter critical path for a per-region caller.  For this context
  *   "run_tiers"       = "depth[,share[,top]]", graded runs: a region's haplotypes are cut into runs of decreasing size (long
  *                       runs first, so what a task pays once is paid rarely; one-haplotype tasks last, so the launch's tail
  *                       stays short): `depth` tasks per resident warp in each tier (default 2; 0 = runs of equal size), no
  *                       task longer than `share` per cent of a warp's steps in the launch (40), at most `top` haplotypes
- *                       per run (4).  Process-wide
+ *                       per run (4).  For this context
  *   "mode"            = "exact" (default): every multiply and add of the float pass is rounded on its own, results are
  *                       bit-identical to the reference's AVX code.  "fast": the float cell update is contracted to
  *                       4 FMUL + 4 FFMA per cell (12 -> 8 instructions); results agree with the reference to a few

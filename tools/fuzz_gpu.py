@@ -42,7 +42,7 @@ while time.time() - t0 < budget:
     it += 1
     regs = [rand_region() for _ in range(int(rng.integers(1, 5)))]
     # these jobs are small: with widening on they run on the 32- and 16-lane variants, off on the ones large jobs use
-    eng.set_option("small_job_widening", str(rng.choice(["on", "off"])))     # process-wide: the other entry points too
+    eng.set_option("small_job_widening", str(rng.choice(["on", "off"])))     # eng's own calls only, not the plugin's or the pool's
     want = [chk.batch(b, threads=8) for b in regs]
     pairs += sum(b.num_pairs for b in regs)
     # staged multi-region job, exact
