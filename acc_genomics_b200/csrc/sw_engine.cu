@@ -88,6 +88,9 @@ int sw_align_batch(sw_ctx* c, uint32_t n_pairs,
         return c->fail(SW_ERR_INVALID, "null argument");
     if (overhang_strategy < 0 || overhang_strategy > 3) return c->fail(SW_ERR_INVALID, "unknown overhang strategy");
     if (!cigar_cap) return c->fail(SW_ERR_INVALID, "cigar_cap must be positive");
+    // within this domain no score or tie-break difference of the fill can overflow (see cells() in sw_kernels.cu)
+    for (const int w : {w_match, w_mismatch, w_open, w_extend})
+        if (w < -kMaxWeight || w > kMaxWeight) return c->fail(SW_ERR_INVALID, "weight outside [-65536, 65536]");
     const auto t0 = std::chrono::steady_clock::now();
     static const bool trace = getenv("SW_TRACE") != nullptr;
     auto mark = [&](const char* what) { if (trace) fprintf(stderr, "[sw] %-10s %.3f ms\n", what, std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count()); };

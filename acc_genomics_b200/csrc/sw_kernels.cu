@@ -130,9 +130,13 @@ __device__ __forceinline__ void fill_matrix(const FillCtx& c)
             // with at most two register operands on the FMA pipe.  Each of the four tie-breaks of a cell is the sign of a
             // difference (a multiply-add by a -1 ptxas cannot see through), and one funnel shift both extracts that sign
             // and appends it to the row's code word: acc = (acc << 1) | (diff >> 31).  Eight steps fill a word, older
-            // codes fall off the top, nothing is ever reset or positioned.  (Differences cannot overflow:
-            // |values| <= 2^30 + 2^20.)  History: compare + select + multiply-add packing with a per-step flush test,
-            // 40 instructions per cell, 433 GCUPS; this form 24.
+            // codes fall off the top, nothing is ever reset or positioned.  Differences cannot overflow because the host
+            // accepts only |weight| <= 2^16 and lengths <= 4095: every H, E and F is the score of a path of at most
+            // 4095 + 4095 moves of one weight each (or the clamp, -10^8, in between), so |H|, |E|, |F| <= 8190 * 2^16
+            // < 2^29; the one other operand is E or F of the boundary plus extend, kLowInit + extend, within
+            // 2^30 + 2^16 of zero.  Every difference is then below 2^30 + 2^29 + 2^16 < 2^31 in magnitude.
+            // History: compare + select + multiply-add packing with a per-step flush test, 40 instructions per cell,
+            // 433 GCUPS; this form 24.
             auto cells = [&](const int j, const int c2, int upH, int upF) {
                 int diag = prev_up;
                 prev_up = upH;
@@ -416,7 +420,9 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, 3) sw_align_kernel(const Ar
                 a.compact_first[pd.index] = first;
                 a.n_elem[pd.index] = n;
                 a.offset[pd.index] = off;
-                if (a.score) a.score[pd.index] = best;
+                // the score of the cell the traceback starts from: INDEL always starts at (nrow, ncol), whatever the
+                // end-cell search found (for IGNORE the walk may move to the last row; its score stays the search's)
+                if (a.score) a.score[pd.index] = strategy == kIndel ? sm.lastcol[nrow] : best;
             }
         }
     }

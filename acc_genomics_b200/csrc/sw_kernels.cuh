@@ -19,6 +19,7 @@ namespace sw {
 
 constexpr int kWarpsPerCta = 4;
 constexpr int kMaxLen = 4095;
+constexpr int kMaxWeight = 1 << 16;      // |match|, |mismatch|, |open|, |extend| at most this (see cells() in sw_kernels.cu)
 
 struct PairDesc {
     uint32_t s1, l1, s2, l2;

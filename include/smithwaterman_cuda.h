@@ -50,12 +50,20 @@ const char* sw_last_error(const sw_ctx* ctx);     /* ctx may be NULL: last error
 /* Align n_pairs pairs.  Pair p is seq1_bytes[seq1_start[p] .. +seq1_len[p]) against seq2_bytes[seq2_start[p] .. +seq2_len[p])
  * (several pairs may name the same reference bytes).  Outputs, all caller-owned host memory:
  *   cigars[p * cigar_cap .. ]  the CIGAR elements of pair p in forward order, at most cigar_cap of them; only the first
- *                              min(n_elem[p], cigar_cap) elements of a row are written, the rest is left as it was
- *   n_elem[p]                  how many elements the CIGAR has (if > cigar_cap the stored CIGAR is truncated: retry larger)
+ *                              min(n_elem[p], cigar_cap) elements of a row are written, the rest is left as it was.
+ *                              When n_elem[p] > cigar_cap the row holds the LAST cigar_cap elements of the CIGAR, in
+ *                              forward order (the traceback runs from the end of the alignment): retry larger
+ *   n_elem[p]                  how many elements the CIGAR has
  *   alignment_offset[p]        the value runSWOnePairBT returns / SWPairwiseAlignmentOneBatch stores
- *   score[p]                   (optional, may be NULL) score of the end cell
+ *   score[p]                   (optional, may be NULL) the score H of the cell where the traceback starts.  For SOFTCLIP,
+ *                              INDEL and LEADING_INDEL that is the score of the returned alignment: match / mismatch per
+ *                              M base, open + (L - 1) * extend per I or D element of length L, 0 per S base (exact
+ *                              unless the -10^8 clamp below acts, or open > extend lets two gaps touch and merge into
+ *                              one element).  For IGNORE it is the score of the end cell the search found
  * Weights are the reference's W_MATCH, W_MISMATCH, W_OPEN, W_EXTEND (host/common.h:15-18: 200, -150, -260, -11 by default
- * in GATK); limits: each sequence at most 4095 bases. */
+ * in GATK), each within [-65536, 65536] (else SW_ERR_INVALID): then no score can overflow 32 bits.  Any sign is accepted.
+ * Limits: each sequence at most 4095 bases.  Like the reference, the diagonal term of the recurrence is clamped at
+ * -10^8 (MATRIX_MIN_CUTOFF); within the weight domain that clamp can act (e.g. mismatch <= -24415 at 4095 bases). */
 int  sw_align_batch(sw_ctx* ctx, uint32_t n_pairs,
                     const uint8_t* seq1_bytes, const uint32_t* seq1_start, const uint32_t* seq1_len,
                     const uint8_t* seq2_bytes, const uint32_t* seq2_start, const uint32_t* seq2_len,

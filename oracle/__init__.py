@@ -119,7 +119,7 @@ def reference(fma: bool = False) -> _Lib | None:
 # ---- Smith-Waterman (SURVEY.md section 8f row 4) ------------------------------------------------------------------
 SW_SOFTCLIP, SW_INDEL, SW_LEADING_INDEL, SW_IGNORE = 0, 1, 2, 3
 SW_WEIGHTS = (200, -150, -260, -11)        # W_MATCH, W_MISMATCH, W_OPEN, W_EXTEND (htc-sw/host/common.h:15-18)
-_CIGAR_CAP = 4096
+_CIGAR_CAP = 8192                          # the most elements a CIGAR of two 4095-base sequences can have
 
 
 class _SwLib:
@@ -148,12 +148,19 @@ class _SwLib:
         if self.kind != "port" and (len(ref) > 1536 or len(alt) > 1536):
             raise ValueError("the reference's Smith-Waterman has fixed 1536-base buffers (MAX_SEQ_LEN); use sw_port()")
         if self.kind == "port":
-            sc = C.c_int()
-            off = self.lib.sw_oracle_align(*weights, ref, len(ref), alt, len(alt), strategy, self._len, self._st, _CIGAR_CAP,
-                                           C.byref(n), C.byref(sc))
-        else:
-            off = self.lib.ref_sw_gkl(*weights, ref, len(ref), alt, len(alt), strategy, self._len, self._st, _CIGAR_CAP, C.byref(n))
+            return self.align_scored(ref, alt, strategy, weights)[:2]
+        off = self.lib.ref_sw_gkl(*weights, ref, len(ref), alt, len(alt), strategy, self._len, self._st, _CIGAR_CAP, C.byref(n))
         return off, [(self._len[k], self._st[k]) for k in range(n.value)]
+
+    def align_scored(self, ref: bytes, alt: bytes, strategy: int, weights=SW_WEIGHTS):
+        """(offset, cigar, score): score is H of the cell the traceback starts from.  The C restatement only: the
+        reference's runSWOnePairBT returns no score."""
+        if self.kind != "port":
+            raise ValueError("only the C restatement reports a score; use sw_port()")
+        n, sc = C.c_int(), C.c_int()
+        off = self.lib.sw_oracle_align(*weights, ref, len(ref), alt, len(alt), strategy, self._len, self._st, _CIGAR_CAP,
+                                       C.byref(n), C.byref(sc))
+        return off, [(self._len[k], self._st[k]) for k in range(n.value)], sc.value
 
     def align_falcon(self, ref: bytes, alt: bytes, strategy: int, option: int = 1):
         """Falcon's own SWPairwiseAlignmentOneBatch (fixed weights); option 1 = scalar baseline, 0 = its SIMD variant."""
@@ -161,6 +168,27 @@ class _SwLib:
         off = self.lib.ref_sw_falcon(ref, len(ref), alt, len(alt), strategy, option, self._len, self._st, _CIGAR_CAP,
                                      C.byref(n), C.byref(rc))
         return rc.value, off, [(self._len[k], self._st[k]) for k in range(n.value)]
+
+
+def sw_rescore(ref: bytes, alt: bytes, weights, offset: int, cigar) -> int:
+    """The score of an alignment given by its offset and CIGAR: match / mismatch per M base, open + (L - 1) * extend per
+    I or D element of length L, nothing for S."""
+    match, mismatch, open_, extend = weights
+    i, j, s = offset, 0, 0
+    for n, st in cigar:
+        if st == 0:
+            s += sum(match if ref[i + k] == alt[j + k] else mismatch for k in range(n))
+            i += n; j += n
+        elif st in (1, 2):
+            s += open_ + (n - 1) * extend
+            i, j = (i, j + n) if st == 1 else (i + n, j)
+        else:
+            if st != 4:
+                raise ValueError(f"CIGAR state {st}")
+            j += n
+    if j != len(alt) or i > len(ref):
+        raise ValueError("the CIGAR does not fit the sequences")
+    return s
 
 
 def sw_port() -> "_SwLib":

@@ -8,7 +8,8 @@
  * matters and is reproduced here (anti-diagonal by anti-diagonal, last row before last column).
  *
  * seq1 = reference (rows, index i), seq2 = alternate (columns, index j).  Cigar states: 0 M, 1 I, 2 D, 4 S
- * (host/common.h:20-23).  Returns the alignment offset; the cigar comes out in forward order as (length, state) pairs.
+ * (host/common.h:20-23).  Returns the alignment offset; the cigar comes out in forward order as (length, state) pairs,
+ * and *score_out is H of the cell the traceback starts from (for IGNORE: the end cell of the search).
  */
 #include <limits.h>
 #include <stdint.h>
@@ -76,7 +77,8 @@ int sw_oracle_align(int match, int mismatch, int open, int extend, const uint8_t
             }
         }
     }
-    if (score_out) *score_out = max_score;
+    /* the score of the cell the traceback starts from (INDEL: the corner, whatever the search found) */
+    if (score_out) *score_out = strategy == STRAT_INDEL ? H[nrow * W + ncol] : max_score;
 
     /* traceback (getCIGAR, :275-437) */
     int* ops = (int*)malloc(sizeof(int) * 2 * (size_t)(nrow + ncol + 4));

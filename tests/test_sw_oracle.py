@@ -49,6 +49,25 @@ def test_port_equals_reference_live(built):
             assert rc != 0 or (off, cig) == port.align(r, a, st)
 
 
+# opening at least as expensive as extending (else two touching gaps merge into one element) and far from the -10^8 clamp
+RESCORE_WEIGHTS = [(200, -150, -260, -11), (3, -1, -4, -3), (25, -50, -110, -6), (10, -15, -30, -5)]
+
+
+@pytest.mark.parametrize("strategy", [oracle.SW_SOFTCLIP, oracle.SW_INDEL, oracle.SW_LEADING_INDEL])
+def test_port_score_is_the_score_of_its_alignment(built, strategy):
+    """For SOFTCLIP, INDEL and LEADING_INDEL the reported score is the score of the returned alignment, recomputed from the
+    sequences, weights, offset and CIGAR.  (INDEL starts its traceback at the corner, not at the end cell of the search.)"""
+    port = oracle.sw_port()
+    pairs = sw.haplotype_pairs(11, 60, ref_len=(20, 160), per_ref=6, sub=0.05, indel=0.04)
+    pairs += [(b"A" * 60, b"A" * 37), (b"AC" * 40, b"AC" * 31 + b"A"), (b"ACG" * 30, b"ACG" * 12 + b"T" + b"ACG" * 10),
+              (b"C" * 9, b"G" * 9), (b"ACGT" * 25, b"TGCA" * 25), (b"A" * 200 + b"C" * 50, b"C" * 50 + b"A" * 200),
+              (b"ACGTTGCA" * 4, b"TTGCA"), (b"G", b"GATTACA"), (b"GATTACA", b"T")]
+    for w in RESCORE_WEIGHTS:
+        for r, a in pairs:
+            off, cig, score = port.align_scored(r, a, strategy, w)
+            assert oracle.sw_rescore(r, a, w, off, cig) == score, (w, r, a, sw.cigar_string(cig), off, score)
+
+
 def test_library_exports_the_sw_abi(built):
     import re
     from acc_genomics_b200 import engine

@@ -14,7 +14,8 @@ budget = float(sys.argv[1]) if len(sys.argv) > 1 else 60.0
 seed = int(sys.argv[2]) if len(sys.argv) > 2 else 1
 rng = np.random.Generator(np.random.PCG64(seed))
 chk = oracle.reference() or oracle.port()
-swchk = oracle.sw_reference() or oracle.sw_port()
+swport = oracle.sw_port()
+swchk = oracle.sw_reference() or swport
 eng = PairHMMEngine(0); fast = PairHMMEngine(0); fast.set_option("mode", "fast")
 pool = PairHMMPool(devices=[0], contexts_per_device=2); pool.set_merge(True)
 al = sw.SmithWaterman(0)
@@ -85,9 +86,27 @@ while time.time() - t0 < budget:
     ps = sw.haplotype_pairs(int(rng.integers(1 << 30)), n, ref_len=(lo, lo + int(rng.integers(0, 300))), per_ref=int(rng.integers(1, 9)),
                             sub=float(rng.choice([0.0, 0.03, 0.2])), indel=float(rng.choice([0.0, 0.01, 0.05])))
     st = int(rng.integers(0, 4))
-    got = al.align(ps, st, cigar_cap=int(rng.choice([2, 16, 64])))
-    for (r, a), (off, cig, _) in zip(ps, got):
-        assert (off, cig) == swchk.align(r, a, st), ("sw", it, st, len(r), len(a))
-    swpairs += n
+    # weights: GATK's default, small random ones, or anywhere in the accepted domain [-2^16, 2^16] (where the -10^8 clamp
+    # can act on long pairs); bytes beyond ACGT: N, lowercase, any byte
+    wkind = int(rng.integers(0, 3))
+    if wkind == 0:   w = sw.DEFAULT_WEIGHTS
+    elif wkind == 1: w = tuple(int(x) for x in rng.integers(-30, 31, 4))
+    else:            w = tuple(int(x) for x in rng.integers(-(1 << 16), (1 << 16) + 1, 4))
+    if wkind == 2 and rng.random() < 0.3:
+        # a long pair and a steep mismatch: the chunk runs the kernel with the clamp, which may act
+        w = (w[0], -int(rng.integers(60000, (1 << 16) + 1)), w[2], w[3])
+        L = int(rng.integers(1700, 4096))
+        r = bytes(rng.choice(np.frombuffer(b"ACGT", np.uint8), L))
+        ps.append((r, bytes(rng.choice(np.frombuffer(b"ACGT", np.uint8), int(rng.integers(1, L + 1))))))
+    if rng.random() < 0.3:
+        ps = [(r, bytes(x if rng.random() > 0.05 else int(rng.choice([78, 110, 97, 0, 255, int(rng.integers(0, 256))])) for x in a))
+              for r, a in ps]
+    got = al.align(ps, st, w, cigar_cap=int(rng.choice([2, 16, 64])))
+    for (r, a), (off, cig, score) in zip(ps, got):
+        sw_want = swport.align_scored(r, a, st, w)
+        assert (off, cig, score) == sw_want, ("sw", it, st, w, len(r), len(a))
+        if swchk is not swport and len(r) <= 1536 and len(a) <= 1536:
+            assert (off, cig) == swchk.align(r, a, st, w), ("sw reference", it, st, w, len(r), len(a))
+    swpairs += len(ps)
 print(f"fuzz ok: {it} iterations, {pairs} PairHMM pairs, {swpairs} Smith-Waterman pairs, {time.time() - t0:.0f} s, seed {seed}, "
       f"checkers {chk.kind}/{swchk.kind}")
