@@ -302,9 +302,9 @@ int stage(pmm_ctx* c, const JobSource& src)
     // carry rows of the striped kernels: one haplotype (+2 separators) per warp, three rows of doubles
     {
         int ctas64 = 1;
-        for (int k : {4, 5, 6, 8}) ctas64 = std::max(ctas64, forward_f64_ctas_per_sm(k, true));
-        const int ctas32 = std::max(std::max(forward_f32_ctas_per_sm(kStripedK, 32, true, false), forward_f32_ctas_per_sm(kStripedK, 32, true, true)),
-                                    recheck_f32_ctas_per_sm());
+        for (int k : kF64Rows) ctas64 = std::max(ctas64, forward_f64_variant(k, true)->ctas_per_sm());
+        const int ctas32 = std::max({forward_f32_variant(kStripedK, 32, true, false)->ctas_per_sm(),
+                                     forward_f32_variant(kStripedK, 32, true, true)->ctas_per_sm(), recheck_f32_variant().ctas_per_sm()});
         // the float and the double kernel of neighbouring launches can be on the GPU together: a scratch of their own each
         PMM_CUDA(c, c->d_scratch.reserve((size_t)c->sm_count * ctas32 * kWarpsPerCta * 3 * (size_t)(job.max_hap_len + 8) * sizeof(float)));
         PMM_CUDA(c, c->d_scratch64.reserve((size_t)c->sm_count * ctas64 * kWarpsPerCta * 3 * (size_t)(job.max_hap_len + 8) * sizeof(double)));
@@ -767,10 +767,11 @@ int pmm_launch(pmm_ctx* c)
         a.ntasks = seg.task_count; a.ntasks_dev = nullptr;
         a.counter = ctrl + cursor; cursor += 32;
         a.out = R.d_raw.p;
-        const int per_sm = forward_f32_ctas_per_sm(seg.v.K, seg.v.W, seg.v.striped, c->fast);
+        const ForwardKernel* fk = forward_f32_variant(seg.v.K, seg.v.W, seg.v.striped, c->fast);
+        const int per_sm = fk ? fk->ctas_per_sm() : 0;
         if (per_sm <= 0) return c->fail(PMM_ERR_INVALID, "kernel variant unavailable");
         const int ctas = (int)std::min<uint64_t>((seg.task_count + kWarpsPerCta - 1) / kWarpsPerCta, (uint64_t)c->sm_count * per_sm);
-        PMM_CUDA(c, launch_forward_f32(seg.v.K, seg.v.W, seg.v.striped, c->fast, a, fq, ctas, s));
+        PMM_CUDA(c, fk->launch(a, fq, ctas, s));
         ++launches;
     }
     if (c->fast) {
@@ -778,7 +779,7 @@ int pmm_launch(pmm_ctx* c)
         a.tasks = static_cast<Task*>(c->d_tiny_tasks.p); a.ntasks = 0; a.ntasks_dev = ctrl + 2;
         a.counter = ctrl + cursor; cursor += 32;
         fq.lo = fq.hi = thr;
-        PMM_CUDA(c, launch_recheck_f32(a, fq, c->sm_count * std::max(1, recheck_f32_ctas_per_sm()), s));
+        PMM_CUDA(c, recheck_f32_variant().launch(a, fq, c->sm_count * std::max(1, recheck_f32_variant().ctas_per_sm()), s));
         ++launches;
     }
     PMM_CUDA(c, cudaEventRecord(R.ev[1], s));
@@ -793,8 +794,8 @@ int pmm_launch(pmm_ctx* c)
     //      of a read together; their number is only known on the device.  On its own stream: the next launch's float pass
     //      (this stream) starts as soon as this one's is over and runs next to it ------------------------------------------
     PMM_CUDA(c, cudaStreamWaitEvent(sd, R.ev[1], 0));
-    const int KD = j.f64_rows;
-    const int f64_ctas = c->sm_count * std::max(1, forward_f64_ctas_per_sm(KD, j.f64_striped));
+    const ForwardKernel* dk = forward_f64_variant(j.f64_rows, j.f64_striped);      // one of kF64Rows: never null
+    const int f64_ctas = c->sm_count * std::max(1, dk->ctas_per_sm());
     FallbackBuild fb{};
     fb.raw = static_cast<float*>(R.d_raw.p);
     fb.regions = section<RegionDesc>(c->d_in.p, j.at.regions);
@@ -809,7 +810,7 @@ int pmm_launch(pmm_ctx* c)
     fb.spos = a.spos;
     fb.max_hap_len = j.max_hap_len;
     fb.capacity = (uint32_t)j.pairs;
-    fb.single_stripe_rows = 32u * (uint32_t)KD;
+    fb.single_stripe_rows = 32u * (uint32_t)j.f64_rows;
     fb.target_tasks = (uint32_t)(f64_ctas * kWarpsPerCta * c->f64_tasks_per_warp);
     fb.max_run = (uint32_t)c->f64_max_run;
     PMM_CUDA(c, launch_build_fallback(fb, c->sm_count, sd));
@@ -818,7 +819,7 @@ int pmm_launch(pmm_ctx* c)
     a.ntasks = 0; a.ntasks_dev = ctrl + 3; a.counter = ctrl + cursor; cursor += 32;
     a.tiny_threshold = ldexp(1.0, -800); a.tiny_count = ctrl + 1;
     a.scratch = c->d_scratch64.p;
-    PMM_CUDA(c, launch_forward_f64(KD, j.f64_striped, a, f64_ctas, sd));
+    PMM_CUDA(c, dk->launch(a, FallbackQueue{}, f64_ctas, sd));
     ++launches;
     PMM_CUDA(c, cudaEventRecord(R.ev[2], sd));
     // What is queued on the launch stream from here on (the next launch, an event of the caller's) comes after the

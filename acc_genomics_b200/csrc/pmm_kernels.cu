@@ -36,16 +36,10 @@
 namespace pmm {
 namespace {
 
-#ifndef PMM_STEADY_UNROLL
-#define PMM_STEADY_UNROLL 4
-#endif
-constexpr int kSteadyUnrollF32 = PMM_STEADY_UNROLL;  // steps per trip of the branch-free loop
+constexpr int kSteadyUnrollF32 = 4;            // steps per trip of the branch-free loop
 // the double kernel is bound by the latency of its dependent DP chains, not by issue slots: a longer trip gives ptxas
 // more independent work to put between them (measured on config 3: 2 steps 2.36 ms, 4 steps 2.30, 8 steps 2.28)
-#ifndef PMM_STEADY_UNROLL_F64
-#define PMM_STEADY_UNROLL_F64 8
-#endif
-constexpr int kSteadyUnrollF64 = PMM_STEADY_UNROLL_F64;
+constexpr int kSteadyUnrollF64 = 8;
 
 __device__ __forceinline__ int base_class(unsigned ch)
 {
@@ -86,63 +80,12 @@ template <bool FLUSH> __device__ __forceinline__ float flush(float x) { return x
 
 template <typename T> __device__ __forceinline__ T ld_cg(const T* p) { return __ldcg(p); }
 
-// ---- TMA bulk copy (cp.async.bulk, global -> shared) completing on an mbarrier: how a warp stages its task's match-weight
-//      tile.  One lane issues the copy; every lane that is to read the tile waits for the barrier's phase. ----------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-[[maybe_unused]] __device__ __forceinline__ void mbar_init(uint64_t* mbar, uint32_t arrivals)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(mbar)), "r"(arrivals) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-[[maybe_unused]] __device__ __forceinline__ void bulk_copy_g2s(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* mbar)
-{
-    // the tile's previous contents were read through the generic proxy; the copy writes through the async proxy
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(mbar)), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 :: "r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(mbar)) : "memory");
-}
-// The same tile by cp.async (LDGSTS): every lane copies 16 bytes per instruction, global -> shared without a register.
-[[maybe_unused]] __device__ __forceinline__ void cp_async_16(void* dst_smem, const void* src_gmem)
-{
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"(smem_u32(dst_smem)), "l"(src_gmem) : "memory");
-}
-[[maybe_unused]] __device__ __forceinline__ void cp_async_wait_all()
-{
-    asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
-}
-[[maybe_unused]] __device__ __forceinline__ void mbar_wait(uint64_t* mbar, uint32_t phase)
-{
-    asm volatile("{\n\t.reg .pred p;\n\tWAIT_%=:\n\t"
-                 "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-                 "@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}"
-                 :: "r"(smem_u32(mbar)), "r"(phase) : "memory");
-}
-
 template <typename T, int K>
 __host__ __device__ constexpr int wtab_elems() { return 5 * ((K + Arith<T>::kVec - 1) / Arith<T>::kVec) * 32 * Arith<T>::kVec; }
 
 // ---------------------------------------------------------------------------------------------------------
 // The forward kernel.
 // ---------------------------------------------------------------------------------------------------------
-// Resident CTAs (of four warps) per SM the register allocator must leave room for: the state of a lane is 8 registers per row
-// (5 parameters + M, X, Y), so K decides the occupancy step (64K registers / 128 threads).
-// Measured (tools/occ_check.py): 15 and 16 rows per lane at two CTAs per SM (up to 255 registers) beat three CTAs at 168
-// registers by 5.6 % (config 4, K = 16 / W = 16: 2 343 -> 2 475 GCUPS); for K <= 14 the difference is within 2 %.
-template <typename T, int K> __host__ __device__ constexpr int min_ctas()
-{
-#ifndef PMM_F32_4CTA_MAXK
-#define PMM_F32_4CTA_MAXK 11
-#endif
-#ifndef PMM_F32_3CTA_MAXK
-#define PMM_F32_3CTA_MAXK 14
-#endif
-#ifndef PMM_F64_4CTA_MAXK
-#define PMM_F64_4CTA_MAXK 0
-#endif
-    return sizeof(T) == 8 ? (K <= PMM_F64_4CTA_MAXK ? 4 : K <= 6 ? 3 : 2) : K <= PMM_F32_4CTA_MAXK ? 4 : K <= PMM_F32_3CTA_MAXK ? 3 : 2;
-}
-
 // ---- fallback count: the float pass counts the pairs whose result is below 1e-28f the moment the result exists ----
 // (Tried and measured on B200, see DESIGN.md section 4.5: *consuming* a fallback list inside the float kernel, so that the
 // double re-run overlaps the float pass, is slower than a separate double launch -- the two loop bodies evict each
@@ -186,22 +129,21 @@ constexpr int kRetry = 16;
 // one haplotype into the next; a lane re-points its stream pointer when it crosses a separator.
 constexpr int kList = 32;
 
-static_assert(!kTileCopy || (wtab_floats(19) == (uint32_t)wtab_elems<float, 19>() && wtab_floats(4) == (uint32_t)wtab_elems<float, 4>() &&
-                             wtab_floats(10) == (uint32_t)wtab_elems<float, 10>()), "the planner's tile size is the kernel's table size");
-
-// Builds with PMM_TILE_COPY != 0 (pmm_types.h): the float pass of one-stripe reads takes its weight table ready-made from
-// read_params_kernel's tile and stages it by cp.async (1: 16 bytes per lane and instruction) or by one TMA bulk copy per task
-// (2: cp.async.bulk + mbarrier).  Both are parity-green and both measured slower than building the table in the kernel from
-// three planes (config 2 float pass 1.775 ms; cp.async 1.787; TMA 1.795 -- its latency is the longest, and a task's first
-// step needs the table), so the default build keeps the in-kernel build.
-template <typename T, bool STRIPED, int F> __host__ __device__ constexpr bool tile_staged()
+// A row's entries in the five class tables of a lane's weight table (w: the row's entry of class 0): the match weight
+// where the haplotype class equals the read's base class or either is N (class 4), the mismatch weight elsewhere.
+template <typename T, int CLS_STRIDE>
+__device__ __forceinline__ void scatter_weights(T* w, unsigned cls, T mw, T xw)
 {
-    return kTileCopy != 0 && sizeof(T) == 4 && !STRIPED && (F & 8 /* kInline */) == 0;
+    #pragma unroll
+    for (int h = 0; h < 5; ++h) {
+        const bool match = (cls == (unsigned)h) || cls == 4 || h == 4;
+        w[h * CLS_STRIDE] = match ? mw : xw;
+    }
 }
 
 template <typename T, int K, int W, bool STRIPED, int F>
 __device__ __forceinline__ void run_task(const ForwardArgs& a, const Task* tk, T* wtab, const int lane,
-                                         const uint32_t gwarp, const FallbackQueue& fq, uint64_t* mbar, uint32_t& phase)
+                                         const uint32_t gwarp, const FallbackQueue& fq)
 {
     using A = Arith<T>;
     constexpr bool FLUSH = (F & kFlush) != 0, PUSH = (F & kPush) != 0, FAST = (F & kFast) != 0, INLINE = (F & kInline) != 0;
@@ -258,36 +200,8 @@ __device__ __forceinline__ void run_task(const ForwardArgs& a, const Task* tk, T
         T pX0 = (T)0;                                                // pC[0] as the X update of row 0 sees it
         unsigned padmask = 0;
         __syncwarp();                                                // previous task / stripe done with wtab
-        if constexpr (tile_staged<T, STRIPED, F>()) {
-            // float pass, one stripe: read_params_kernel left the group's weight tile in the layout of wtab; lane 0 has the
-            // TMA unit copy it (12.8 KB for K = 19) while all lanes load their 5 K transition parameters -- W consecutive
-            // lanes read consecutive floats, all loads independent -- and everyone waits for the tile's barrier phase.
-            constexpr int KW = K * W;
-            constexpr uint32_t kTileBytes = (uint32_t)wtab_elems<float, K>() * (uint32_t)sizeof(float);   // == wtab_floats(K)
-            const float* gb = a.params + tk->param_off;
-            const float* gtile = gb + (size_t)kParamPlanes * 32 * K;
-            if constexpr (kTileCopy == 2) {
-                if (lane == 0) bulk_copy_g2s(wtab, gtile, kTileBytes, mbar);
-            } else {
-                #pragma unroll
-                for (uint32_t o = 0; o < kTileBytes; o += 512)
-                    cp_async_16(reinterpret_cast<char*>(wtab) + o + lane * 16, reinterpret_cast<const char*>(gtile) + o + lane * 16);
-            }
-            const float* pb = gb + (size_t)g * (kParamPlanes * KW) + l;
-            #pragma unroll
-            for (int j = 0; j < K; ++j) {
-                const float* pj = pb + j * W;
-                pMM[j] = __ldg(pj + 0 * KW); pG[j] = __ldg(pj + 1 * KW); pMX[j] = __ldg(pj + 2 * KW);
-                pMY[j] = __ldg(pj + 3 * KW); pC[j] = __ldg(pj + 4 * KW);
-            }
-            // boundary rows: the rows above the read (all rows of an unused slot)
-            const int first = valid ? pad - l * K : K;                // rows j < first of this lane are boundary rows
-            padmask = first >= K ? (1u << K) - 1u : first > 0 ? (1u << first) - 1u : 0u;
-            pX0 = (padmask & 1u) ? 0.0f : pC[0];
-            if constexpr (kTileCopy == 2) { mbar_wait(mbar, phase); phase ^= 1u; }
-            else { cp_async_wait_all(); __syncwarp(); }
-        } else if constexpr (kIsFloat && !INLINE) {
-            // striped float pass: the rows were prepared once per read by read_params_kernel; W consecutive lanes read
+        if constexpr (kIsFloat && !INLINE) {
+            // float pass: the rows were prepared once per read by read_params_kernel; W consecutive lanes read
             // consecutive floats, all 8K loads are independent
             constexpr int KW = K * W;
             const float* pb = a.params + tk->param_off + ((size_t)(STRIPED ? 0 : g) * nstripes + stripe) * (kParamPlanes * KW) + l;
@@ -300,11 +214,7 @@ __device__ __forceinline__ void run_task(const ForwardArgs& a, const Task* tk, T
                 const unsigned cls = __float_as_uint(__ldg(pj + 7 * KW));
                 if (cls == kPadClass) padmask |= 1u << j;
                 if (j == 0) pX0 = cls == kPadClass ? 0.0f : pC[0];
-                #pragma unroll
-                for (int h = 0; h < 5; ++h) {
-                    const bool match = (cls == (unsigned)h) || cls == 4 || h == 4;
-                    wlane[h * CLS_STRIDE + (j / VEC) * 32 * VEC + (j % VEC)] = match ? mw : xw;
-                }
+                scatter_weights<T, CLS_STRIDE>(wlane + (j / VEC) * 32 * VEC + (j % VEC), cls, mw, xw);
             }
         } else {
             #pragma unroll
@@ -313,6 +223,8 @@ __device__ __forceinline__ void run_task(const ForwardArgs& a, const Task* tk, T
                 T mw = (T)0, xw = (T)0;
                 int cls = 0;
                 if (r0 >= 0 && valid) {
+                    // the same derivation as read_params_kernel's (kept in two places: as one helper it changes the
+                    // SASS of the double kernels or of read_params_kernel)
                     const uint8_t* b = a.read_blob + rd.off + r0;
                     cls = base_class(b[0]);
                     const int q_ = b[rd.stride] & 127, i_ = b[2 * rd.stride] & 127;
@@ -334,11 +246,7 @@ __device__ __forceinline__ void run_task(const ForwardArgs& a, const Task* tk, T
                     pMM[j] = (T)0; pG[j] = (T)0; pMX[j] = (T)0; pMY[j] = (T)0; pC[j] = (T)1.0;
                     padmask |= 1u << j;
                 }
-                #pragma unroll
-                for (int h = 0; h < 5; ++h) {
-                    const bool match = (cls == h) || cls == 4 || h == 4;
-                    wlane[h * CLS_STRIDE + (j / VEC) * 32 * VEC + (j % VEC)] = match ? mw : xw;
-                }
+                scatter_weights<T, CLS_STRIDE>(wlane + (j / VEC) * 32 * VEC + (j % VEC), (unsigned)cls, mw, xw);
             }
         }
         __syncwarp();
@@ -542,17 +450,11 @@ __device__ __forceinline__ void run_task(const ForwardArgs& a, const Task* tk, T
 }
 
 template <typename T, int K, int W, bool STRIPED, int F>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, min_ctas<T, K>() * (4 / kWarpsPerCta)) pmm_forward_kernel(const ForwardArgs a, const FallbackQueue fq)
+__global__ void __launch_bounds__(kWarpsPerCta * 32, resident_ctas<T>(K)) pmm_forward_kernel(const ForwardArgs a, const FallbackQueue fq)
 {
     extern __shared__ uint4 smem_raw[];
-    __shared__ uint64_t tile_bar[kWarpsPerCta];                  // one transaction barrier per warp (weight tile by TMA)
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     T* wtab = reinterpret_cast<T*>(smem_raw) + warp * wtab_elems<T, K>();
-    uint32_t phase = 0;
-    if constexpr (tile_staged<T, STRIPED, F>() && kTileCopy == 2) {
-        if (lane == 0) mbar_init(&tile_bar[warp], 1);
-        __syncwarp();
-    }
     const uint32_t ntasks = a.ntasks_dev ? *a.ntasks_dev : a.ntasks;
     const uint32_t gwarp = blockIdx.x * kWarpsPerCta + warp;
     for (;;) {
@@ -560,7 +462,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, min_ctas<T, K>() * (4 / kWa
         if (lane == 0) ti = atomicAdd(a.counter, 1u);
         ti = __shfl_sync(0xffffffffu, ti, 0);
         if (ti >= ntasks) break;
-        run_task<T, K, W, STRIPED, F & ~kRetry>(a, a.tasks + ti, wtab, lane, gwarp, fq, &tile_bar[warp], phase);
+        run_task<T, K, W, STRIPED, F & ~kRetry>(a, a.tasks + ti, wtab, lane, gwarp, fq);
         if constexpr ((F & kRetry) != 0) {
             // Intermediate products below DBL_MIN are flushed to zero on the reference's x86 (FTZ on); they can only
             // influence results that are themselves tiny.  Everything below tiny_threshold (2^-800, scaled by 2^1020) is
@@ -579,7 +481,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, min_ctas<T, K>() * (4 / kWa
                     Task one = tk;
                     one.hap_first = tk.hap_first + n; one.nhaps = 1; one.out_base[0] = tk.out_base[0] + n;
                     if (lane == 0) atomicAdd(a.tiny_count, 1u);
-                    run_task<T, K, W, STRIPED, (F & ~kRetry) | kFlush>(a, &one, wtab, lane, gwarp, fq, &tile_bar[warp], phase);
+                    run_task<T, K, W, STRIPED, (F & ~kRetry) | kFlush>(a, &one, wtab, lane, gwarp, fq);
                 }
             }
         }
@@ -722,9 +624,6 @@ __global__ void __launch_bounds__(128) read_params_kernel(const uint8_t* __restr
     const GroupDesc gd = groups[blockIdx.x];
     const uint32_t K = gd.K, W = gd.W, KW = K * W, rows = gd.nstripes * KW;
     const uint32_t slots = gd.nstripes > 1 ? 1u : 32u / W;
-    // one-stripe groups: the weight tile behind the planes (pmm_types.h), staged by the forward kernel with one bulk copy
-    float* tile = (gd.nstripes > 1 || !kTileCopy) ? nullptr : params + gd.param_off + (size_t)kParamPlanes * 32 * K;
-    const uint32_t cls_stride = ((K + 3) / 4) * 128;
     for (uint32_t slot = 0; slot < slots; ++slot) {
         const bool valid = slot < gd.nreads;
         ReadDesc rd = {0u, 0u, 0u};
@@ -753,15 +652,6 @@ __global__ void __launch_bounds__(128) read_params_kernel(const uint8_t* __restr
             float* o = base + (size_t)s * kParamPlanes * KW + idx;
             #pragma unroll
             for (int p = 0; p < kParamPlanes; ++p) o[(size_t)p * KW] = v[p];
-            if (tile) {
-                const unsigned cls = __float_as_uint(v[7]);
-                float* t = tile + (j / 4) * 128 + (slot * W + l) * 4 + (j % 4);
-                #pragma unroll
-                for (int h = 0; h < 5; ++h) {
-                    const bool match = (cls == (unsigned)h) || cls == 4 || h == 4;
-                    t[h * cls_stride] = match ? v[5] : v[6];
-                }
-            }
         }
     }
 }
@@ -840,14 +730,17 @@ __global__ void __launch_bounds__(256) fp64_probe_kernel(double* sink, int iters
 constexpr int kMaxDevices = 64;
 inline int current_device() { int d = 0; if (cudaGetDevice(&d) != cudaSuccess || d < 0 || d >= kMaxDevices) d = -1; return d; }
 
+// dynamic shared memory of a variant: the weight tables of its warps
+template <typename T, int K> constexpr int variant_smem() { return kWarpsPerCta * wtab_elems<T, K>() * (int)sizeof(T); }
+
 template <typename T, int K, int W, bool STRIPED, int F>
 cudaError_t prepare_variant()
 {
     static std::atomic<bool> ready[kMaxDevices];
     const int dev = current_device();
     if (dev >= 0 && ready[dev].load(std::memory_order_acquire)) return cudaSuccess;
-    constexpr int smem = kWarpsPerCta * wtab_elems<T, K>() * (int)sizeof(T);
-    const cudaError_t e = cudaFuncSetAttribute(pmm_forward_kernel<T, K, W, STRIPED, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    const cudaError_t e = cudaFuncSetAttribute(pmm_forward_kernel<T, K, W, STRIPED, F>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               variant_smem<T, K>());
     if (e == cudaSuccess && dev >= 0) ready[dev].store(true, std::memory_order_release);
     return e;
 }
@@ -855,10 +748,9 @@ cudaError_t prepare_variant()
 template <typename T, int K, int W, bool STRIPED, int F>
 cudaError_t launch_variant(const ForwardArgs& a, const FallbackQueue& fq, int ctas, cudaStream_t s)
 {
-    constexpr int smem = kWarpsPerCta * wtab_elems<T, K>() * (int)sizeof(T);
     const cudaError_t e = prepare_variant<T, K, W, STRIPED, F>();
     if (e != cudaSuccess) return e;
-    pmm_forward_kernel<T, K, W, STRIPED, F><<<ctas, kWarpsPerCta * 32, smem, s>>>(a, fq);
+    pmm_forward_kernel<T, K, W, STRIPED, F><<<ctas, kWarpsPerCta * 32, variant_smem<T, K>(), s>>>(a, fq);
     return cudaGetLastError();
 }
 
@@ -868,74 +760,43 @@ int variant_ctas_per_sm()
     static std::atomic<int> cached[kMaxDevices];               // occupancy + 1; 0 = not looked up yet
     const int dev = current_device();
     if (dev >= 0) { const int v = cached[dev].load(std::memory_order_relaxed); if (v) return v - 1; }
-    constexpr int smem = kWarpsPerCta * wtab_elems<T, K>() * (int)sizeof(T);
     if (prepare_variant<T, K, W, STRIPED, F>() != cudaSuccess) return 0;
     int n = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, pmm_forward_kernel<T, K, W, STRIPED, F>, kWarpsPerCta * 32, smem) != cudaSuccess) return 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, pmm_forward_kernel<T, K, W, STRIPED, F>, kWarpsPerCta * 32,
+                                                      variant_smem<T, K>()) != cudaSuccess) return 0;
     if (dev >= 0) cached[dev].store(n + 1, std::memory_order_relaxed);
     return n;
 }
 
+template <typename T, int K, int W, bool STRIPED, int F>
+constexpr ForwardKernel kVariant{&variant_ctas_per_sm<T, K, W, STRIPED, F>, &launch_variant<T, K, W, STRIPED, F>};
+
 }  // namespace
 
-cudaError_t launch_forward_f32(int K, int W, bool striped, bool fast, const ForwardArgs& a, const FallbackQueue& fq, int ctas, cudaStream_t s)
+const ForwardKernel* forward_f32_variant(int K, int W, bool striped, bool fast)
 {
     if (striped) {
-        if (K != kStripedK || W != 32) return cudaErrorInvalidValue;
-        return fast ? launch_variant<float, kStripedK, 32, true, kPush | kFast>(a, fq, ctas, s)
-                    : launch_variant<float, kStripedK, 32, true, kPush>(a, fq, ctas, s);
+        if (K != kStripedK || W != 32) return nullptr;
+        return fast ? &kVariant<float, kStripedK, 32, true, kPush | kFast> : &kVariant<float, kStripedK, 32, true, kPush>;
     }
-#define X(k, w) if (K == k && W == w) return fast ? launch_variant<float, k, w, false, kPush | kFast>(a, fq, ctas, s) \
-                                                   : launch_variant<float, k, w, false, kPush>(a, fq, ctas, s);
+#define X(k, w) if (K == k && W == w) return fast ? &kVariant<float, k, w, false, kPush | kFast> : &kVariant<float, k, w, false, kPush>;
     PMM_F32_VARIANTS(X)
 #undef X
-    return cudaErrorInvalidValue;
-}
-
-int forward_f32_ctas_per_sm(int K, int W, bool striped, bool fast)
-{
-    if (striped) {
-        if (K != kStripedK || W != 32) return 0;
-        return fast ? variant_ctas_per_sm<float, kStripedK, 32, true, kPush | kFast>() : variant_ctas_per_sm<float, kStripedK, 32, true, kPush>();
-    }
-#define X(k, w) if (K == k && W == w) return fast ? variant_ctas_per_sm<float, k, w, false, kPush | kFast>() \
-                                                   : variant_ctas_per_sm<float, k, w, false, kPush>();
-    PMM_F32_VARIANTS(X)
-#undef X
-    return 0;
+    return nullptr;
 }
 
 // Exact float re-check of single pairs (fast mode's guard band): one read per warp, any length, parameters inline.
-cudaError_t launch_recheck_f32(const ForwardArgs& a, const FallbackQueue& fq, int ctas, cudaStream_t s)
-{
-    return launch_variant<float, kStripedK, 32, true, kPush | kInline>(a, fq, ctas, s);
-}
-
-int recheck_f32_ctas_per_sm() { return variant_ctas_per_sm<float, kStripedK, 32, true, kPush | kInline>(); }
-
-// Double re-run: rows per lane K in {4, 5, 6, 8} (W = 32, multi-stripe capable); see pick_f64_rows().
-#define PMM_F64_ROWS(X) X(4) X(5) X(6) X(8)
+const ForwardKernel& recheck_f32_variant() { return kVariant<float, kStripedK, 32, true, kPush | kInline>; }
 
 // striped = false: every read of the job fits one stripe (32 K - 1 bases), the common case; the loop then carries no
 // row through scratch memory (in the striped variant those loads, stores and their branches are a fifth of the
 // steady loop's non-DP instructions).
-cudaError_t launch_forward_f64(int K, bool striped, const ForwardArgs& a, int ctas, cudaStream_t s)
+const ForwardKernel* forward_f64_variant(int K, bool striped)
 {
-    const FallbackQueue none{};
-#define X(k) if (K == k) return striped ? launch_variant<double, k, 32, true, kRetry | kList>(a, none, ctas, s) \
-                                        : launch_variant<double, k, 32, false, kRetry | kList>(a, none, ctas, s);
+#define X(k) if (K == k) return striped ? &kVariant<double, k, 32, true, kRetry | kList> : &kVariant<double, k, 32, false, kRetry | kList>;
     PMM_F64_ROWS(X)
 #undef X
-    return cudaErrorInvalidValue;
-}
-
-int forward_f64_ctas_per_sm(int K, bool striped)
-{
-#define X(k) if (K == k) return striped ? variant_ctas_per_sm<double, k, 32, true, kRetry | kList>() \
-                                        : variant_ctas_per_sm<double, k, 32, false, kRetry | kList>();
-    PMM_F64_ROWS(X)
-#undef X
-    return 0;
+    return nullptr;
 }
 
 // Rows per lane of the double kernel for a job whose longest read has max_read_len bases: the block (128, 160, 192 or
@@ -944,7 +805,7 @@ int pick_f64_rows(uint32_t max_read_len)
 {
     const uint32_t rows = max_read_len + 1;
     int best = 0; uint32_t best_padded = 0;
-    for (int k : {4, 5, 6, 8}) {
+    for (int k : kF64Rows) {
         const uint32_t blk = 32u * k, padded = (rows + blk - 1) / blk * blk;
         if (!best || padded <= best_padded) { best = k; best_padded = padded; }
     }

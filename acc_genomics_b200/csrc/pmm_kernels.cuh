@@ -95,20 +95,20 @@ cudaError_t launch_build_fallback(const FallbackBuild& b, int sm_count, cudaStre
 
 // Launch helpers implemented in pmm_kernels.cu -------------------------------------------------------------
 
-// Float pass.  (K rows per lane) x (W lanes per read); W in {8,16,32}.  Returns cudaErrorInvalidValue for an
-// uninstantiated (K, W).  `striped` selects the multi-stripe variant for reads longer than W*K - 1 bases.  Results
-// below 1e-28f are appended to fq as they are produced.
-cudaError_t launch_forward_f32(int K, int W, bool striped, bool fast, const ForwardArgs& a, const FallbackQueue& fq, int ctas, cudaStream_t s);
+// One instantiated variant of the forward kernel: CTAs per SM it reaches (0 if unknown) and its launch on `ctas` CTAs.
+struct ForwardKernel {
+    int (*ctas_per_sm)();
+    cudaError_t (*launch)(const ForwardArgs& a, const FallbackQueue& fq, int ctas, cudaStream_t s);
+};
+// Float pass.  (K rows per lane) x (W lanes per read); W in {8,16,32}; null for an uninstantiated (K, W).  `striped`
+// selects the multi-stripe variant for reads longer than W*K - 1 bases.  Results below 1e-28f are appended to fq.
+const ForwardKernel* forward_f32_variant(int K, int W, bool striped, bool fast);
 // Exact float re-run of the single-pair tasks on the re-check list (fast mode), overwriting their results.
-cudaError_t launch_recheck_f32(const ForwardArgs& a, const FallbackQueue& fq, int ctas, cudaStream_t s);
-int recheck_f32_ctas_per_sm();
-// Double re-run of the tasks fallback_tasks_kernel wrote, K in {4, 5, 6, 8} rows per lane from pick_f64_rows().  Results below
-// a.tiny_threshold are recomputed in the same kernel with x86 flush-to-zero emulated on every product.
-cudaError_t launch_forward_f64(int K, bool striped, const ForwardArgs& a, int ctas, cudaStream_t s);
+const ForwardKernel& recheck_f32_variant();
+// Double re-run (fq unused) of the tasks fallback_tasks_kernel wrote, K from pick_f64_rows(); null for a K not in kF64Rows.
+// Results below a.tiny_threshold are recomputed in the same kernel with x86 flush-to-zero emulated on every product.
+const ForwardKernel* forward_f64_variant(int K, bool striped);
 int pick_f64_rows(uint32_t max_read_len);
-// CTAs per SM the given variant reaches.
-int forward_f32_ctas_per_sm(int K, int W, bool striped, bool fast = false);
-int forward_f64_ctas_per_sm(int K, bool striped);
 
 cudaError_t launch_build_stream(const uint8_t* hap_blob, const HapDesc* haps, const uint32_t* spos, uint32_t num_hap,
                                 uint8_t* stream, float* inity_f, double* inity_d, float ic_f, double ic_d,

@@ -226,11 +226,11 @@ int plan_job(uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, cons
     uint32_t top = plan.haps_per_task;
     const RunTiers& tiers = opt.tiers;
     if (tiers.depth > 0 && group_haps > 0) {
-        // resident warps of the launch most groups belong to (min_ctas<float, K> of pmm_kernels.cu x 4 warps)
+        // resident warps of the launch most groups belong to
         std::vector<uint32_t> by_k(kMaxK + 2, 0);
         for (const Group& g : groups) ++by_k[g.v.striped ? kMaxK + 1 : g.v.K];
         const int kmaj = (int)(std::max_element(by_k.begin(), by_k.end()) - by_k.begin());
-        const uint64_t wr = (uint64_t)std::max(1, sm_count) * 4 * (kmaj <= 11 ? 4 : kmaj <= 14 ? 3 : 2);
+        const uint64_t wr = (uint64_t)std::max(1, sm_count) * kWarpsPerCta * resident_ctas<float>(kmaj);
         const double u = (double)group_haps, u1 = (double)tiers.depth * wr, u2 = 2.0 * tiers.depth * wr;
         // the largest run: even made of the job's longest haplotypes, a task may not take more than `share` per cent of
         // the steps a warp does in the whole launch (config 4, 1-2 kb haplotypes and seven per warp: runs lose 5 %)
@@ -299,12 +299,11 @@ int plan_job(uint32_t num_read, const uint32_t* read_off, uint32_t num_hap, cons
         const uint32_t kw = gd.K * gd.W;
         gd.nstripes = gr.v.striped ? (read_off[gr.reads[0] + 1] - read_off[gr.reads[0]] + kw) / kw : 1u;
         const uint64_t slots = gr.v.striped ? 1u : 32u / gd.W;
-        if (plan.param_floats + slots * gd.nstripes * kParamPlanes * kw + wtab_floats(kMaxK) >= (1ull << 32)) {
+        if (plan.param_floats + slots * gd.nstripes * kParamPlanes * kw >= (1ull << 32)) {
             err = "row parameters of one job exceed 16 GiB: split it"; return PMM_ERR_INVALID;
         }
         gd.param_off = (uint32_t)plan.param_floats;
         plan.param_floats += slots * gd.nstripes * kParamPlanes * kw;
-        if (!gr.v.striped) plan.param_floats += wtab_floats(gr.v.K);     // the group's weight tile, see pmm_types.h
         plan.groups.push_back(gd);
         if (plan.segs.empty() || !(plan.segs.back().v == gr.v)) plan.segs.push_back(LaunchSeg{gr.v, (uint32_t)ntasks, 0});
         const uint32_t nruns = table_of(gr.region, gr.v.striped).count;

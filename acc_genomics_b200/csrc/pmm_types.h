@@ -7,17 +7,28 @@ namespace pmm {
 constexpr int kMaxGroups = 4;           // reads per warp: 32 / W, W >= 8
 // Warps per CTA of the forward kernels.  Every warp works alone (its own tasks, its own slice of shared memory; no
 // __syncthreads anywhere), so the CTA size only decides the granularity at which the SM's registers and shared memory are
-// taken and given back.  Measured with 1 (build option WARPS_PER_CTA): no difference anywhere -- in particular a one-warp
-// CTA of the double kernel does not slip in beside the float kernel's eight warps per SM, because registers are per
-// SMSP (16 384 each, two float warps of 7 424 leave 1 536): DESIGN.md section 4.5.
-#ifndef PMM_WARPS_PER_CTA
-#define PMM_WARPS_PER_CTA 4
-#endif
-constexpr int kWarpsPerCta = PMM_WARPS_PER_CTA;
-static_assert(kWarpsPerCta == 1 || kWarpsPerCta == 2 || kWarpsPerCta == 4, "warps per CTA");
+// taken and given back.  Measured with 1: no difference anywhere -- in particular a one-warp CTA of the double kernel does
+// not slip in beside the float kernel's eight warps per SM, because registers are per SMSP (16 384 each, two float warps
+// of 7 424 leave 1 536): DESIGN.md section 4.5.
+constexpr int kWarpsPerCta = 4;
 constexpr int kF64K = 6;                // rows per lane of the double kernel (W = 32): 191-base reads in one stripe
 constexpr int kMaxK = 20;               // most rows per lane of any float variant
 constexpr int kStripedK = 8;            // rows per lane of the striped float kernel (W = 32)
+// Rows per lane of the double kernel's instantiations (W = 32), of which pick_f64_rows() chooses one per job.
+#define PMM_F64_ROWS(X) X(4) X(5) X(6) X(8)
+#define PMM_F64_ROWS_ITEM(k) k,
+constexpr int kF64Rows[] = {PMM_F64_ROWS(PMM_F64_ROWS_ITEM)};
+#undef PMM_F64_ROWS_ITEM
+
+// Resident CTAs per SM of the forward kernel for element type T and K rows per lane: what its __launch_bounds__ asks the
+// register allocator to leave room for, and what the planner counts on.  The state of a lane is 8 registers per row
+// (5 parameters + M, X, Y), so K decides the occupancy step (64K registers / 128 threads).
+// Measured (tools/occ_check.py): 15 and 16 rows per lane at two CTAs per SM (up to 255 registers) beat three CTAs at 168
+// registers by 5.6 % (config 4, K = 16 / W = 16: 2 343 -> 2 475 GCUPS); for K <= 14 the difference is within 2 %.
+template <typename T> constexpr int resident_ctas(int K)
+{
+    return sizeof(T) == 8 ? (K <= 6 ? 3 : 2) : K <= 11 ? 4 : K <= 14 ? 3 : 2;
+}
 
 struct ReadDesc { uint32_t off, stride, len; };
 struct HapDesc  { uint32_t off, len; };
@@ -44,19 +55,8 @@ static_assert(sizeof(Task) == 48, "Task layout");
 // [stripe][plane][j][l]: plane p of the row that is row j of lane l -- consecutive lanes read consecutive addresses.
 // Planes: 0 pMM, 1 pGAPM, 2 pMX, 3 pMY, 4 pXX = pYY, 5 match weight 1 - e, 6 mismatch weight e / 3, 7 base class
 // as an integer (0..4, kPadClass for a boundary row above the read or an unused slot).
-// Behind the planes of a one-stripe group comes (builds with PMM_TILE_COPY != 0) its match-weight tile, wtab_floats(K) floats: the [5 haplotype classes]
-// [K rows] weights of the group's (up to 32/W) reads in exactly the layout the forward kernel keeps in shared memory --
-// element (class h, row j, lane) at h * (KQ * 128) + (j / 4) * 128 + lane * 4 + j % 4, KQ = ceil(K / 4) -- so that a warp
-// stages it with one bulk copy (TMA, cp.async.bulk) per task instead of rebuilding it from the planes.
-// PMM_TILE_COPY (build option): 0 = no tile, every task builds its table from planes 5-7 (the default: fastest, see
-// DESIGN.md section 4.1b); 1 = tile staged by cp.async; 2 = by one TMA bulk copy per task.
-#ifndef PMM_TILE_COPY
-#define PMM_TILE_COPY 0
-#endif
-constexpr int kTileCopy = PMM_TILE_COPY;
 constexpr int kParamPlanes = 8;
 constexpr uint32_t kPadClass = 5;
-inline constexpr uint32_t wtab_floats(int K) { return kTileCopy ? 5u * (uint32_t)((K + 3) / 4) * 128u : 0u; }
 struct GroupDesc {
     uint32_t read[kMaxGroups];
     uint32_t nreads;

@@ -186,7 +186,7 @@ int sw_align_batch(sw_ctx* c, uint32_t n_pairs,
         a.n_elem = static_cast<int32_t*>(c->d_nelem.p); a.offset = static_cast<int32_t*>(c->d_off.p);
         a.score = static_cast<int32_t*>(c->d_score.p);
         a.max_l1 = 0; a.max_l2 = 0;
-        a.k_neg1 = -1; a.k_one = 1;
+        a.k_neg1 = -1;
         for (uint32_t k = ch.first; k < ch.second; ++k) { a.max_l1 = std::max(a.max_l1, hp[k].l1); a.max_l2 = std::max(a.max_l2, hp[k].l2); }
         SW_CUDA(c, cudaMemsetAsync(a.counter, 0, sizeof(uint32_t), s));
         SW_CUDA(c, launch_align(a, c->sm_count, s, nullptr));

@@ -79,7 +79,7 @@ struct FillCtx {
     int nrow, ncol, lane;
     int match, mismatch, open, extend;
     bool indel;
-    int neg1, one;
+    int neg1;
 };
 
 // CUTOFF: apply max(MATRIX_MIN_CUTOFF, .) to the diagonal term like the reference (PairWiseSW.h:31).  The host drops it
@@ -92,12 +92,6 @@ __device__ __forceinline__ void fill_matrix(const FillCtx& c)
     const int match = c.match, mismatch = c.mismatch, open = c.open, extend = c.extend;
     const bool indel = c.indel;
     const int neg1 = c.neg1;                       // -1, kept opaque to the compiler (see cells())
-#ifndef SW_FMA_ADDS
-#define SW_FMA_ADDS 0                              // bit 0: E/F adds, bit 1: diagonal add as multiply-adds (FMA pipe)
-#endif
-    const int one = c.one;
-    auto add_ef = [&](int x, int y) { return (SW_FMA_ADDS & 1) ? imad(x, one, y) : x + y; };
-    auto add_m = [&](int x, int y) { return (SW_FMA_ADDS & 2) ? imad(x, one, y) : x + y; };
     {
         const int nblk = (nrow + 32 * K - 1) / (32 * K);
         #pragma unroll 1
@@ -144,13 +138,13 @@ __device__ __forceinline__ void fill_matrix(const FillCtx& c)
                 #pragma unroll
                 for (int k = 0; k < K; ++k) {
                     const int hleft = Hrow[k];
-                    const int ext_h = add_ef(E[k], extend), open_h = add_ef(hleft, open);
+                    const int ext_h = E[k] + extend, open_h = hleft + open;
                     const int e11 = max(ext_h, open_h);
                     const int d_ins_open = imad(open_h, neg1, ext_h);           // < 0: open_h > ext_h; ties extend
-                    const int ext_v = add_ef(fup, extend), open_v = add_ef(hup, open);
+                    const int ext_v = fup + extend, open_v = hup + open;
                     const int f11 = max(ext_v, open_v);
                     const int d_del_open = imad(open_v, neg1, ext_v);
-                    const int m11 = add_m(diag, c1[k] == c2 ? match : mismatch);
+                    const int m11 = diag + (c1[k] == c2 ? match : mismatch);
                     const int h0 = CUTOFF ? max(kMinCutoff, m11) : m11;
                     const int d_take_ins = imad(e11, neg1, h0);                 // < 0: e11 > h0
                     const int h1 = max(h0, e11);
@@ -284,7 +278,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, 3) sw_align_kernel(const Ar
 
         // ---- matrix fill -----------------------------------------------------------------------------------------
         {
-            const FillCtx fc{sm, a.seq1 + pd.s1, B, stride, nrow, ncol, lane, a.match, a.mismatch, open, extend, indel, a.k_neg1, a.k_one};
+            const FillCtx fc{sm, a.seq1 + pd.s1, B, stride, nrow, ncol, lane, a.match, a.mismatch, open, extend, indel, a.k_neg1};
             switch (K) {
 #define X(k) case k: fill_matrix<k, CUTOFF>(fc); break;
                 SW_ROWS_PER_LANE(X)

@@ -48,7 +48,7 @@ struct Args {
     int32_t*        offset;
     int32_t*        score;
     uint32_t        max_l1, max_l2;      // of the chunk: sizes the per-warp shared memory
-    int             k_neg1, k_one;       // -1 and 1: multipliers kept opaque to the compiler (see cells() in sw_kernels.cu)
+    int             k_neg1;              // -1: multiplier kept opaque to the compiler (see cells() in sw_kernels.cu)
 };
 
 size_t smem_bytes_per_warp(uint32_t max_l1, uint32_t max_l2);
