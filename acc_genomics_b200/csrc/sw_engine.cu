@@ -1,12 +1,15 @@
 // sw_engine.cu -- the C ABI of include/smithwaterman_cuda.h: validation, chunking by backtrack-memory budget, largest
 // pairs first, one kernel launch per chunk, results back.  Stands where the reference has its per-pair CPU loop
 // (/root/reference/htc-sw/host/FalconSW_AVX.cpp:304-313) and the FPGA dispatch (host/sw_host.cpp:13-15).  No CPU path.
+// sw_extend_batch, BWA-MEM's seed extension, shares the context: its stream, events and grow-only buffers.
 #include "../../include/smithwaterman_cuda.h"
 #include "cuda_util.h"
 #include "host_workers.h"
+#include "sw_extend_kernels.cuh"
 #include "sw_kernels.cuh"
 
 #include <algorithm>
+#include <atomic>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -19,6 +22,21 @@ using namespace sw;
 
 namespace {
 std::string g_sw_create_error;
+
+// Largest jobs first: warps pull jobs in order, the tail of the launch is made of the small ones.  A stable counting
+// sort on 4096 size classes (size >> shift, which the caller keeps below 4096), linear in the number of jobs: the order
+// inside a class does not matter for the tail.
+template <class Size>
+std::vector<uint32_t> largest_first(uint32_t n, int shift, const Size& size)
+{
+    constexpr uint32_t kClasses = 4096;
+    std::vector<uint32_t> order(n), first(kClasses + 1, 0);
+    auto cls = [&](uint32_t p) { return kClasses - 1 - (uint32_t)(size(p) >> shift); };
+    for (uint32_t p = 0; p < n; ++p) ++first[cls(p) + 1];
+    for (uint32_t k = 0; k < kClasses; ++k) first[k + 1] += first[k];
+    for (uint32_t p = 0; p < n; ++p) order[first[cls(p)]++] = p;
+    return order;
+}
 }  // namespace
 
 constexpr uint64_t kCigarScratchBytes = 256ull << 20;   // per-chunk scratch rows of the traceback (cigar_cap elements per pair)
@@ -107,18 +125,7 @@ int sw_align_batch(sw_ctx* c, uint32_t n_pairs,
     }
     if (ext1 >= (1ull << 31) || ext2 >= (1ull << 31)) return c->fail(SW_ERR_INVALID, "sequence blobs larger than 2 GiB");
 
-    // largest pairs first: warps pull pairs in order, the tail of the launch is made of the small ones.  A stable
-    // counting sort on 4096 size classes (cells / 4096), linear in the number of pairs: the order inside a class does
-    // not matter for the tail.
-    std::vector<uint32_t> order(n_pairs);
-    {
-        constexpr uint32_t kClasses = 4096;                              // cells < 2^24
-        std::vector<uint32_t> first(kClasses + 1, 0);
-        auto cls = [&](uint32_t p) { return kClasses - 1 - (uint32_t)(((uint64_t)seq1_len[p] * seq2_len[p]) >> 12); };
-        for (uint32_t p = 0; p < n_pairs; ++p) ++first[cls(p) + 1];
-        for (uint32_t k = 0; k < kClasses; ++k) first[k + 1] += first[k];
-        for (uint32_t p = 0; p < n_pairs; ++p) order[first[cls(p)]++] = p;
-    }
+    const std::vector<uint32_t> order = largest_first(n_pairs, 12, [&](uint32_t p) { return (uint64_t)seq1_len[p] * seq2_len[p]; });
 
     mark("sorted");
     SW_CUDA(c, c->d_seq1.reserve(ext1)); SW_CUDA(c, c->d_seq2.reserve(ext2));
@@ -237,6 +244,110 @@ int sw_align_batch(sw_ctx* c, uint32_t n_pairs,
     c->stats = sw_stats_t{};
     c->stats.pairs = n_pairs; c->stats.cells = cells; c->stats.bytes_backtrack = max_words * sizeof(uint32_t);
     c->stats.kernel_launches = launches; c->stats.chunks = (uint32_t)chunks.size();
+    cudaEventElapsedTime(&c->stats.ms_kernel, c->ev[0], c->ev[1]);
+    c->stats.ms_total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return SW_OK;
+}
+
+int sw_extend_batch(sw_ctx* c, uint32_t n_jobs, const uint8_t* query_bytes, const uint8_t* target_bytes,
+                    const sw_extend_job_t* jobs, int m, const int8_t* mat,
+                    int o_del, int e_del, int o_ins, int e_ins, int zdrop, sw_extend_result_t* out)
+{
+    using namespace swx;
+    if (!c) return SW_ERR_INVALID;
+    if (!n_jobs) return SW_OK;
+    if (!query_bytes || !target_bytes || !jobs || !mat || !out) return c->fail(SW_ERR_INVALID, "null argument");
+    if (m < 1 || m > kMaxAlphabet) return c->fail(SW_ERR_INVALID, "alphabet size m outside [1, 16]");
+    if (o_del < 0 || o_del > kMaxGap || o_ins < 0 || o_ins > kMaxGap) return c->fail(SW_ERR_INVALID, "gap open outside [0, 4096]");
+    if (e_del < 1 || e_del > kMaxGap || e_ins < 1 || e_ins > kMaxGap) return c->fail(SW_ERR_INVALID, "gap extension outside [1, 4096]");
+    const auto t0 = std::chrono::steady_clock::now();
+    int mx = 0;                                           // bwa's largest matrix entry, at least 0
+    for (int k = 0; k < m * m; ++k) mx = std::max<int>(mx, mat[k]);
+    uint64_t extq = 0, extt = 0;
+    uint32_t max_qlen = 0;
+    for (uint32_t k = 0; k < n_jobs; ++k) {
+        const sw_extend_job_t& j = jobs[k];
+        if (j.q_len < 1 || j.q_len > (uint32_t)kMaxQuery) return c->fail(SW_ERR_INVALID, "query length outside [1, 4095]");
+        if (j.t_len < 1 || j.t_len > (uint32_t)kMaxTarget) return c->fail(SW_ERR_INVALID, "target length outside [1, 65535]");
+        if (j.h0 < 1 || j.h0 > kMaxH0) return c->fail(SW_ERR_INVALID, "h0 outside [1, 2^24]");
+        if (j.w < 0 || j.w > kMaxBand) return c->fail(SW_ERR_INVALID, "band w outside [0, 65535]");
+        if (j.end_bonus < 0 || j.end_bonus > kMaxEndBonus) return c->fail(SW_ERR_INVALID, "end_bonus outside [0, 65536]");
+        extq = std::max<uint64_t>(extq, (uint64_t)j.q_start + j.q_len);
+        extt = std::max<uint64_t>(extt, (uint64_t)j.t_start + j.t_len);
+        max_qlen = std::max(max_qlen, j.q_len);
+    }
+    if (extq >= (1ull << 31) || extt >= (1ull << 31)) return c->fail(SW_ERR_INVALID, "sequence blobs larger than 2 GiB");
+    {
+        // every byte of every job below m (the kernel indexes the m x m matrix with them), on the host workers
+        std::atomic<bool> bad{false};
+        pmm::host_parallel_for(n_jobs, 2048, [&](uint64_t k0, uint64_t k1) {
+            bool b = false;
+            for (uint64_t k = k0; k < k1 && !b; ++k) {
+                const sw_extend_job_t& j = jobs[k];
+                for (uint32_t x = 0; x < j.q_len; ++x) b |= query_bytes[j.q_start + x] >= m;
+                for (uint32_t x = 0; x < j.t_len; ++x) b |= target_bytes[j.t_start + x] >= m;
+            }
+            if (b) bad = true;
+        });
+        if (bad) return c->fail(SW_ERR_INVALID, "sequence byte not below m");
+    }
+    cudaSetDevice(c->device);
+    cudaStream_t s = c->stream;
+
+    const std::vector<uint32_t> order = largest_first(n_jobs, 16, [&](uint32_t k) { return (uint64_t)jobs[k].q_len * jobs[k].t_len; });
+    // staging: query bytes, target bytes, job descriptors (in the order warps take them), into pinned memory
+    const size_t off_jobs = (extq + extt + 15) & ~(size_t)15;
+    SW_CUDA(c, c->h_stage.reserve(off_jobs + sizeof(JobDesc) * (size_t)n_jobs));
+    SW_CUDA(c, c->d_seq1.reserve(extq)); SW_CUDA(c, c->d_seq2.reserve(extt));
+    SW_CUDA(c, c->d_pairs.reserve(sizeof(JobDesc) * (size_t)n_jobs));
+    const size_t res_bytes = sizeof(sw_extend_result_t) * (size_t)n_jobs;    // then the batch's cell count
+    SW_CUDA(c, c->d_compact.reserve(res_bytes + sizeof(uint64_t)));
+    SW_CUDA(c, c->d_counter.reserve(256));
+    SW_CUDA(c, c->h_out.reserve(res_bytes + sizeof(uint64_t)));
+    char* hs = static_cast<char*>(c->h_stage.p);
+    auto copy_in = [&](char* dst, const uint8_t* src, uint64_t n) {
+        pmm::host_parallel_for(n, 1 << 18, [&](uint64_t b0, uint64_t b1) { memcpy(dst + b0, src + b0, b1 - b0); });
+    };
+    copy_in(hs, query_bytes, extq); copy_in(hs + extq, target_bytes, extt);
+    JobDesc* hj = reinterpret_cast<JobDesc*>(hs + off_jobs);
+    pmm::host_parallel_for(n_jobs, 4096, [&](uint64_t k0, uint64_t k1) {
+        for (uint64_t k = k0; k < k1; ++k) {
+            const sw_extend_job_t& j = jobs[order[k]];
+            // bwa's band cap, in double as bwa computes it (ksw_extend2 of bwa 0.7.17)
+            const int qlen = (int)j.q_len;
+            const int max_ins = std::max(1, (int)((double)(qlen * mx + j.end_bonus - o_ins) / e_ins + 1.));
+            const int max_del = std::max(1, (int)((double)(qlen * mx + j.end_bonus - o_del) / e_del + 1.));
+            hj[k] = JobDesc{j.q_start, j.q_len, j.t_start, j.t_len, j.h0, std::min(j.w, std::min(max_ins, max_del)), order[k], 0u};
+        }
+    });
+    SW_CUDA(c, cudaMemcpyAsync(c->d_seq1.p, hs, extq, cudaMemcpyHostToDevice, s));
+    SW_CUDA(c, cudaMemcpyAsync(c->d_seq2.p, hs + extq, extt, cudaMemcpyHostToDevice, s));
+    SW_CUDA(c, cudaMemcpyAsync(c->d_pairs.p, hj, sizeof(JobDesc) * (size_t)n_jobs, cudaMemcpyHostToDevice, s));
+
+    swx::Args a{};
+    a.query = static_cast<uint8_t*>(c->d_seq1.p); a.target = static_cast<uint8_t*>(c->d_seq2.p);
+    a.jobs = static_cast<JobDesc*>(c->d_pairs.p); a.njobs = n_jobs;
+    a.counter = static_cast<uint32_t*>(c->d_counter.p);
+    a.out = static_cast<int32_t*>(c->d_compact.p);
+    a.cells = reinterpret_cast<unsigned long long*>(static_cast<char*>(c->d_compact.p) + res_bytes);
+    a.max_qlen = max_qlen;
+    a.m = m; a.o_del = o_del; a.e_del = e_del; a.o_ins = o_ins; a.e_ins = e_ins; a.zdrop = zdrop;
+    memcpy(a.mat, mat, (size_t)m * m);
+    SW_CUDA(c, cudaMemsetAsync(a.counter, 0, sizeof(uint32_t), s));
+    SW_CUDA(c, cudaMemsetAsync(a.cells, 0, sizeof(uint64_t), s));
+    SW_CUDA(c, cudaEventRecord(c->ev[0], s));
+    SW_CUDA(c, launch_extend(a, c->sm_count, s));
+    SW_CUDA(c, cudaEventRecord(c->ev[1], s));
+    SW_CUDA(c, cudaMemcpyAsync(c->h_out.p, c->d_compact.p, res_bytes + sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
+    SW_CUDA(c, cudaStreamSynchronize(s));
+    static_assert(sizeof(sw_extend_result_t) == 6 * sizeof(int32_t), "result layout");
+    const char* ho = static_cast<const char*>(c->h_out.p);
+    pmm::host_parallel_for(res_bytes, 1 << 20, [&](uint64_t b0, uint64_t b1) { memcpy(reinterpret_cast<char*>(out) + b0, ho + b0, b1 - b0); });
+
+    c->stats = sw_stats_t{};
+    c->stats.pairs = n_jobs;
+    memcpy(&c->stats.cells, ho + res_bytes, sizeof(uint64_t));
+    c->stats.kernel_launches = 1; c->stats.chunks = 1;
     cudaEventElapsedTime(&c->stats.ms_kernel, c->ev[0], c->ev[1]);
     c->stats.ms_total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return SW_OK;

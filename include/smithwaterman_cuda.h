@@ -70,6 +70,24 @@ int  sw_align_batch(sw_ctx* ctx, uint32_t n_pairs,
                     int w_match, int w_mismatch, int w_open, int w_extend, int overhang_strategy,
                     uint32_t cigar_cap, sw_cigar_elem_t* cigars, int32_t* n_elem, int32_t* alignment_offset, int32_t* score);
 
+/* BWA-MEM seed extension: ksw_extend2 of bwa 0.7.17 (ksw.c), the banded affine-gap DP that extends a seed into the
+ * read on one side; the reference's bwa-sw FPGA kernel (bwa-sw/sdaccel/smithwaterman.cpp, sw_core) does the same job.
+ * Job k extends query_bytes[q_start .. +q_len) along target_bytes[t_start .. +t_len) from the score h0 of what is
+ * already aligned.  For a left extension the caller passes both sequences reversed, as bwa does.  h0, the band w and
+ * end_bonus are per job (bwa passes pen_clip5 for left and pen_clip3 for right extensions); the m x m matrix `mat`
+ * (row = target byte, column = query byte) and the gap penalties are per batch.  out[k] holds bwa's return value and
+ * its five outputs, identical to ksw_extend2 field by field.
+ * Domain (else SW_ERR_INVALID, and nothing is written to out): m in 1..16, every byte of a job's sequences < m,
+ * q_len in 1..4095, t_len in 1..65535, h0 in 1..2^24, o_del and o_ins in 0..4096, e_del and e_ins in 1..4096, w in
+ * 0..65535, end_bonus in 0..65536; zdrop <= 0 switches the Z-drop test off.  Stats: pairs = jobs, cells = DP cells
+ * visited (those of ksw_extend2's inner loop), chunks = 1, bytes_backtrack = 0. */
+typedef struct { uint32_t q_start, q_len, t_start, t_len; int32_t h0, w, end_bonus; } sw_extend_job_t;
+typedef struct { int32_t score, qle, tle, gtle, gscore, max_off; } sw_extend_result_t;
+
+int  sw_extend_batch(sw_ctx* ctx, uint32_t n_jobs, const uint8_t* query_bytes, const uint8_t* target_bytes,
+                     const sw_extend_job_t* jobs, int m, const int8_t* mat,
+                     int o_del, int e_del, int o_ins, int e_ins, int zdrop, sw_extend_result_t* out);
+
 int  sw_get_stats(const sw_ctx* ctx, sw_stats_t* out);
 
 #ifdef __cplusplus
