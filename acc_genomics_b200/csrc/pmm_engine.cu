@@ -966,19 +966,6 @@ static int log10_of_fallback(const uint32_t* fb_index, const double* fb_value, u
     return PMM_OK;
 }
 
-// The final doubles of the last launch: log10f of the raw floats is taken while the double pass is still running.
-static int fetch_log10_common(pmm_ctx* c, double* out, uint32_t* nfb_out)
-{
-    int rc = ensure_raw(c);
-    if (rc) return rc;
-    const HostOut o = host_out(c->R(), c->job.pairs);
-    log10_of_raw(o.raw, c->job.pairs, out);
-    if ((rc = ensure_lists(c))) return rc;
-    if (log10_of_fallback(o.idx, o.dres, o.ctrl[0], c->job.pairs, out) != PMM_OK) return c->fail(PMM_ERR_CUDA, "fallback index out of range");
-    if (nfb_out) *nfb_out = o.ctrl[0];
-    return PMM_OK;
-}
-
 int pmm_fetch_raw(pmm_ctx* c, float* out_raw, uint64_t cap)
 {
     if (!c || !out_raw) return PMM_ERR_INVALID;
@@ -1010,32 +997,19 @@ int pmm_host_finish_log10(const float* raw, uint64_t n, const uint32_t* fb_index
     return log10_of_fallback(fb_index, fb_value, n_fb, n, out);
 }
 
+// The final doubles of the last launch: log10f of the raw floats is taken while the double pass is still running.
 int pmm_fetch_log10(pmm_ctx* c, double* out, uint64_t cap, uint64_t* n_fallback)
 {
     if (!c || !out) return PMM_ERR_INVALID;
     if (cap < c->job.pairs) return c->fail(PMM_ERR_INVALID, "output buffer too small");
     auto t0 = std::chrono::steady_clock::now();
-    uint32_t nfb = 0;
-    int rc = fetch_log10_common(c, out, &nfb);
+    int rc = ensure_raw(c);
     if (rc) return rc;
-    if (n_fallback) *n_fallback = nfb;
-    c->stats.ms_fetch = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    return PMM_OK;
-}
-
-int pmm_fetch_log10_indexed(pmm_ctx* c, double* out, uint64_t cap, uint32_t* fb_index, uint64_t fb_cap, uint64_t* n_fallback)
-{
-    if (!c || !out || !n_fallback) return PMM_ERR_INVALID;
-    if (cap < c->job.pairs) return c->fail(PMM_ERR_INVALID, "output buffer too small");
-    auto t0 = std::chrono::steady_clock::now();
-    uint32_t nfb = 0;
-    int rc = fetch_log10_common(c, out, &nfb);
-    if (rc) return rc;
-    *n_fallback = nfb;
-    if (fb_index) {
-        if (fb_cap < nfb) return c->fail(PMM_ERR_INVALID, "fallback index buffer too small");
-        memcpy(fb_index, host_out(c->R(), c->job.pairs).idx, sizeof(uint32_t) * nfb);
-    }
+    const HostOut o = host_out(c->R(), c->job.pairs);
+    log10_of_raw(o.raw, c->job.pairs, out);
+    if ((rc = ensure_lists(c))) return rc;
+    if (log10_of_fallback(o.idx, o.dres, o.ctrl[0], c->job.pairs, out) != PMM_OK) return c->fail(PMM_ERR_CUDA, "fallback index out of range");
+    if (n_fallback) *n_fallback = o.ctrl[0];
     c->stats.ms_fetch = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return PMM_OK;
 }

@@ -26,7 +26,7 @@
 namespace {
 
 struct Job {
-    uint64_t ticket = 0, cells = 0, generation = 0;
+    uint64_t ticket = 0, cells = 0, pairs = 0, generation = 0;
     // flat layout, borrowed from the caller until pmm_pool_wait returns
     uint32_t num_read = 0, num_hap = 0, num_region = 0;
     const uint32_t* read_off = nullptr; const uint8_t* tr[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -67,11 +67,6 @@ struct pmm_pool {
     std::vector<uint64_t> cells_per_device, jobs_per_device;
     int n_devices = 0;
     std::vector<int> devices;
-    // Feeders can merge small waiting jobs into one GPU job (pmm_pool_set_merge).  Off by default: with two contexts per
-    // feeder and several feeders per GPU, single-region jobs of 4 000 pairs stream at 1 910-1 940 GCUPS unmerged against
-    // 1 090-1 630 merged (the host copies of merging cost more than the launches they save; tools/small_pool.py).
-    bool merge = false;
-    uint64_t merged_batches = 0;
     bool tracing = false;               // pmm_pool_trace: one record per GPU job
     std::vector<pmm_pool_trace_t> trace;
     std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
@@ -81,46 +76,18 @@ static thread_local std::string g_pool_error;      // errors of calls without a 
 
 static double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
-// Merging thresholds: a feeder that finds several jobs waiting takes more of them while the merged job stays below
-// kMergeCells cells, kMergeJobs jobs and the engine's per-job limits.  A job that is already large runs alone.
-constexpr uint64_t kMergeCells = 3000000000ull;
-constexpr size_t kMergeJobs = 64;
-constexpr uint64_t kMergeBytes = 1ull << 29, kMergePairs = 1ull << 27;
-
-struct MergeBuf {                       // per feeder, reused from batch to batch
-    std::vector<uint32_t> read_off, hap_off, fb_index;
-    std::vector<uint8_t> tr[5], hap;
-    std::vector<pmm_region_t> regions;
-    std::vector<double> out;
-    std::vector<uint64_t> out_first;    // result offset of each merged job (+ total at the end)
-};
-
-static uint64_t job_pairs(const Job* j)
-{
-    uint64_t n = 0;
-    for (uint32_t g = 0; g < j->num_region; ++g) n += (uint64_t)j->regions[g].num_read * j->regions[g].num_hap;
-    return n;
-}
-static uint64_t job_bytes(const Job* j)
-{
-    return 5ull * (j->read_off[j->num_read] - j->read_off[0]) + (j->hap_off[j->num_hap] - j->hap_off[0]);
-}
-
-// One GPU job of a feeder: the submitted jobs it serves, where it is in its life, and the host times of the trace.
+// One GPU job of a feeder: the submitted job it serves, where it is in its life, and the host times of the trace.
 struct Flight {
-    std::vector<Job*> batch;
-    MergeBuf m;                         // merged inputs / outputs (batch.size() > 1)
+    Job* job = nullptr;
     bool active = false;                // staged and launched, results not yet fetched
-    bool merged = false;
-    int rc = PMM_OK;
+    int rc = PMM_OK;                    // of staging and launch
     double t_take = 0, t_staged = 0, t_launched = 0;
 };
 
 // Stage and launch; the kernels run while the caller does something else.
-static void start_single(pmm_ctx* c, Flight& f)
+static void start_job(pmm_ctx* c, Flight& f)
 {
-    Job* j = f.batch[0];
-    f.merged = false;
+    const Job* j = f.job;
     f.rc = pmm_stage_flat(c, j->num_read, j->read_off, j->tr[0], j->tr[1], j->tr[2], j->tr[3], j->tr[4],
                           j->num_hap, j->hap_off, j->hap, j->num_region, j->regions);
     f.t_staged = now_s();
@@ -128,105 +95,32 @@ static void start_single(pmm_ctx* c, Flight& f)
     f.t_launched = now_s();
 }
 
-static void finish_single(pmm_ctx* c, Job* j, int rc)
+// Fetch the results into the caller's buffer and record the job's status.
+static void finish_job(pmm_ctx* c, const Flight& f)
 {
+    Job* j = f.job;
     uint64_t nfb = 0;
+    int rc = f.rc;
     if (rc == PMM_OK) rc = pmm_fetch_log10(c, j->out, j->out_capacity, &nfb);
     j->rc = rc; j->n_fallback = nfb;
     if (rc != PMM_OK) j->err = pmm_last_error(c);
 }
 
-static void start_merged(pmm_ctx* c, Flight& f)
+// Takes the next job off the queue.  wait = false: returns nullptr at once if nothing is queued.  Returns nullptr also
+// when the pool is stopping and drained.
+static Job* take_job(pmm_pool* p, bool wait)
 {
-    MergeBuf& m = f.m;
-    f.merged = true;
-    m.read_off.assign(1, 0); m.hap_off.assign(1, 0); m.regions.clear(); m.out_first.assign(1, 0);
-    for (int t = 0; t < 5; ++t) m.tr[t].clear();
-    m.hap.clear();
-    for (Job* j : f.batch) {
-        const uint32_t rbase = (uint32_t)m.read_off.size() - 1, hbase = (uint32_t)m.hap_off.size() - 1;
-        const uint32_t r0 = j->read_off[0], h0 = j->hap_off[0];
-        const uint32_t rshift = m.read_off.back(), hshift = m.hap_off.back();
-        for (uint32_t k = 1; k <= j->num_read; ++k) m.read_off.push_back(j->read_off[k] - r0 + rshift);
-        for (uint32_t k = 1; k <= j->num_hap; ++k) m.hap_off.push_back(j->hap_off[k] - h0 + hshift);
-        const size_t rb = j->read_off[j->num_read] - r0, hb = j->hap_off[j->num_hap] - h0;
-        for (int t = 0; t < 5; ++t) m.tr[t].insert(m.tr[t].end(), j->tr[t] + r0, j->tr[t] + r0 + rb);
-        m.hap.insert(m.hap.end(), j->hap + h0, j->hap + h0 + hb);
-        for (uint32_t g = 0; g < j->num_region; ++g) {
-            const pmm_region_t& r = j->regions[g];
-            m.regions.push_back(pmm_region_t{r.read_first + rbase, r.num_read, r.hap_first + hbase, r.num_hap});
-        }
-        m.out_first.push_back(m.out_first.back() + job_pairs(j));
-    }
-    const uint64_t total = m.out_first.back();
-    m.out.resize(total); m.fb_index.resize(total);
-    f.rc = pmm_stage_flat(c, (uint32_t)m.read_off.size() - 1, m.read_off.data(), m.tr[0].data(), m.tr[1].data(), m.tr[2].data(),
-                          m.tr[3].data(), m.tr[4].data(), (uint32_t)m.hap_off.size() - 1, m.hap_off.data(), m.hap.data(),
-                          (uint32_t)m.regions.size(), m.regions.data());
-    f.t_staged = now_s();
-    if (f.rc == PMM_OK) f.rc = pmm_launch(c);
-    f.t_launched = now_s();
-}
-
-static void finish_merged(pmm_ctx* c, Flight& f)
-{
-    MergeBuf& m = f.m;
-    std::vector<Job*>& batch = f.batch;
-    const uint64_t total = m.out_first.back();
-    int rc = f.rc;
-    uint64_t nfb = 0;
-    if (rc == PMM_OK) rc = pmm_fetch_log10_indexed(c, m.out.data(), total, m.fb_index.data(), total, &nfb);
-    if (rc == PMM_ERR_INVALID) {
-        // One caller's bad job must not fail the others it happened to be merged with (submit-time validation should
-        // have caught it; this is the second line): run every job on its own, so that only the bad one fails.
-        for (Job* j : batch) {
-            Flight one; one.batch.assign(1, j);
-            start_single(c, one);
-            finish_single(c, j, one.rc);
-        }
-        f.rc = PMM_ERR_INVALID;
-        return;
-    }
-    f.rc = rc;
-    const std::string err = rc == PMM_OK ? std::string() : std::string(pmm_last_error(c));
-    for (size_t b = 0; b < batch.size(); ++b) {
-        Job* j = batch[b];
-        j->rc = rc; j->err = err; j->n_fallback = 0;
-        if (rc == PMM_OK) memcpy(j->out, m.out.data() + m.out_first[b], sizeof(double) * (m.out_first[b + 1] - m.out_first[b]));
-    }
-    if (rc == PMM_OK)
-        for (uint64_t k = 0; k < nfb; ++k) {
-            const size_t b = std::upper_bound(m.out_first.begin(), m.out_first.end(), (uint64_t)m.fb_index[k]) - m.out_first.begin() - 1;
-            if (b < batch.size()) batch[b]->n_fallback++;
-        }
-}
-
-// Takes the next job (and, when merging, the small jobs waiting behind it) off the queue.  wait = false: returns false at
-// once if nothing is queued.  Returns false with an empty batch also when the pool is stopping and drained.
-static bool take_batch(pmm_pool* p, std::vector<Job*>& batch, bool wait)
-{
-    batch.clear();
     std::unique_lock<std::mutex> lk(p->mu);
     if (wait) p->cv_work.wait(lk, [&] { return p->stopping || !p->queue.empty(); });
-    if (p->queue.empty()) return false;
+    if (p->queue.empty()) return nullptr;
     Job* j = p->queue.top(); p->queue.pop();
-    batch.push_back(j);
-    // the queue is ordered largest first: everything behind a small job is small too
-    uint64_t cells = j->cells, bytes = job_bytes(j), pairs = job_pairs(j);
-    while (p->merge && !p->queue.empty() && batch.size() < kMergeJobs) {
-        Job* n = p->queue.top();
-        if (cells + n->cells > kMergeCells || bytes + job_bytes(n) > kMergeBytes || pairs + job_pairs(n) > kMergePairs) break;
-        p->queue.pop();
-        batch.push_back(n);
-        cells += n->cells; bytes += job_bytes(n); pairs += job_pairs(n);
-    }
-    return true;
+    return j;
 }
 
 // A feeder thread drives two contexts of one GPU in turn: it stages and launches a job on one while the job on the other
 // is still running, and only then waits for that other one.  So a job is always queued on the GPU behind the one whose
-// results the thread is fetching: the host work between two jobs of a context (copy-back, log10, merging, packing the next
-// one, about a millisecond) never leaves the GPU idle, and neither does the wake-up of a sleeping wait.  (One thread per
+// results the thread is fetching: the host work between two jobs of a context (copy-back, log10, packing the next one,
+// about a millisecond) never leaves the GPU idle, and neither does the wake-up of a sleeping wait.  (One thread per
 // context -- round 1 -- let all contexts of a GPU fall into step: kernels launched together share the GPU, finish
 // together, and the GPU then waits for all their feeders at once; profiles/r02_pool_timeline_n8.jsonl.)
 static void feeder_main(pmm_pool* p, size_t slot_a, size_t slot_b)
@@ -243,9 +137,9 @@ static void feeder_main(pmm_pool* p, size_t slot_a, size_t slot_b)
             Flight& f = fl[k];
             if (f.active) continue;
             const bool any_active = fl[0].active || fl[1].active;
-            if (take_batch(p, f.batch, !any_active)) {
+            if ((f.job = take_job(p, !any_active))) {
                 f.t_take = now_s();
-                if (f.batch.size() == 1) start_single(p->ctxs[slots[k]], f); else start_merged(p->ctxs[slots[k]], f);
+                start_job(p->ctxs[slots[k]], f);
                 f.active = true; started[k] = ++seq;
             } else if (!any_active) {
                 stopping = true;                          // woken with an empty queue: the pool is shutting down
@@ -260,16 +154,17 @@ static void feeder_main(pmm_pool* p, size_t slot_a, size_t slot_b)
         Flight& g = fl[fin];
         {
             pmm_ctx* c = p->ctxs[slots[fin]];
-            if (g.merged) finish_merged(c, g); else { finish_single(c, g.batch[0], g.rc); g.rc = g.batch[0]->rc; }
+            Job* j = g.job;
+            finish_job(c, g);
             const double t_fetched = now_s();
             pmm_pool_trace_t rec{};
             bool have_rec = false;
-            if (p->tracing && g.rc == PMM_OK) {          // (read without the lock: a stale value only adds or drops one record)
+            if (p->tracing && j->rc == PMM_OK) {          // (read without the lock: a stale value only adds or drops one record)
                 pmm_timeline_t tl;
                 if (pmm_get_timeline(c, &tl) == PMM_OK) {
                     const double origin = std::chrono::duration<double>(p->t0.time_since_epoch()).count();
-                    rec.device = p->ctx_device[slots[fin]]; rec.context = (int32_t)slots[fin]; rec.jobs = (uint32_t)g.batch.size();
-                    for (Job* j : g.batch) { rec.regions += j->num_region; rec.cells += j->cells; rec.pairs += job_pairs(j); }
+                    rec.device = p->ctx_device[slots[fin]]; rec.context = (int32_t)slots[fin];
+                    rec.regions = j->num_region; rec.cells = j->cells; rec.pairs = j->pairs;
                     rec.t_take = g.t_take - origin; rec.t_staged = g.t_staged - origin; rec.t_launched = g.t_launched - origin;
                     rec.t_fetched = t_fetched - origin;
                     rec.d_start = tl.ref_host_s + tl.kernels_start_s - origin; rec.d_f32_end = tl.ref_host_s + tl.f32_end_s - origin;
@@ -280,12 +175,9 @@ static void feeder_main(pmm_pool* p, size_t slot_a, size_t slot_b)
             {
                 std::lock_guard<std::mutex> lk(p->mu);
                 if (have_rec && p->tracing) p->trace.push_back(rec);
-                for (Job* j : g.batch) {
-                    j->device = p->ctx_device[slots[fin]]; j->done = true;
-                    for (int d = 0; d < p->n_devices; ++d)
-                        if (p->devices[d] == j->device) { p->cells_per_device[d] += j->cells; p->jobs_per_device[d]++; }
-                }
-                p->merged_batches += g.batch.size() > 1;
+                j->device = p->ctx_device[slots[fin]]; j->done = true;
+                for (int d = 0; d < p->n_devices; ++d)
+                    if (p->devices[d] == j->device) { p->cells_per_device[d] += j->cells; p->jobs_per_device[d]++; }
             }
             p->cv_done.notify_all();
             g.active = false;
@@ -325,8 +217,6 @@ int pmm_pool_create(const int* devices, int n_devices, int contexts_per_device, 
                 return rc;
             }
             p->ctxs.push_back(c); p->ctx_device.push_back(d);
-            // PMM_POOL_PRIORITY=1: the contexts of a device get distinct stream priorities (tuning; see DESIGN.md section 7)
-            if (const char* e = getenv("PMM_POOL_PRIORITY")) if (atoi(e) > 0) pmm_set_option(c, "priority", std::to_string(rep).c_str());
         }
     // Waits spin by default.  Measured on an 8-GPU box with 32 host cores (24 feeder threads): spinning 14 100 GCUPS,
     // sleeping on a blocking event 13 400 -- the wake-up latency costs more than the cores it frees.  PMM_POOL_SYNC=block
@@ -380,8 +270,9 @@ int pmm_pool_submit_flat(pmm_pool* p, uint32_t num_read, const uint32_t* read_of
         std::lock_guard<std::mutex> lk(p->mu);
         p->err = "null or empty input"; return PMM_ERR_INVALID;
     }
-    // Validate here, so that a malformed job fails its own ticket and never reaches a merged GPU job (whose size
-    // arithmetic trusts ascending offsets): offsets ascend strictly (no read or haplotype of length 0), totals fit.
+    // Validate here, so that a malformed job fails its caller at submit rather than on a feeder, and so that the pool's
+    // own reads of it are sound (`cells` below comes from read_off / hap_off at the region bounds): offsets ascend
+    // strictly (no read or haplotype of length 0), totals fit.
     {
         const char* bad = nullptr;
         for (uint32_t k = 0; k < num_read && !bad; ++k) if (read_off[k + 1] <= read_off[k]) bad = "read offsets must ascend strictly (no read of length 0)";
@@ -397,7 +288,6 @@ int pmm_pool_submit_flat(pmm_pool* p, uint32_t num_read, const uint32_t* read_of
     j->hap_off = hap_off; j->hap = hap_bases;
     if (regions && num_region) { j->regions = regions; j->num_region = num_region; }
     else { j->one_region = pmm_region_t{0, num_read, 0, num_hap}; j->regions = &j->one_region; j->num_region = 1; }
-    uint64_t pairs = 0;
     for (uint32_t g = 0; g < j->num_region; ++g) {
         const pmm_region_t& r = j->regions[g];
         if ((uint64_t)r.read_first + r.num_read > num_read || (uint64_t)r.hap_first + r.num_hap > num_hap) {
@@ -405,11 +295,11 @@ int pmm_pool_submit_flat(pmm_pool* p, uint32_t num_read, const uint32_t* read_of
             std::lock_guard<std::mutex> lk(p->mu);
             p->err = "region out of range"; return PMM_ERR_INVALID;
         }
-        pairs += (uint64_t)r.num_read * r.num_hap;
+        j->pairs += (uint64_t)r.num_read * r.num_hap;
         j->cells += (uint64_t)(read_off[r.read_first + r.num_read] - read_off[r.read_first]) *
                     (uint64_t)(hap_off[r.hap_first + r.num_hap] - hap_off[r.hap_first]);
     }
-    if (out_capacity < pairs) {
+    if (out_capacity < j->pairs) {
         delete j;
         std::lock_guard<std::mutex> lk(p->mu);
         p->err = "output buffer too small"; return PMM_ERR_INVALID;
@@ -443,15 +333,6 @@ int pmm_pool_wait(pmm_pool* p, uint64_t ticket, uint64_t* n_fallback, int* devic
     p->jobs.erase(it);
     delete j;
     return rc;
-}
-
-int pmm_pool_set_merge(pmm_pool* p, int on, uint64_t* merged_batches)
-{
-    if (!p) return PMM_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(p->mu);
-    if (on >= 0) p->merge = on != 0;
-    if (merged_batches) *merged_batches = p->merged_batches;
-    return PMM_OK;
 }
 
 int pmm_pool_trace(pmm_pool* p, int on)

@@ -21,10 +21,10 @@ PMM_OK, PMM_ERR_INVALID, PMM_ERR_CUDA, PMM_ERR_NO_DEVICE, PMM_ERR_STATE = 0, 1, 
 EXPORTS = [
     "pmm_create", "pmm_destroy", "pmm_last_error", "pmm_device_count", "pmm_set_option",
     "pmm_forward_raw_serialized", "pmm_forward_log10", "pmm_forward_log10_serialized", "pmm_forward_log10_testcases",
-    "pmm_stage_flat", "pmm_stage_serialized", "pmm_fetch_fallback", "pmm_fetch_log10_indexed", "pmm_launch", "pmm_join", "pmm_sync", "pmm_fetch_raw", "pmm_fetch_log10", "pmm_fetch_fallback_mask",
+    "pmm_stage_flat", "pmm_stage_serialized", "pmm_fetch_fallback", "pmm_launch", "pmm_join", "pmm_sync", "pmm_fetch_raw", "pmm_fetch_log10", "pmm_fetch_fallback_mask",
     "pmm_get_stats", "pmm_measure_fp32_peak", "pmm_measure_fp64_peak", "pmm_plan_flat", "pmm_host_table", "pmm_host_finish_log10",
     "pmm_pool_create", "pmm_pool_destroy", "pmm_pool_last_error", "pmm_pool_num_devices", "pmm_pool_submit_flat",
-    "pmm_pool_wait", "pmm_pool_device_load", "pmm_pool_set_merge", "pmm_pool_trace", "pmm_pool_get_trace", "pmm_get_timeline",
+    "pmm_pool_wait", "pmm_pool_device_load", "pmm_pool_trace", "pmm_pool_get_trace", "pmm_get_timeline",
 ]
 
 
@@ -44,7 +44,7 @@ class PmmTimeline(C.Structure):
 
 
 class PmmPoolTrace(C.Structure):
-    _fields_ = [("device", C.c_int32), ("context", C.c_int32), ("jobs", C.c_uint32), ("regions", C.c_uint32),
+    _fields_ = [("device", C.c_int32), ("context", C.c_int32), ("regions", C.c_uint32),
                 ("cells", C.c_uint64), ("pairs", C.c_uint64), ("t_take", C.c_double), ("t_staged", C.c_double),
                 ("t_launched", C.c_double), ("t_fetched", C.c_double), ("d_start", C.c_double), ("d_f32_end", C.c_double),
                 ("d_end", C.c_double)]
@@ -99,7 +99,6 @@ def load_library() -> C.CDLL:
         L.pmm_stage_flat.argtypes = [vp, u32, vp, vp, vp, vp, vp, vp, u32, vp, vp, u32, vp]
         L.pmm_stage_serialized.argtypes = [vp, vp, u64, vp, u64, C.POINTER(C.c_int), C.POINTER(C.c_int)]
         L.pmm_fetch_fallback.argtypes = [vp, vp, vp, u64, C.POINTER(u64)]
-        L.pmm_fetch_log10_indexed.argtypes = [vp, vp, u64, vp, u64, C.POINTER(u64)]
         L.pmm_launch.argtypes = [vp]; L.pmm_sync.argtypes = [vp]; L.pmm_join.argtypes = [vp]
         L.pmm_fetch_raw.argtypes = [vp, vp, u64]
         L.pmm_fetch_log10.argtypes = [vp, vp, u64, C.POINTER(u64)]
@@ -117,7 +116,6 @@ def load_library() -> C.CDLL:
         L.pmm_pool_submit_flat.argtypes = [vp, u32, vp, vp, vp, vp, vp, vp, u32, vp, vp, u32, vp, vp, u64, C.POINTER(u64)]
         L.pmm_pool_wait.argtypes = [vp, u64, C.POINTER(u64), C.POINTER(C.c_int)]
         L.pmm_pool_device_load.argtypes = [vp, C.c_int, C.POINTER(C.c_int), C.POINTER(u64), C.POINTER(u64)]
-        L.pmm_pool_set_merge.argtypes = [vp, C.c_int, C.POINTER(u64)]
         L.pmm_pool_trace.argtypes = [vp, C.c_int]
         L.pmm_pool_get_trace.argtypes = [vp, vp, u64, C.POINTER(u64)]
         L.pmm_get_timeline.argtypes = [vp, C.POINTER(PmmTimeline)]
@@ -369,12 +367,6 @@ class PairHMMPool:
         if rc != PMM_OK:
             raise PmmError(rc, self.lib.pmm_pool_last_error(self.h).decode())
         return out, int(nfb.value), int(dev.value)
-
-    def set_merge(self, on: bool | None = None) -> int:
-        """Switch the merging of small waiting jobs (None: leave as is); returns the number of merged GPU jobs so far."""
-        n = C.c_uint64()
-        self.lib.pmm_pool_set_merge(self.h, -1 if on is None else int(on), C.byref(n))
-        return int(n.value)
 
     def trace(self, on: bool) -> None:
         """Start (and clear) or stop recording one timeline record per GPU job (pmm_pool_trace)."""

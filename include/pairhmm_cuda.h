@@ -157,10 +157,6 @@ int  pmm_join(pmm_ctx* ctx);
 int  pmm_sync(pmm_ctx* ctx);
 int  pmm_fetch_raw(pmm_ctx* ctx, float* out_raw, uint64_t out_capacity);
 int  pmm_fetch_log10(pmm_ctx* ctx, double* out, uint64_t out_capacity, uint64_t* n_fallback);
-/* pmm_fetch_log10 that also hands out which results took the double re-run (positions in `out`, any order), from the same
- * device-to-host copy; fb_index may be NULL.  Used by the pool to split the results of a merged job. */
-int  pmm_fetch_log10_indexed(pmm_ctx* ctx, double* out, uint64_t out_capacity, uint32_t* fb_index, uint64_t fb_capacity,
-                             uint64_t* n_fallback);
 /* The pairs that took the double re-run: index[k] = position in the read-major result, value[k] = the double
  * likelihood scaled by 2^1020 (what compute_fp_avxd returns, client/PairHMMWorker.cpp:182).  With index == value ==
  * NULL only the count is returned. */
@@ -179,14 +175,12 @@ int  pmm_get_timeline(pmm_ctx* ctx, pmm_timeline_t* out);
 /* ---- multi-GPU work queue --------------------------------------------------------------------------------
  * Independent read x haplotype regions are partitioned across the GPUs of one box by a host-side queue; nothing is
  * reduced, so there is no collective (SURVEY.md section 8e).  The pool owns contexts_per_device contexts on each of
- * the given devices (NULL / 0 = every visible GPU) and one feeder thread per context; jobs are taken largest first.
+ * the given devices (NULL / 0 = every visible GPU) and one feeder thread per pair of contexts of a device; each
+ * submitted job runs as one GPU job, served by generation (a run of consecutive tickets) and largest first inside one.
  * This is what stands where the reference has Blaze's accelerator queue (client/PairHMMWorker.cpp:217-251 hands
  * tiles to client_->start() one after another) and the per-PU balancer (interface/PairHMMFpgaInterface.cpp:67-170).
  *   pmm_pool_submit_flat : same layout as pmm_stage_flat (regions == NULL: one region of everything); the input
  *                          arrays and out_log10 are borrowed until pmm_pool_wait(ticket) returns.  Thread-safe.
- * On request (pmm_pool_set_merge) small jobs that are waiting together are merged by the feeder into one multi-region GPU
- * job (up to about 3e9 cells or 64 jobs) and their results split again; off by default, the contexts' concurrency already
- * streams single-region jobs at the rate of large ones.
  *   pmm_pool_wait        : blocks until that job is done; returns the job's status, the number of pairs that took
  *                          the double re-run and the device that ran it.  Each ticket is waited for exactly once. */
 typedef struct pmm_pool pmm_pool;
@@ -200,18 +194,15 @@ int  pmm_pool_submit_flat(pmm_pool* pool, uint32_t num_read, const uint32_t* rea
                           uint32_t num_region, const pmm_region_t* regions,
                           double* out_log10, uint64_t out_capacity, uint64_t* ticket);
 int  pmm_pool_wait(pmm_pool* pool, uint64_t ticket, uint64_t* n_fallback, int* device);
-/* on = 1 / 0 switches the merging of small waiting jobs (default off), on < 0 leaves it; merged_batches (may be NULL)
- * receives how many merged GPU jobs have run so far. */
-int  pmm_pool_set_merge(pmm_pool* pool, int on, uint64_t* merged_batches);
 /* Jobs and cells completed so far by the slot-th device of the pool (0 <= slot < pmm_pool_num_devices). */
 int  pmm_pool_device_load(const pmm_pool* pool, int slot, int* device, uint64_t* jobs, uint64_t* cells);
-/* Timeline of the pool's GPU jobs (one record per job a feeder ran; merged jobs count once), for finding idle time:
+/* Timeline of the pool's GPU jobs (one record per submitted job that ran without error), for finding idle time:
  * host times of the feeder's stages and the device times of the job's kernels, all in seconds since the pool was
  * created.  pmm_pool_trace(pool, 1) starts recording (and clears), 0 stops; pmm_pool_get_trace copies up to capacity
  * records and returns how many exist. */
 typedef struct {
     int32_t  device, context;           /* CUDA device and the pool's context index that ran the job          */
-    uint32_t jobs, regions;             /* submitted jobs merged into this GPU job, regions in it               */
+    uint32_t regions;                   /* regions in the job                                                   */
     uint64_t cells, pairs;
     double   t_take, t_staged, t_launched, t_fetched;   /* host: job taken from the queue, pmm_stage_flat returned,
                                                             pmm_launch returned, results delivered                */

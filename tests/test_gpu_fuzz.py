@@ -1,5 +1,5 @@
 """A short run of tools/fuzz_gpu.py: random region shapes and multi-region jobs through every entry point (staged, serialized,
-read_t/hap_t arrays, pool with job merging), exact and fast mode, plus Smith-Waterman -- every result against the oracle."""
+read_t/hap_t arrays, pool), exact and fast mode, plus Smith-Waterman -- every result against the oracle."""
 import os
 import subprocess
 import sys

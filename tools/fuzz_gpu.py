@@ -17,7 +17,7 @@ chk = oracle.reference() or oracle.port()
 swport = oracle.sw_port()
 swchk = oracle.sw_reference() or swport
 eng = PairHMMEngine(0); fast = PairHMMEngine(0); fast.set_option("mode", "fast")
-pool = PairHMMPool(devices=[0], contexts_per_device=2); pool.set_merge(True)
+pool = PairHMMPool(devices=[0], contexts_per_device=2)
 al = sw.SmithWaterman(0)
 t0 = time.time(); it = 0; pairs = 0; swpairs = 0
 
@@ -70,7 +70,7 @@ while time.time() - t0 < budget:
     os.environ["PAIRHMM_WORKER_TILES"] = str(int(rng.integers(1, 6)))
     o5, nre = hostlayer.worker_forward(b0)
     assert same(o5, want[0][1].ravel()) and nre == int(want[0][2].sum()), ("worker", it)
-    # pool (merging of small jobs included)
+    # pool: each region a job of its own
     tk = [pool.submit(b) for b in regs]
     for t, w in zip(tk, want):
         assert same(pool.wait(t)[0], w[1].ravel()), ("pool", it)

@@ -1,5 +1,5 @@
-"""GPU box: a stream of small jobs (config 1, 4 096 pairs each) through a one-GPU pool: throughput, how many jobs each GPU
-job merged, and where the time between jobs goes (pool timeline)."""
+"""GPU box: a stream of small jobs (config 1, 4 096 pairs each) through a one-GPU pool: throughput and where the time
+between jobs goes (pool timeline)."""
 import json, os, sys, time
 from collections import deque
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -10,8 +10,6 @@ cfg = int(os.environ.get("CFG", "1")); ctxs = int(os.environ.get("CTX", "4")); d
 b = synth.config(cfg, scale=float(os.environ.get("SCALE", "1.0")))
 job = concat_regions(b); cells = sum(x.num_cells for x in b)
 pool = PairHMMPool(devices=[0], contexts_per_device=ctxs)
-if os.environ.get("MERGE") == "0":
-    pool.set_merge(False)
 outs = [np.empty(job["pairs"]) for _ in range(depth + 1)]
 def run(n):
     live = deque()
@@ -27,9 +25,8 @@ n = 200
 t0 = time.perf_counter(); run(n); dt = time.perf_counter() - t0
 pool.trace(False)
 tr = pool.get_trace()
-merged = [r["jobs"] for r in tr]
-print(json.dumps({"cfg": cfg, "contexts": ctxs, "depth": depth, "merge": os.environ.get("MERGE", "1"), "us_per_job": round(dt / n * 1e6, 1),
-                  "gcups": round(cells * n / dt * 1e-9, 1), "gpu_jobs": len(tr), "mean_merged": round(float(np.mean(merged)), 2),
+print(json.dumps({"cfg": cfg, "contexts": ctxs, "depth": depth, "us_per_job": round(dt / n * 1e6, 1),
+                  "gcups": round(cells * n / dt * 1e-9, 1), "gpu_jobs": len(tr),
                   "stage_us": round(float(np.mean([r["t_staged"] - r["t_take"] for r in tr])) * 1e6, 1),
                   "launch_us": round(float(np.mean([r["t_launched"] - r["t_staged"] for r in tr])) * 1e6, 1),
                   "kernels_us": round(float(np.mean([r["d_end"] - r["d_start"] for r in tr])) * 1e6, 1),

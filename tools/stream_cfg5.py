@@ -18,7 +18,7 @@ ap.add_argument("--regions-per-job", type=int, default=25)
 ap.add_argument("--contexts", type=int, default=3)
 ap.add_argument("--repeat", type=int, default=1, help="stream the same jobs this many times (longer timed region)")
 ap.add_argument("--check", type=int, default=2, help="jobs to verify against the oracle afterwards")
-ap.add_argument("--depth", type=int, default=0, help="jobs in flight (default: 2 per context, more for small jobs so that feeders can merge them)")
+ap.add_argument("--depth", type=int, default=0, help="jobs in flight (default: 2 per context, more for small jobs)")
 args = ap.parse_args()
 
 t0 = time.time()
@@ -64,6 +64,6 @@ if args.check:
         ok &= bool(np.array_equal(want.view(np.uint64), got.view(np.uint64)))
 print(json.dumps({"workload": synth.CONFIG_NAMES[5], "scale": args.scale, "regions": len(regions), "jobs": len(jobs) * args.repeat,
                   "pairs": pairs * args.repeat, "cells": cells * args.repeat, "n_gpus": ndev, "contexts_per_gpu": args.contexts,
-                  "jobs_in_flight": depth, "merged_gpu_jobs": pool.set_merge(), "wall_s": wall, "e2e_gcups": cells * args.repeat / wall * 1e-9, "fallback_pairs": nfb,
+                  "jobs_in_flight": depth, "wall_s": wall, "e2e_gcups": cells * args.repeat / wall * 1e-9, "fallback_pairs": nfb,
                   "bit_identical_to_oracle": ok, "device_load": pool.device_load()}))
 pool.close()
